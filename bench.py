@@ -30,6 +30,10 @@ independent replica beams (no collective, weak scaling) is kept as the extra key
 as-is reference (oracle/_ref, built by oracle/build_ref.py) for config 1, the oracle port (scipy
 BFGS over numpy columns -- the as-is reference cannot run at N >= ~1e4) for the others; one step =
 all candidates of one beam on all cores, one pool for the whole run.
+
+`--dump-outputs DIR` writes, after the timed steps, what the fit returned in the last timed step as
+DIR/<name>.npy (see dump_outputs).  The workload is seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -79,7 +83,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-api", action="store_true", help="skip the refine_hypotheses end-to-end loop")
     ap.add_argument("--rows", default="", help="comma separated table row names (default: table order)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the fit returned in the last timed step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU fit (--impl b200)")
     c = CONFIGS[a.config]
     a.points = a.points or c["points"]
     a.cand = a.cand or c["cand"]
@@ -221,7 +231,7 @@ class ClockSampler:
 # ---- CPU arm: the reference's path on the host cores ----------------------------------------------
 def _cpu_fit(job):
     """One candidate through the CPU implementation.  kind 'port': oracle/vectorised.py; kind
-    'reference': the unmodified reference's own bfgs_wrapper (oracle/_ref or /root/reference), with
+    'reference': the unmodified reference's own bfgs_wrapper (oracle/_ref or $VISYMRE_REFERENCE), with
     its per-restart np.random.randn draws fed from the workload's starting points."""
     import warnings
     warnings.filterwarnings("ignore")
@@ -357,13 +367,10 @@ def run_reference(args):
     _, t_probe, _ = arm.step(beams[0], limit=arm.cores)
     rounds = max(1, int(12.0 / max(t_probe, 1e-3)))
     limit = None if rounds * arm.cores >= args.cand else rounds * arm.cores
-    t_all = time.time()
     for s in range(args.warmup + args.steps):
         a, d, f = arm.step(beams[s], limit=limit)
         if s >= args.warmup:
             n, dt, nfev, steps = n + a, dt + d, nfev + f, steps + 1
-        if time.time() - t_all > 240 and steps >= 2:
-            break
     arm.close()
     v = n / dt
     line = {"impl": "reference", "metric": "candidate_fits_per_sec", "value": v, "unit": "candidate-fits/s",
@@ -376,6 +383,39 @@ def run_reference(args):
                                        f"{dt:.1f} s, nfev {nfev}", "seconds": dt, "nfev": nfev},
             "e2e": {"value": v, "unit": "candidate-fits/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     emit(line)
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, winners, res):
+    """Writes what ``fit_step`` returned as ``.npy`` files: the per-run FitResult fields and, when
+    sharded, the gathered per-candidate winners.  A non-finite entry is not a number to compare but
+    the absence of one (NaN fills the columns past a run's number of constants and every column of a
+    run with none; a score is NaN or inf where the expression is not real at the fitted point, and
+    the refinement skips it), so each float field is written as its finite entries in row-major
+    order, ``<name>.npy`` (float64), with ``<name>_finite.npy`` (float32, the field's shape, 1 where
+    the entry is finite).  ``info``'s int32 status / nit / nfev are written as float64, exactly.
+    Outputs over DUMP_LIMIT keep the same seeded sample of runs in every field, listed in ``runs.npy``."""
+    runs = {f: getattr(res, f).cpu().numpy() for f in ("consts", "lastx", "loss", "final_mse", "info")}
+    extra = {} if winners is None else {"winners": winners.cpu().numpy()}
+    n_runs = len(runs["loss"])
+    # at most 8 bytes per value and 4 per mask entry (info: 8 per entry, no mask)
+    per_run = sum(a[0].size * (8 if f == "info" else 12) for f, a in runs.items())
+    budget = DUMP_LIMIT - sum(a.size * 12 for a in extra.values())
+    out = {}
+    if n_runs * per_run > budget:
+        keep = np.sort(np.random.RandomState(0).choice(n_runs, int(budget // (per_run + 8)), replace=False))
+        runs = {f: a[keep] for f, a in runs.items()}
+        out["runs"] = keep.astype(np.float64)
+    out["info"] = runs.pop("info").astype(np.float64)
+    for name, a in {**runs, **extra}.items():
+        finite = np.isfinite(a)
+        out[name] = a[finite].astype(np.float64)
+        out[f"{name}_finite"] = finite.astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def workload_config(args):
@@ -530,6 +570,8 @@ def main():
     launches = sum(s["eng"].launches for s in setups.values()) - launches0
     fit_ms, fit_n, score_ms = prof[0], prof[1], prof[2]
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, winners[-1], results[-1])
 
     # ---- algorithmic work of the timed steps (from the runs' own evaluation counts) ----
     flops = pevals = abytes = 0.0

@@ -13,9 +13,9 @@ Modules
                   (tests/golden/ref_bfgs_*.json, made by oracle/make_golden.py).
   vm.py           a numpy interpreter for the skeleton bytecode, to check the
                   compiler against sympy.lambdify without a GPU.
-  ref_harness.py  imports the UNMODIFIED reference from /root/reference through inert
-                  stubs for packages absent here; only usable where /root/reference
-                  exists (this container), used to generate the golden vectors.
+  ref_harness.py  imports the UNMODIFIED reference from a checkout named by VISYMRE_REFERENCE
+                  through inert stubs for packages absent here; used to generate the
+                  golden vectors.
   hostsim/        g++ build of the kernels' portable cores (interpreter + BFGS state
                   machine) for logic checks against scipy on the CPU.
 """

@@ -1,20 +1,20 @@
 """Recipe for oracle/_ref: the UNMODIFIED reference hot path, byte-compiled where it lies.
 
 The reference is pure Python (no build system).  This script compiles the few modules its
-``bfgs()`` needs -- straight from ``/root/reference/src/visymre`` -- to code objects in ONE
+``bfgs()`` needs -- straight from ``$VISYMRE_REFERENCE/src/visymre`` -- to code objects in ONE
 archive ``oracle/_ref/modules.bin`` (no reference source text is copied into the repo) and extracts the pickled vocabulary record from ``scripts/weights/meta/metadata.h5`` (bytes
-2048..4974, SURVEY 8c).  ``oracle/_ref/`` is git-ignored but travels to the GPU box, where
-``/root/reference`` does not exist: there ``bench.py --impl reference --config 1`` times this
+2048..4974, SURVEY 8c).  ``oracle/_ref/`` is git-ignored; copied along with the tree to a machine without the
+checkout, it lets ``bench.py --impl reference --config 1`` time this
 as-is reference (``cpu_baseline.kind = "reference"``) and ``oracle/ref_harness.load()`` finds it.
 
-Run:  python oracle/build_ref.py      (``__graft_entry__.build()`` does, when /root/reference exists)
+Run:  python oracle/build_ref.py      (``__graft_entry__.build()`` does, when VISYMRE_REFERENCE names a checkout)
 TEST INFRASTRUCTURE: nothing under vision-sr_b200/ imports oracle/.
 """
 import os
 import shutil
 import sys
 
-REF = "/root/reference"
+REF = os.environ.get("VISYMRE_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(HERE, "_ref")
 # what `import src.visymre.architectures.bfgs` / `.model` pull in (SURVEY 2.1), nothing else
@@ -34,8 +34,8 @@ def build(ref=REF, out=OUT):
     ``marshal``: what a ``.pyc`` holds, without the file names a snapshot tool may filter)."""
     import marshal
     import pickle
-    if not os.path.isdir(ref):
-        raise FileNotFoundError(f"{ref} is not here: oracle/_ref can only be built in the build container")
+    if not ref or not os.path.isdir(ref):
+        raise FileNotFoundError("oracle/_ref is built from a checkout of the reference: set VISYMRE_REFERENCE")
     if os.path.isdir(out):
         shutil.rmtree(out)
     os.makedirs(out)

@@ -1,7 +1,7 @@
 """Generate tests/golden/ref_bfgs.json from the UNMODIFIED reference.
 
-Run here (build container) only:  python oracle/make_golden.py
-It imports /root/reference through oracle/ref_harness.py, runs the reference's own
+Run with VISYMRE_REFERENCE naming a reference checkout:  python oracle/make_golden.py
+It imports the reference (VISYMRE_REFERENCE) through oracle/ref_harness.py, runs the reference's own
 ``bfgs()`` / ``bfgs_wrapper()`` on small seeded cases and records inputs, outputs and
 per-restart optimiser facts (captured by wrapping the ``minimize`` name inside the
 reference module; the reference source is not modified).

@@ -8,7 +8,7 @@ Two things are recorded for seeded random beams of prefix sequences:
     the reference file AT GENERATION TIME (between its own two marker comments), dedented and
     executed unchanged with the names the method has in scope at that point.
 
-Run here (build container) only:  python oracle/make_golden_beam.py
+Run with VISYMRE_REFERENCE naming a reference checkout:  python oracle/make_golden_beam.py
 TEST INFRASTRUCTURE: nothing under vision-sr_b200/ imports this.
 """
 import json

@@ -2,7 +2,7 @@
 BASELINE config 1: rows of scripts/low_benchmarks.csv, N = 500 points, R = 10 restarts -- the only
 configuration the as-is reference can run at full size (SURVEY.md section 8d).
 
-Run here (build container) only:  python oracle/make_golden_low.py [rows] [candidates per row]
+Run with VISYMRE_REFERENCE naming a reference checkout:  python oracle/make_golden_low.py [rows] [candidates per row]
 
 Two processes, because the product package and the reference are both a top-level package
 named ``src``:

@@ -1,7 +1,8 @@
 """Import the UNMODIFIED reference hot path (TEST INFRASTRUCTURE, generation only).
 
-``/root/reference`` exists only in the build container, never on the GPU box, so
-this module is used by ``oracle/make_golden.py`` alone.  The reference's
+A checkout of the reference (aidalee123/Vision-SR), named by the environment variable
+``VISYMRE_REFERENCE``, is needed to regenerate the golden vectors under ``tests/golden/``; the tests
+read those vectors, except ``tests/test_overlay.py``, which skips without the checkout.  The reference's
 ``src/visymre/architectures/bfgs.py`` imports cleanly once the packages that are
 absent here -- none of which ``bfgs()`` touches -- are replaced by inert stubs
 (SURVEY.md section 8c).  Run it in a process that does NOT have ``vision-sr_b200`` on
@@ -13,7 +14,8 @@ import pickle
 import sys
 import types
 
-REF_ROOT = "/root/reference"
+# a checkout of aidalee123/Vision-SR; unset: only oracle/_ref (oracle/build_ref.py) can serve the reference
+REF_ROOT = os.environ.get("VISYMRE_REFERENCE", "")
 _STUBS = ("numexpr", "hydra", "pytorch_lightning", "func_timeout", "h5py", "omegaconf")
 
 
@@ -56,9 +58,9 @@ VENDORED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")   # 
 
 
 def available():
-    """Where the unmodified reference can be imported from: its tree (build container) or the
-    byte-compiled copy oracle/build_ref.py made (GPU box); None when neither is here."""
-    if os.path.isdir(os.path.join(REF_ROOT, "src", "visymre")):
+    """Where the unmodified reference can be imported from: its checkout (VISYMRE_REFERENCE) or the
+    byte-compiled copy oracle/build_ref.py made; None when neither is here."""
+    if REF_ROOT and os.path.isdir(os.path.join(REF_ROOT, "src", "visymre")):
         return REF_ROOT
     tag = os.path.join(VENDORED, "PYTHON")
     if os.path.exists(tag) and open(tag).read().strip() == f"{sys.version_info.major}.{sys.version_info.minor}":
@@ -94,7 +96,7 @@ def load(ref_root=None):
     """Returns (bfgs_module, model_module_or_None, test_data)."""
     ref_root = ref_root or available()
     if ref_root is None:
-        raise ImportError("neither /root/reference nor oracle/_ref (python oracle/build_ref.py) is here")
+        raise ImportError("neither VISYMRE_REFERENCE nor oracle/_ref (python oracle/build_ref.py) is here")
     _install_stubs()
     archive = os.path.join(ref_root, "modules.bin")
     if os.path.exists(archive):

@@ -8,7 +8,7 @@ on a SCRIPTED decoder: the network parts (``MultiModalEncoder``, ``decoder_trans
 ...) are replaced by stand-ins that steer the reference's unmodified beam loop towards two known
 skeletons, so everything from line 292 of model.py down to the returned dict is the tree's code.
 In the patched tree the numeric fit inside ``refine_hypotheses`` is served by the CPU oracle
-(there is no GPU in the build container); the reference tree runs its own process-pool BFGS.
+(the test needs no GPU); the reference tree runs its own process-pool BFGS.
 """
 import json
 import os
@@ -37,7 +37,7 @@ info = {"has_refine_call": "refine_hypotheses(" in src, "has_process_pool": "Pro
 
 import pickle  # noqa: E402
 
-raw = open("/root/reference/scripts/weights/meta/metadata.h5", "rb").read()
+raw = open(os.path.join(tree, "scripts/weights/meta/metadata.h5"), "rb").read()   # overlay.install copies it
 td = pickle.loads(raw[2048:2048 + 2926])
 w = td.word2id
 n_words = max(w.values()) + 1

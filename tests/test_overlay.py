@@ -2,7 +2,8 @@
 the package over a copy of the reference checkout, ``scripts/visymre_utils.py`` imports as the
 drivers import it, and the checkout's own ``Model.fitfunc2`` -- beam loop and all -- ends in
 ``refine_hypotheses``.  Its output dict is compared with the UNPATCHED reference run on the same
-scripted decoder.  Needs /root/reference (build container only)."""
+scripted decoder.  Needs a checkout of the reference, named by VISYMRE_REFERENCE (oracle/ref_harness.py);
+skips without one."""
 import json
 import os
 import subprocess
@@ -11,16 +12,16 @@ import sys
 import pytest
 
 from conftest import PKG, ROOT
+from oracle.ref_harness import REF_ROOT as REF
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "visymre")),
-                                reason="the reference checkout is only present in the build container")
+pytestmark = pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "src", "visymre")),
+                                reason="needs a checkout of the reference: set VISYMRE_REFERENCE")
 
 
 def _run(tree, patched, out):
     env = {k: v for k, v in os.environ.items() if k != "PYTHONPATH"}
     p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "_overlay_driver.py"), tree, "1" if patched else "0",
-                        ROOT, out], capture_output=True, text=True, timeout=900, cwd="/tmp", env=env)
+                        ROOT, out], capture_output=True, text=True, timeout=900, cwd=os.path.dirname(out), env=env)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-4000:]
     return json.load(open(out))
 

@@ -1,6 +1,6 @@
 """Extract the equation tables the benchmark workloads are built from.
 
-Run in the build container only (reads /root/reference):
+Run with VISYMRE_REFERENCE naming a checkout of the reference (aidalee123/Vision-SR):
     python tools/make_workload_tables.py
 Writes vision-sr_b200/src/visymre/workloads/tables.json with, per table row, just what the
 workload generator needs: name, formula string, variable names and sampling ranges.
@@ -17,7 +17,8 @@ import sys
 import zipfile
 from xml.etree import ElementTree as ET
 
-REF = "/root/reference/scripts"
+CHECKOUT = os.environ.get("VISYMRE_REFERENCE", "")
+REF = os.path.join(CHECKOUT, "scripts")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(ROOT, "vision-sr_b200", "src", "visymre", "workloads", "tables.json")
 
@@ -177,7 +178,7 @@ def main():
             out[key] = [dict(name=r["name"], n_vars=int(r["variables"]), formula=r["expression"],
                              range=json.loads(r["range_"])) for r in csv.DictReader(fh)]
     # vocabulary
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, CHECKOUT)
     import pickle
     import src.visymre.dclasses  # noqa: F401  (the pickle names this module)
     raw = open(os.path.join(REF, "weights/meta/metadata.h5"), "rb").read()
