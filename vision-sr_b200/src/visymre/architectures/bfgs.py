@@ -14,6 +14,9 @@ config.yaml does not have them, so drivers keep working unchanged):
               forward differences, reproduces the reference's trajectories)
   precision   "fp64" (default, what the reference's loss uses) or "fp32"
   prune_threshold / prune_tolerance   as in the reference (bfgs.py:143-144)
+  devices     None (default: one engine on the current device), "all" (every visible CUDA device) or
+              a list of device indices / torch.devices, the first one the home device: the beam's
+              runs are dealt over one engine per entry in this process (``resolve_devices``)
 """
 import re
 
@@ -49,6 +52,49 @@ def _opt(cfg, name, default=None):
         return b[name]
     except (KeyError, TypeError, IndexError):
         return default
+
+
+def resolve_devices(cfg):
+    """``cfg.bfgs.devices`` as a list of CUDA ``torch.device``s (the first one is the home device, where
+    the inputs and the fit's results live), or None when it is unset or None.
+
+    ``"all"``: every visible CUDA device.  A list of device indices or devices: those, in that order; an
+    entry may repeat, which puts a further engine on that device.  More than one device in a process that
+    has a torch.distributed process group is a ``ValueError``: the runs are dealt over the ranks there
+    (``bfgs.shard``), and dealing them over the ranks and the devices at once is not defined."""
+    spec = _opt(cfg, "devices", None)
+    if spec is None:
+        return None
+    if isinstance(spec, str) and spec.strip().lower() == "all":
+        devs = [torch.device("cuda", i) for i in range(torch.cuda.device_count())]
+    else:
+        items = [spec] if isinstance(spec, (int, str, torch.device)) else list(spec)
+        devs = []
+        for d in items:
+            try:
+                d = torch.device(d) if isinstance(d, (str, torch.device)) else torch.device("cuda", int(d))
+            except (RuntimeError, TypeError, ValueError) as exc:
+                raise ValueError(f"cfg.bfgs.devices: {d!r} is not a CUDA device") from exc
+            if d.type != "cuda":
+                raise ValueError(f"cfg.bfgs.devices: {d} is not a CUDA device (the engine has no CPU path)")
+            devs.append(d)
+    if len(devs) > 1 and _process_group():
+        raise ValueError("cfg.bfgs.devices names several devices in a process with a torch.distributed process "
+                         "group: deal the runs over the ranks (bfgs.shard) or over the devices of one process, "
+                         "not both")
+    if not devs:
+        raise ValueError(f"cfg.bfgs.devices = {spec!r}: no CUDA device")
+    n = torch.cuda.device_count()
+    devs = [torch.device("cuda", torch.cuda.current_device()) if d.index is None else d for d in devs]
+    for d in devs:
+        if d.index >= n:
+            raise ValueError(f"cfg.bfgs.devices: {d} does not exist ({n} CUDA devices visible)")
+    return devs
+
+
+def _process_group():
+    import torch.distributed as dist
+    return dist.is_available() and dist.is_initialized()
 
 
 def skeleton_string(pred_str, cfg, test_data):
@@ -505,6 +551,9 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
         LAST_TIMING[name] = LAST_TIMING.get(name, 0.0) + (now - _t[0]) * 1e3
         _t[0] = now
     LAST_TIMING.clear()
+    devices = resolve_devices(cfg)
+    if devices and engine is not None and engine.device != devices[0]:
+        raise ValueError(f"engine on {engine.device}, but the home device of cfg.bfgs.devices is {devices[0]}")
     y = y.squeeze()
     Xt = torch.as_tensor(X)
     if Xt.dim() == 2:
@@ -547,7 +596,7 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
         raise KeyError(norm)
 
     eng = engine if engine is not None else fitter.get_engine(
-        Xt.device if Xt.is_cuda else None)
+        devices[0] if devices else (Xt.device if Xt.is_cuda else None))
     score_dtype = fitter.F32 if Xt.dtype == torch.float32 else fitter.F64
     eval_dtype = fitter.F32 if str(_opt(cfg, "precision", "fp64")).lower() == "fp32" else fitter.F64
     eng.set_points(Xt[0], yt_fit, dtypes=tuple({eval_dtype, score_dtype, fitter.F64}))
@@ -558,13 +607,20 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
     _mark("upload")
 
     world = sharding.world_size() if _opt(cfg, "shard", True) and not rows_removed else 1
+    # cfg.bfgs.devices with several entries: the runs are dealt over one engine per entry, in this process
+    # (like the ranks: one stage, one record per candidate back).  Rows dropped by idx_remove keep the fit
+    # on the home device, as they keep it on one rank.
+    spread = devices is not None and len(devices) > 1 and not rows_removed
+    if spread:
+        engines = fitter.device_engines(devices, home=eng)
+        fitter.share_points(engines)
     # Stages: the skeletons are compiled heaviest first (most constants = longest fits); the fit of a
     # FIRST stage starts as soon as enough candidates to fill the GPU are compiled -- whichever they
     # are: sympy takes 3 ms for most skeletons and 30-60 ms for a few -- on the main engine; the rest
     # follows on side engines and streams that share the points, stragglers in a stage of their own.
     # One stage when there is nothing to overlap.
     def _stages():
-        if not (comp.staged and world == 1 and n_cand >= 24 and _opt(cfg, "pipeline", True)):
+        if not (comp.staged and world == 1 and not spread and n_cand >= 24 and _opt(cfg, "pipeline", True)):
             yield list(range(n_cand))
             return
         for j in (1, 2, 3):                    # the side engines exist before the first stage is launched
@@ -610,7 +666,7 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
                 start[li * R + r, :k] = v
         return start
 
-    win_of = {}     # candidate -> record of the all-gather                (sharded)
+    win_of = {}     # candidate -> record of the all-gather                (sharded, spread)
     launched = []
     for si, stage in enumerate(_stages()):
         live_s = _collect(stage)
@@ -618,16 +674,26 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
         if not live_s:
             continue
         start = _starts(live_s)
-        if world > 1:
-            # SURVEY 8e: the (candidate, restart) runs of the beam are dealt over the ranks of the default
-            # process group, every rank fits its share, ONE all-gather brings back a record per candidate
-            # (score, restart, constants) and every rank takes the same argmin.  Every rank must have
-            # been called with the same candidates and points; the starting points are rank 0's.
-            eng.set_programs([cands[i].prog for i in live_s])
-            start_dev = sharding.broadcast_from_rank0(torch.from_numpy(start).to(eng.device))
+        if world > 1 or spread:
             cost = np.repeat([(cands[ci].k + 1.0) * cands[ci].prog.n_insns for ci in live_s], R)
-            win, _ = sharding.fit_sharded(eng, [cands[ci].k for ci in live_s], R, start_dev, opts, cost=cost,
-                                          key_dtype=torch.float32 if score_dtype == fitter.F32 else None)
+            key_dtype = torch.float32 if score_dtype == fitter.F32 else None
+            if spread:
+                # the same dealing, per-part records and merge as the ranks', over the engines of this process
+                for e in engines:
+                    with torch.cuda.device(e.device):
+                        e.set_programs([cands[i].prog for i in live_s])
+                win, _ = sharding.fit_devices(engines, [cands[ci].k for ci in live_s], R,
+                                              torch.from_numpy(start).to(eng.device), opts, cost=cost,
+                                              key_dtype=key_dtype)
+            else:
+                # SURVEY 8e: the (candidate, restart) runs of the beam are dealt over the ranks of the default
+                # process group, every rank fits its share, ONE all-gather brings back a record per candidate
+                # (score, restart, constants) and every rank takes the same argmin.  Every rank must have
+                # been called with the same candidates and points; the starting points are rank 0's.
+                eng.set_programs([cands[i].prog for i in live_s])
+                start_dev = sharding.broadcast_from_rank0(torch.from_numpy(start).to(eng.device))
+                win, _ = sharding.fit_sharded(eng, [cands[ci].k for ci in live_s], R, start_dev, opts, cost=cost,
+                                              key_dtype=key_dtype)
             win = win.cpu().numpy()
             for li, ci in enumerate(live_s):
                 win_of[ci] = win[li]

@@ -16,7 +16,7 @@ repo's own package ``architectures/model.py`` re-exports it under the reference'
 import numpy as np
 import torch
 
-from .bfgs import LazyStrings, bfgs, bfgs_batch
+from .bfgs import LazyStrings, bfgs, bfgs_batch, resolve_devices
 
 UNARY_NAMES = ("abs", "asin", "cos", "exp", "ln", "sin", "sqrt", "tan")   # model.py:295
 BINARY_NAMES = ("add", "div", "mul", "pow", "sub")                        # model.py:296
@@ -80,7 +80,9 @@ def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None):
     ``hyps``: ``generated_hyps.hyp``, a list of ``(score, tokens)``; ``X`` ``[1, N, 10]``
     and ``y`` ``[1, N, 1]`` as fitfunc2 holds them (any device).  Returns the reference's
     output dict.  Candidates come back in beam order (the reference's order is process
-    completion order, which is not reproducible).
+    completion order, which is not reproducible).  ``cfg_params.bfgs.devices`` spreads the fit
+    over several GPUs of this process (``bfgs.resolve_devices``); an invalid value raises
+    ``ValueError`` here instead of failing every candidate.
     """
     w2i = test_data.word2id
     arity_1 = {w2i[n] for n in UNARY_NAMES if n in w2i}
@@ -110,6 +112,7 @@ def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None):
 
     P_bfgs, L_bfgs, token = [], [], []
     if valid:
+        resolve_devices(cfg_params)     # a wrong cfg.bfgs.devices is the caller's error, not every candidate's
         try:
             outs = bfgs_batch(valid, X, y, cfg_params, test_data, x0=x0, engine=engine, lazy_strings=True)
         except Exception as exc:  # noqa: BLE001 -- a batch-level failure fails every candidate

@@ -325,3 +325,37 @@ def side_stream(device, i):
     if key not in _SIDE_STREAMS:
         _SIDE_STREAMS[key] = torch.cuda.Stream(device=dev)
     return _SIDE_STREAMS[key]
+
+
+def device_engines(devices, home=None):
+    """One engine per entry of ``devices`` (CUDA devices, the first one the home device).  The first
+    entry of a device gets that device's process-wide engine (``get_engine``; ``home`` for the first
+    entry when given), every further entry of the same device another engine beside it
+    (``get_side_engine``, the j-th repeat on side stream j), so that one GPU can hold several parts of
+    a beam."""
+    engines, first = [], {}
+    for i, d in enumerate(devices):
+        d = torch.device(d)
+        with torch.cuda.device(d):          # creating a handle makes its device current: not the caller's
+            if d not in first:
+                first[d] = home if (i == 0 and home is not None) else get_engine(d)
+                engines.append(first[d])
+            else:
+                engines.append(get_side_engine(first[d], sum(1 for e in engines if e.device == d)))
+    return engines
+
+
+def share_points(engines):
+    """Give every engine the points ``engines[0]`` holds (``set_points`` was called on it).  Each other
+    device gets one copy, made from the home device's tensors: a peer copy on the home stream that torch
+    orders before the device's own stream.  Further engines of a device adopt that device's copy."""
+    home = engines[0]
+    X, y = home._src
+    holder = {home.device: home}
+    for eng in engines[1:]:
+        if eng.device in holder:
+            eng.adopt_points(holder[eng.device])
+            continue
+        with torch.cuda.device(eng.device):
+            eng.set_points(X, y, dtypes=home._want_dtypes, n_vars=home.n_vars)
+        holder[eng.device] = eng

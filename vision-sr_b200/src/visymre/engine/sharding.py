@@ -10,7 +10,12 @@ Ties and all-nan candidates resolve to the lowest restart index -- what ``np.nan
 over the restarts gives on a single GPU (bfgs.py:134-141).
 
 torch.distributed is plumbing here (NCCL on GPUs, gloo in the CPU tests).
+
+``fit_devices`` is the same dealing and merge inside ONE process that holds an engine per device:
+device-to-device copies of the records take the place of the all-gather.
 """
+import contextlib
+
 import numpy as np
 import torch
 import torch.distributed as dist
@@ -139,3 +144,95 @@ def fit_sharded(engine, programs_k, n_restarts, x0, opts, cost=None, group=None,
     mine[torch.as_tensor(mine_idx, device=mine.device)] = True
     rec = local_best_records(res.final_mse, res.loss, res.lastx, C, R, mine, key_dtype)
     return allgather_best(rec, group, n_restarts=R), res
+
+
+def _engine_streams(engines):
+    """The stream each engine fits on: its device's current stream for the first engine of a device, side
+    stream j for the j-th further one (``fitter.device_engines`` made it with that stream); None off CUDA."""
+    from . import fitter
+    seen, out = {}, []
+    for eng in engines:
+        dev = torch.device(eng.device)
+        j = seen.get(dev, 0)
+        seen[dev] = j + 1
+        if dev.type != "cuda":
+            out.append(None)
+        else:
+            out.append(torch.cuda.current_stream(dev) if j == 0 else fitter.side_stream(dev, j))
+    return out
+
+
+def _on(dev, stream):
+    ctx = contextlib.ExitStack()
+    if stream is not None:
+        ctx.enter_context(torch.cuda.device(dev))
+        ctx.enter_context(torch.cuda.stream(stream))
+    return ctx
+
+
+def fit_devices(engines, programs_k, n_restarts, x0, opts, cost=None, key_dtype=None):
+    """Fit a beam with its runs dealt over the engines of ONE process, ``engines[0]``'s device being the
+    home device: the single-process twin of ``fit_sharded``, with the same dealing (``partition_runs``),
+    the same per-part reduction (``local_best_records``) and the same merge (``merge_records``), so that
+    the winners are those of one engine that fits every run.
+
+    Every engine holds the same points and the same program list (``fitter.share_points``,
+    ``set_programs``); an engine may share its device with others.  x0: [C*R, kmax] on the home device
+    (or the host); it is copied once to every other device on the home stream.  Every engine's fit is
+    enqueued before the host waits on any of them, so that they run concurrently.  The records travel
+    to the home device by device-to-device copies.  Returns ``(winners [C, 4+kmax] on the home device,
+    [FitResult per engine])`` -- the layout of ``fit_sharded``.  When any device fails, ``VsrError``
+    names it, raised once every device's work has finished.
+    """
+    from .native import VsrError
+    C, R = len(programs_k), n_restarts
+    if cost is None:
+        cost = np.repeat(np.asarray(programs_k, dtype=np.float64) + 1.0, R)
+    parts = partition_runs(cost, len(engines))
+    home = torch.device(engines[0].device)
+    x0 = torch.as_tensor(x0, dtype=torch.float64).to(home)
+    kstride = int(x0.shape[1])
+    x0_on = {}
+    for eng in engines:        # peer copies on the home stream; torch makes the device's stream wait for them
+        x0_on.setdefault(torch.device(eng.device), None)
+    for dev in x0_on:
+        x0_on[dev] = x0.to(dev, non_blocking=True)
+    streams = _engine_streams(engines)
+    results, recs, errors = [None] * len(engines), [None] * len(engines), []
+    for i, (eng, mine_idx, stream) in enumerate(zip(engines, parts, streams)):
+        dev = torch.device(eng.device)
+        cur = torch.cuda.current_stream(dev) if stream is not None else None
+        try:
+            with _on(dev, stream):
+                x0_d = x0_on[dev]
+                if stream is not None and stream != cur:   # a further engine of the device: after the uploads
+                    stream.wait_stream(cur)
+                    x0_d.record_stream(stream)
+                if len(mine_idx):
+                    res = eng.fit((mine_idx // R).astype(np.int32), mine_idx.astype(np.int32), x0_d, opts)
+                else:      # more engines than runs (vsr_fit rejects an empty run list)
+                    res = empty_result(C * R, kstride, dev)
+                mine = torch.zeros(C * R, dtype=torch.bool)
+                mine[torch.as_tensor(mine_idx, dtype=torch.long)] = True
+                # pageable host -> device without a stream synchronisation: the fit above stays in flight
+                mine = mine.to(dev, non_blocking=True)
+                rec = local_best_records(res.final_mse, res.loss, res.lastx, C, R, mine, key_dtype)
+            if stream is not None and stream != cur:
+                cur.wait_stream(stream)
+                rec.record_stream(cur)          # read there by the copy or the merge
+            with _on(dev, cur):
+                recs[i] = rec.to(home, non_blocking=True)
+            results[i] = res
+        except Exception as exc:  # noqa: BLE001 -- raised below, once no device works any more
+            errors.append((dev, exc))
+    for dev in x0_on:
+        if dev.type == "cuda":
+            try:
+                torch.cuda.synchronize(dev)
+            except Exception as exc:  # noqa: BLE001 -- an asynchronous error of that device's work
+                errors.append((dev, exc))
+    if errors:
+        dev, exc = errors[0]
+        more = f" (and {len(errors) - 1} more: {', '.join(str(d) for d, _ in errors[1:])})" if len(errors) > 1 else ""
+        raise VsrError(f"fit on {dev} failed: {exc}{more}") from exc
+    return merge_records(torch.stack(recs), R), results
