@@ -109,6 +109,18 @@ int vsr_score(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row,
               int32_t n_pairs, const double* consts, int32_t kstride, int32_t dtype,
               double* out_mse, void* stream);
 
+/* Gauss-Newton statistics of n_pairs (program, constants) pairs over all points, fp64:
+ *   out_rss[p]          = sum_i (f(x_i; c) - y_i)^2
+ *   out_jtj[p][a][b]    = sum_i df(x_i)/dc_a * df(x_i)/dc_b   (a, b < k; full symmetric,
+ *                          row stride kstride; entries with a or b >= k are not written)
+ * Same pair arguments as vsr_eval.  Programs with k > VSR_MAX_DUAL: jtj rows nan.
+ * What a covariance of fitted constants is built from (sigma^2 (J^T J)^-1, as
+ * scipy.optimize.curve_fit's pcov); the reference has no counterpart.  Always reads the VSR_F64
+ * point slot.  Non-finite values propagate: a point where f is not real makes both outputs nan.
+ * The result of a pair does not depend on the other pairs of the call, bit for bit. */
+int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, int32_t n_pairs,
+             const double* consts, int32_t kstride, double* out_rss, double* out_jtj, void* stream);
+
 /* Multi-restart BFGS for n_runs (program, restart) runs; run r of the list fits program
  * run_prog[r] from x0[run_slot[r]] and writes every output at row run_slot[r]
  * (slots let a rank fit a shard of a C x R problem in place).  run_prog and run_slot

@@ -244,6 +244,15 @@ cudaError_t launch_eval_tile(int K, const vsr::EvalTileArgs& a, size_t smem, cud
   return cudaErrorInvalidValue;
 }
 
+cudaError_t launch_gram(int K, const vsr::GramArgs& a, size_t smem, cudaStream_t st) {
+  switch (K) {
+#define C(KK) case KK: return vsr::launch_gram_K<KK>(a, smem, st);
+    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
+#undef C
+  }
+  return cudaErrorInvalidValue;
+}
+
 int eval_tile_threads_of(int K) {
   switch (K) {
 #define C(KK) case KK: return vsr::eval_tile_threads<KK>();
@@ -818,6 +827,88 @@ int vsr_eval(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, i
   }
   if (out_grad) {
     // width-0 pairs (k == 0) have no gradient entries to write
+  }
+  return VSR_OK;
+}
+
+int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, int32_t n_pairs,
+             const double* consts, int32_t kstride, double* out_rss, double* out_jtj, void* stream) {
+  int rc = check_ready(h, VSR_F64);
+  if (rc) return rc;
+  if (!prog_idx || n_pairs <= 0 || !out_rss || kstride < 0 || ((!consts || !out_jtj) && kstride > 0))
+    return fail(h, VSR_EINVAL, "bad gram arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  VSR_CUDA(h, cudaSetDevice(h->device));
+  // group pairs by tangent width; programs wider than VSR_MAX_DUAL go with the width-0 group (rss
+  // only, gram_finalize writes their jtj as nan)
+  std::vector<Group> groups(kNumWidths);
+  std::vector<std::vector<int32_t>> outs(kNumWidths);
+  for (int i = 0; i < kNumWidths; ++i) groups[i].K = kWidths[i];
+  for (int p = 0; p < n_pairs; ++p) {
+    const int c = prog_idx[p];
+    if (c < 0 || c >= h->n_programs) return fail(h, VSR_EINVAL, "pair %d: program %d out of range", p, c);
+    const int k = h->h_k[c];
+    if (k > kstride) return fail(h, VSR_EINVAL, "pair %d: %d constants > kstride %d", p, k, kstride);
+    if ((rc = check_vars(h, c, VSR_F64))) return rc;
+    const int w = pick_width(k);
+    const int gi = w < 0 ? 0 : (int)(std::find(kWidths, kWidths + kNumWidths, w) - kWidths);
+    Group& g = groups[gi];
+    g.prog.push_back(c);
+    g.slot.push_back(const_row ? const_row[p] : p);
+    g.kmax = std::max(g.kmax, k);
+    g.max_insn = std::max(g.max_insn, h->h_ninsn[c]);
+    g.max_imm = std::max(g.max_imm, h->h_nimm[c]);
+    outs[gi].push_back(p);
+  }
+  std::vector<int32_t> all;
+  std::vector<size_t> off(kNumWidths, 0);
+  for (int gi = 0; gi < kNumWidths; ++gi) {
+    off[gi] = all.size();
+    all.insert(all.end(), groups[gi].prog.begin(), groups[gi].prog.end());
+    all.insert(all.end(), groups[gi].slot.begin(), groups[gi].slot.end());
+    all.insert(all.end(), outs[gi].begin(), outs[gi].end());
+  }
+  rc = stage_lists(h, all, st);
+  if (rc) return rc;
+  const int32_t* dl = (const int32_t*)h->d_lists.p;
+  const PointSlot& ps = h->pts[VSR_F64];
+  // the groups share the partial buffer: size it for all of them at once, so that a reserve (which
+  // frees the old block) never happens while an earlier group's partials are still to be summed
+  size_t need = 0;
+  for (int gi = 0; gi < kNumWidths; ++gi) {
+    const int K = groups[gi].K;
+    const int nsplit = vsr::gram_nsplit(ps.n, (int64_t)vsr::kGramThreads * points_per_thread(K));
+    need += groups[gi].prog.size() * (size_t)nsplit * vsr::gram_entries(K);
+  }
+  VSR_CUDA(h, h->d_partial.reserve(need * sizeof(double)));
+  double* partial = (double*)h->d_partial.p;
+  for (int gi = 0; gi < kNumWidths; ++gi) {
+    const Group& g = groups[gi];
+    const int n = (int)g.prog.size();
+    if (!n) continue;
+    const int K = g.K;
+    const int tile = vsr::kGramThreads * points_per_thread(K);
+    vsr::GramArgs a;
+    a.pt = table_of(h);
+    a.pts = points_of(ps);
+    a.pair_prog = dl + off[gi];
+    a.pair_row = dl + off[gi] + n;
+    a.n_pairs = n;
+    a.kstride = kstride;
+    a.consts = consts;
+    a.partial = partial;
+    a.nsplit = vsr::gram_nsplit(ps.n, tile);
+    const size_t smem = sizeof(double) * ((size_t)(K + 1) * vsr::gram_col_stride(tile) + g.kmax + 1 + g.max_imm) +
+                        sizeof(vsr_insn_t) * (g.max_insn + 1);
+    cudaError_t e = launch_gram(K, a, smem, st);
+    if (e != cudaSuccess) return fail(h, VSR_ECUDA, "gram kernel launch failed: %s", cudaGetErrorString(e));
+    const int64_t total = (int64_t)n * (1 + (int64_t)kstride * kstride);
+    vsr::gram_finalize<<<(unsigned)((total + 127) / 128), 128, 0, st>>>(partial, a.pair_prog, dl + off[gi] + 2 * n,
+                                                                         a.pt.k, n, a.nsplit, K, kstride, out_rss,
+                                                                         out_jtj);
+    VSR_CUDA(h, cudaGetLastError());
+    h->launches += 2;
+    partial += (size_t)n * a.nsplit * vsr::gram_entries(K);
   }
   return VSR_OK;
 }

@@ -1,5 +1,6 @@
 // vsr_inst.cu -- one instantiation of fit_kernel / eval_kernel and their launch wrappers:
-// compiled once per (VSR_INST_T, VSR_INST_K) pair, see the Makefile.
+// compiled once per (VSR_INST_T, VSR_INST_K) pair, see the Makefile.  The double units
+// (VSR_INST_GRAM) also hold gram_kernel of their width.
 #include <algorithm>
 
 #include "vsr_launch.h"
@@ -91,6 +92,15 @@ cudaError_t launch_eval_tile_T(const EvalTileArgs& a, size_t smem, cudaStream_t 
   kern<<<a.e.nsplit, eval_tile_threads<K>(), smem, st>>>(a);
   return cudaGetLastError();
 }
+
+#if defined(VSR_INST_GRAM)
+template <int K>
+cudaError_t launch_gram_K(const GramArgs& a, size_t smem, cudaStream_t st) {
+  gram_kernel<K, points_per_thread(K)><<<dim3(a.n_pairs, a.nsplit), kGramThreads, smem, st>>>(a);
+  return cudaGetLastError();
+}
+template cudaError_t launch_gram_K<VSR_INST_K>(const GramArgs&, size_t, cudaStream_t);
+#endif
 
 template <typename T, int K>
 cudaError_t preload_T() {

@@ -12,6 +12,8 @@
 //                       splits the points.  Replaces bfgs.py:106-112 and :120-132.
 //   eval_tile_kernel    the same over chunks of the points that all pairs of a launch share (N >= 5e5).
 //   eval_finalize       deterministic fixed-order sum of the split partials.
+//   gram_kernel<K,P>    fp64 sum r^2 and J^T J of (program, constants) pairs (Gauss-Newton statistics
+//                       for the covariance of fitted constants); gram_finalize sums its splits.
 //
 // Work mapping: lanes stride over points (coalesced column reads), P points per thread
 // share one instruction decode; per-thread partial sums are fp64 and parked in shared memory, then
@@ -1293,6 +1295,115 @@ __global__ void __launch_bounds__((eval_tile_threads<K>()), 1) eval_tile_kernel(
   }
 }
 
+// ---- Gauss-Newton statistics of (program, constants) pairs -----------------------------------------
+// For each pair, over all N points, in fp64 from the fp64 point slot:
+//   rss = sum_i r_i^2,   jtj[a][b] = sum_i J_ia J_ib   (a <= b < K),
+// r_i = f(x_i; c) - y_i and J_ia the tangent of constant a.  The grid is (pairs x point splits) like
+// eval_kernel's.  A CTA interprets one tile of blockDim.x * P points at a time, parks r and J of the
+// tile's points in shared memory, and after one barrier thread t adds ITS entry of the upper triangle
+// (t = 0: rss) over the tile's points in point order, into a register carried from tile to tile.  The
+// split count is a function of N alone (gram_nsplit) and every sum runs in a fixed order, so a pair's
+// result does not depend on the other pairs of the call or on its place in the list.  Non-finite
+// values propagate (no penalty rule): a point where f is not real makes the outputs nan.
+// partial[pair][split][gram_entries(K)] in the order rss, (0,0), (0,1) .. (0,K-1), (1,1) ..
+struct GramArgs {
+  ProgramTable pt;
+  Points pts;  // the fp64 slot
+  const int32_t* pair_prog;  // [n_pairs]
+  const int32_t* pair_row;   // [n_pairs] row of `consts`
+  int32_t n_pairs;
+  int32_t kstride;
+  const double* consts;
+  double* partial;  // [n_pairs][nsplit][gram_entries(K)]
+  int32_t nsplit;
+};
+
+constexpr int kGramThreads = 256;
+__host__ __device__ constexpr int gram_entries(int K) { return 1 + K * (K + 1) / 2; }
+static_assert(gram_entries(VSR_MAX_DUAL) <= kGramThreads, "one thread per Gram entry");
+// splits of the points: at least 16 tiles each, at most 128 splits (a function of N only)
+__host__ __device__ inline int gram_nsplit(int64_t N, int64_t tile) {
+  const int64_t tiles = (N + tile - 1) / tile;
+  const int64_t s = tiles / 16;
+  return (int)(s < 1 ? 1 : (s > 128 ? 128 : s));
+}
+// column stride (doubles) of the tile's values in shared memory: odd, so that the lanes of a warp,
+// which read the same point of different tangent columns, hit different banks
+__host__ __device__ constexpr int gram_col_stride(int tile) { return tile + 1; }
+
+// dynamic shared memory of gram_kernel, in doubles: tile[(K+1) * gram_col_stride] | cst[k] | imm | insn
+template <int K, int P>
+__global__ void __launch_bounds__(kGramThreads) gram_kernel(const GramArgs a) {
+  extern __shared__ double smem[];
+  const int pair = blockIdx.x;
+  const int split = blockIdx.y;
+  const int tid = threadIdx.x;
+  constexpr int kTile = kGramThreads * P;
+  constexpr int kLd = gram_col_stride(kTile);
+  constexpr int kEnt = gram_entries(K);
+  const int prog = a.pair_prog[pair];
+  const int k = a.pt.k[prog];
+  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K)
+  double* cst = s_val + (K + 1) * kLd;
+  double* s_imm = cst + k + 1;
+  const int m_imm = a.pt.imm_off[prog + 1] - a.pt.imm_off[prog];
+  vsr_insn_t* s_insn = reinterpret_cast<vsr_insn_t*>(s_imm + m_imm);
+  int n_insn, n_imm;
+  load_program(a.pt, prog, s_insn, s_imm, n_insn, n_imm);
+  const double* c = a.consts + (int64_t)a.pair_row[pair] * a.kstride;
+  for (int i = tid; i < k; i += kGramThreads) cst[i] = c[i];
+  __syncthreads();
+  for (int i = tid; i < n_insn; i += kGramThreads) s_insn[i] = predecode(s_insn[i]);
+  __syncthreads();
+
+  // the entry this thread owns: 0 = rss, else (ea, eb) of the upper triangle
+  int ea = 0, eb = 0;
+  if (tid > 0 && tid < kEnt) {
+    int t = tid - 1;
+    while (t >= K - ea) t -= K - ea++;
+    eb = ea + t;
+  }
+  const double* col_a = s_val + (tid == 0 ? 0 : 1 + ea) * kLd;
+  const double* col_b = s_val + (tid == 0 ? 0 : 1 + eb) * kLd;
+
+  const int64_t N = a.pts.n;
+  const int64_t tiles = (N + kTile - 1) / kTile;
+  const int64_t per = (tiles + a.nsplit - 1) / a.nsplit;
+  const int64_t n0 = min((int64_t)split * per * kTile, N);
+  const int64_t n1 = min((int64_t)(split + 1) * per * kTile, N);
+  const double* X = static_cast<const double*>(a.pts.X);
+  const double* y = static_cast<const double*>(a.pts.y);
+  Stack<double, K, P> stk;
+  GlobalPoints<double, P> xs;
+  xs.X = X;
+  xs.ldx = a.pts.ldx;
+  double acc = 0.0;
+  for (int64_t base = n0; base < n1; base += kTile) {
+    const int cnt = (int)min((int64_t)kTile, n1 - base);
+#pragma unroll
+    for (int p = 0; p < P; ++p) {
+      const int64_t i = base + (int64_t)p * kGramThreads + tid;
+      xs.idx[p] = i < n1 ? i : (n1 - 1);
+    }
+    Dual<double, K> v[P];
+    eval_points<double, K, P>(s_insn, s_imm, cst, xs, v, stk);
+#pragma unroll
+    for (int p = 0; p < P; ++p) {
+      const int j = p * kGramThreads + tid;  // = point index - base
+      if (j < cnt) {
+        s_val[j] = v[p].v - __ldg(y + xs.idx[p]);
+#pragma unroll
+        for (int t = 0; t < K; ++t) s_val[(1 + t) * kLd + j] = v[p].d[t];
+      }
+    }
+    __syncthreads();
+    if (tid < kEnt)
+      for (int j = 0; j < cnt; ++j) acc = fma(col_a[j], col_b[j], acc);
+    __syncthreads();  // the tile's values may be overwritten
+  }
+  if (tid < kEnt) a.partial[((int64_t)pair * a.nsplit + split) * kEnt + tid] = acc;
+}
+
 #if defined(VSR_API_TU)  // plain kernels: defined once, in the API translation unit
 // out_loss[row] = sum_splits partial / N ; out_grad[row][t] = 2 * sum / N  (t < k, else 0)
 __global__ void eval_finalize(const double* partial, const int32_t* pair_prog,
@@ -1313,6 +1424,40 @@ __global__ void eval_finalize(const double* partial, const int32_t* pair_prog,
     const int t = comp - 1;
     if (t < kstride) out_grad[(int64_t)row * kstride + t] = t < prog_k[pair_prog[pair]] ? 2.0 * acc * inv_n : 0.0;
   }
+}
+
+// out_rss[row] = sum_splits partial[rss]; out_jtj[row][a][b] = sum_splits partial[(min, max)] for a, b < k,
+// splits added in index order (both triangles from the same sum, so the matrix is exactly symmetric).
+// A pair whose program has more constants than the group's width K (k > VSR_MAX_DUAL, value-only
+// group) gets nan for its k x k entries.
+__global__ void gram_finalize(const double* partial, const int32_t* pair_prog, const int32_t* pair_out,
+                              const int32_t* prog_k, int n_pairs, int nsplit, int K, int kstride,
+                              double* out_rss, double* out_jtj) {
+  const int per = 1 + kstride * kstride;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int pair = (int)(idx / per);
+  const int e = (int)(idx - (int64_t)pair * per);
+  if (pair >= n_pairs) return;
+  const int k = prog_k[pair_prog[pair]];
+  const int row = pair_out[pair];
+  const int n_ent = 1 + K * (K + 1) / 2;
+  int ent = 0;
+  if (e > 0) {
+    const int r = (e - 1) / kstride, c = (e - 1) % kstride;
+    if (r >= k || c >= k) return;
+    if (k > K) {
+      out_jtj[((int64_t)row * kstride + r) * kstride + c] = __longlong_as_double(0x7ff8000000000000ll);
+      return;
+    }
+    const int lo = r < c ? r : c, hi = r < c ? c : r;
+    ent = 1 + lo * K - lo * (lo - 1) / 2 + (hi - lo);
+  }
+  double acc = 0.0;
+  for (int s = 0; s < nsplit; ++s) acc += partial[((int64_t)pair * nsplit + s) * n_ent + ent];
+  if (e == 0)
+    out_rss[row] = acc;
+  else
+    out_jtj[((int64_t)row * kstride + (e - 1) / kstride) * kstride + (e - 1) % kstride] = acc;
 }
 
 // fill rows of a [n][kstride] f64 array with nan (gradients of pairs too wide for duals)

@@ -20,6 +20,7 @@ is first copied there and the copy is patched):
                                    stays for CPU tensors; the network and the rest of the beam loop
                                    stay the reference's own code
   scoring.py, hlsc_batch.py added  driver-side scoring / batched HLSC evaluation (optional)
+  uncertainty.py added            covariance / standard errors of fitted constants (optional)
 
 The reference's drivers (``scripts/*_test.py`` through ``scripts/visymre_utils.py``) then run
 unchanged: ``from src.visymre.architectures.model import Model`` still finds the reference's
@@ -108,6 +109,7 @@ def install(checkout, out=None):
     shutil.copy(os.path.join(PKG, "architectures", "bfgs.py"), os.path.join(src, "architectures", "bfgs.py"))
     shutil.copy(os.path.join(PKG, "scoring.py"), os.path.join(src, "scoring.py"))
     shutil.copy(os.path.join(PKG, "hlsc.py"), os.path.join(src, "hlsc_batch.py"))
+    shutil.copy(os.path.join(PKG, "uncertainty.py"), os.path.join(src, "uncertainty.py"))
     # Model.fitfunc2
     mp = os.path.join(src, "architectures", "model.py")
     with open(mp) as fh:

@@ -219,6 +219,34 @@ class Engine:
                                       self._stream()))
         return loss, g
 
+    def gram(self, prog_idx, consts, const_row=None):
+        """Gauss-Newton statistics (``vsr_gram``, fp64 points) of pairs (program prog_idx[p],
+        constants consts[row[p]]).
+
+        Returns device tensors ``rss [n]`` (sum of squared residuals) and ``jtj [n, kstride, kstride]``
+        (J^T J over the program's k constants; entries past k stay nan, and so do all k x k entries of
+        a program with more than ``isa.MAX_DUAL`` constants).
+        """
+        self.ensure_dtype(F64)
+        prog_idx = np.ascontiguousarray(np.asarray(prog_idx, dtype=np.int32))
+        n = int(prog_idx.shape[0])
+        consts = torch.as_tensor(consts, dtype=torch.float64, device=self.device)
+        if consts.dim() == 1:
+            consts = consts.reshape(n, -1) if consts.numel() else consts.reshape(n, 0)
+        if consts.shape[1] == 0:
+            consts = torch.zeros((consts.shape[0], 1), dtype=torch.float64, device=self.device)
+        consts = consts.contiguous()
+        kstride = int(consts.shape[1])
+        rows = None
+        if const_row is not None:
+            rows = np.ascontiguousarray(np.asarray(const_row, dtype=np.int32))
+        rss = torch.empty(n, dtype=torch.float64, device=self.device)
+        jtj = torch.full((n, kstride, kstride), float("nan"), dtype=torch.float64, device=self.device)
+        self._check(self.lib.vsr_gram(self._h, _np_ptr(prog_idx),
+                                      _np_ptr(rows) if rows is not None else ctypes.c_void_p(0),
+                                      n, _ptr(consts), kstride, _ptr(rss), _ptr(jtj), self._stream()))
+        return rss, jtj
+
     def score(self, prog_idx, consts=None, dtype=F64, const_row=None):
         """Driver-side scoring (``vsr_score``): mean squared error of every pair with the
         prediction passed through numpy's ``nan_to_num`` first.  Returns a device tensor [n]."""

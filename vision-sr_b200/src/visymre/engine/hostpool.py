@@ -134,6 +134,19 @@ def format_chunk(job):
     return out
 
 
+def compile_skeletons(job):
+    """[(skeleton string, k)] -> [Program | Exception], variables x_1..x_10 (uncertainty.covariances)."""
+    from .compiler import compile_skeleton
+    variables = [f"x_{i}" for i in range(1, 11)]
+    out = []
+    for expr, k in job:
+        try:
+            out.append(compile_skeleton(expr, k, variables))
+        except Exception as exc:  # noqa: BLE001 -- raised again in the parent
+            out.append(_portable(exc))
+    return out
+
+
 def _portable(exc):
     """Exceptions cross the process boundary by pickle; some (sympy's) do not survive it."""
     import pickle

@@ -1,0 +1,141 @@
+"""Covariance and standard errors of fitted constants, from statistics computed on the device.
+
+``bfgs()`` returns ``(string, consts, loss, skeleton)`` and says nothing about how well the data
+determine the constants.  ``covariances`` answers that for a list of such fits the way
+``scipy.optimize.curve_fit`` does with its default ``absolute_sigma=False``::
+
+    cov = s^2 (J^T J)^-1,   s^2 = rss / (N - k_free),   stderr = sqrt(diag(cov))
+
+with ``J`` the N x k Jacobian of the skeleton in its constants at the fitted point.  The device
+evaluates every point as a dual number whose tangents are a row of ``J``; one ``vsr_gram`` launch
+reduces them to ``rss`` and ``J^T J`` for every fit of the list (``csrc/vsr_kernels.cuh``,
+``gram_kernel``).  Only the k x k matrix comes back to the host, where this module inverts it.
+
+Conventions:
+
+* Free constants.  The reference's prune fixes constants at an exact ``0.0`` (bfgs.py:184-196); the
+  4-tuple returns them as ``0.0`` and they are not fitted, so only the nonzero constants enter the
+  matrix.  Rows and columns of a fixed constant are nan, so is its ``stderr``, and
+  ``dof = N - k_free``.
+* Undeterminable.  When ``dof <= 0``, when ``rss`` or ``J^T J`` holds a nan or inf (the expression
+  is not real at some point), or when ``J^T J`` is numerically rank-deficient, the covariance of the
+  free constants is ``inf``, as curve_fit reports "covariance of the parameters could not be
+  estimated".  Rank-deficient means an eigenvalue ``lambda_i <= max(N, k) * eps * lambda_max``;
+  ``rank`` is the number of eigenvalues above that bound (0 when the Gram holds a non-finite value).
+* The one deviation from curve_fit.  The rank test is on ``J^T J``, which carries half the digits of
+  ``J``: a direction of ``J`` whose singular value is below about ``sqrt(max(N, k) * eps)`` times the
+  largest is called unidentifiable here.  curve_fit, working on ``J`` itself, would keep it, with a
+  variance at least 1e12 times that of the best-determined direction.
+
+The points are taken as given: pass the rows the fit saw (with ``idx_remove``, the kept rows).  A
+skeleton's ``x_j`` reads column j-1 of ``X``, which is the fit's convention (not the drivers'
+by-rank pairing of ``scoring.py``).
+"""
+from dataclasses import dataclass
+
+import numpy as np
+import torch
+
+from .engine import fitter, hostpool
+from .engine.compiler import compile_skeleton
+
+_VARS = [f"x_{i}" for i in range(1, 11)]
+# skeletons compiled in the host pool from this many on (below it the pool's round trip costs more
+# than it saves; see DESIGN.md section 6c)
+POOL_MIN = 16
+
+
+@dataclass
+class ConstantCovariance:
+    """Uncertainty of the constants of one fit (host numpy arrays, k = number of constants)."""
+    consts: np.ndarray   # [k] the fitted constants
+    free: np.ndarray     # [k] bool: False for a constant the prune fixed at 0.0
+    cov: np.ndarray      # [k, k] covariance; nan in rows / columns of fixed constants
+    stderr: np.ndarray   # [k] sqrt(diag(cov))
+    rss: float           # sum of squared residuals at consts
+    dof: int             # N - number of free constants
+    rank: int            # numerical rank of J^T J over the free constants
+    jtj: np.ndarray      # [k, k] J^T J over all constants
+
+
+def covariance_from_gram(rss, jtj, n, free):
+    """``(cov, stderr, dof, rank)`` from the sum of squared residuals, ``J^T J`` ([k, k]), the number
+    of points and the mask of free constants, with curve_fit's conventions (module docstring)."""
+    jtj = np.asarray(jtj, dtype=np.float64)
+    free = np.asarray(free, dtype=bool)
+    k = free.shape[0]
+    kf = int(free.sum())
+    dof = int(n) - kf
+    cov = np.full((k, k), np.nan)
+    rank = 0
+    if kf > 0:
+        sub = jtj[np.ix_(free, free)]
+        cov_f = np.full((kf, kf), np.inf)
+        if np.isfinite(rss) and np.isfinite(sub).all():
+            w, V = np.linalg.eigh(sub)
+            rank = int((w > max(int(n), kf) * np.finfo(np.float64).eps * w.max()).sum())
+            if rank == kf and dof > 0:
+                cov_f = (V / w) @ V.T * (float(rss) / dof)
+                cov_f = 0.5 * (cov_f + cov_f.T)
+        cov[np.ix_(free, free)] = cov_f
+    with np.errstate(invalid="ignore"):
+        stderr = np.sqrt(np.diag(cov))
+    return cov, stderr, dof, rank
+
+
+def _compile(items):
+    """Programs of ``[(skeleton, k)]``, in the host pool when the list is long enough."""
+    pool = hostpool.get_pool(hostpool.default_workers()) if len(items) >= POOL_MIN else None
+    if pool is None:
+        return [compile_skeleton(expr, k, _VARS) for expr, k in items]
+    n = hostpool._POOL_N
+    chunks = [list(range(j, len(items), n)) for j in range(min(n, len(items)))]
+    out = [None] * len(items)
+    for ch, res in zip(chunks, pool.map(hostpool.compile_skeletons, [[items[i] for i in ch] for ch in chunks])):
+        for i, r in zip(ch, res):
+            if isinstance(r, Exception):
+                r = compile_skeleton(items[i][0], items[i][1], _VARS)   # raises here, where it belongs
+            out[i] = r
+    return out
+
+
+def covariances(fits, X, y, engine=None):
+    """Covariance of the constants of every fit of ``fits``.
+
+    ``fits``: ``bfgs()`` / ``bfgs_batch()`` 4-tuples ``(string, consts, loss, skeleton)``; an
+    ``Exception`` or ``None`` in the list gives ``None``.  ``X``: ``[1, N, d]`` or ``[N, d]`` on any
+    device, fp32 or fp64; ``y``: squeezable to ``[N]``.  Returns one ``ConstantCovariance`` (or
+    ``None``) per entry.  The whole list is evaluated with one ``vsr_gram`` call on ``engine`` (default:
+    the process-wide engine of X's device, or of the current CUDA device); its points and programs are
+    replaced.
+    """
+    X = torch.as_tensor(X)
+    if X.dim() == 3:
+        X = X[0]
+    y = torch.as_tensor(y).reshape(-1)
+    out = [None] * len(fits)
+    items = []
+    for i, f in enumerate(fits):
+        if f is None or isinstance(f, Exception):
+            continue
+        items.append((i, str(f[3]), np.asarray(f[1], dtype=np.float64).reshape(-1)))
+    if not items:
+        return out
+    progs = _compile([(skel, c.shape[0]) for _, skel, c in items])
+    eng = engine if engine is not None else fitter.get_engine(X.device if X.is_cuda else None)
+    eng.set_points(X, y, dtypes=(fitter.F64,), n_vars=max(1, max(p.var_mask.bit_length() for p in progs)))
+    eng.set_programs(progs)
+    consts = np.zeros((len(items), max(1, max(c.shape[0] for _, _, c in items))))
+    for j, (_, _, c) in enumerate(items):
+        consts[j, :c.shape[0]] = c
+    rss, jtj = eng.gram(np.arange(len(items)), torch.from_numpy(consts))
+    rss, jtj = rss.cpu().numpy(), jtj.cpu().numpy()
+    n = int(X.shape[0])
+    for j, (i, _, c) in enumerate(items):
+        k = c.shape[0]
+        free = c != 0.0
+        g = jtj[j, :k, :k].copy()
+        cov, stderr, dof, rank = covariance_from_gram(rss[j], g, n, free)
+        out[i] = ConstantCovariance(consts=c, free=free, cov=cov, stderr=stderr, rss=float(rss[j]),
+                                    dof=dof, rank=rank, jtj=g)
+    return out
