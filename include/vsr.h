@@ -121,6 +121,18 @@ int vsr_score(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row,
 int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, int32_t n_pairs,
              const double* consts, int32_t kstride, double* out_rss, double* out_jtj, void* stream);
 
+/* Per-point values, and optionally delta-method variances, of n_pairs (program, constants) pairs
+ * over all points of the `dtype` slot:
+ *   out_value[p][i] = f_{prog[p]}(x_i; consts[row[p]])                       (nan / inf allowed)
+ *   out_var[p][i]   = g_i^T cov[row[p]] g_i,  g_i = d f / d c at x_i        (f64 arithmetic)
+ * cov [rows][kstride][kstride] f64 device, entries a, b < k read; cov == NULL <=> out_var == NULL.
+ * Outputs are f64 device arrays with row stride ld_out >= n_points.  y is not read.
+ * Programs with k > VSR_MAX_DUAL: out_var row nan.  A pair's outputs do not depend on the other
+ * pairs of the call, bit for bit. */
+int vsr_predict(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, int32_t n_pairs,
+                const double* consts, int32_t kstride, const double* cov, int32_t dtype,
+                double* out_value, double* out_var, int64_t ld_out, void* stream);
+
 /* Multi-restart BFGS for n_runs (program, restart) runs; run r of the list fits program
  * run_prog[r] from x0[run_slot[r]] and writes every output at row run_slot[r]
  * (slots let a rank fit a shard of a C x R problem in place).  run_prog and run_slot

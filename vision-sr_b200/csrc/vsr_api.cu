@@ -244,6 +244,16 @@ cudaError_t launch_eval_tile(int K, const vsr::EvalTileArgs& a, size_t smem, cud
   return cudaErrorInvalidValue;
 }
 
+template <typename T>
+cudaError_t launch_predict(int K, const vsr::PredictArgs& a, size_t smem, cudaStream_t st) {
+  switch (K) {
+#define C(KK) case KK: return vsr::launch_predict_T<T, KK>(a, smem, st);
+    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
+#undef C
+  }
+  return cudaErrorInvalidValue;
+}
+
 cudaError_t launch_gram(int K, const vsr::GramArgs& a, size_t smem, cudaStream_t st) {
   switch (K) {
 #define C(KK) case KK: return vsr::launch_gram_K<KK>(a, smem, st);
@@ -909,6 +919,82 @@ int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, i
     VSR_CUDA(h, cudaGetLastError());
     h->launches += 2;
     partial += (size_t)n * a.nsplit * vsr::gram_entries(K);
+  }
+  return VSR_OK;
+}
+
+int vsr_predict(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, int32_t n_pairs,
+                const double* consts, int32_t kstride, const double* cov, int32_t dtype,
+                double* out_value, double* out_var, int64_t ld_out, void* stream) {
+  int rc = check_ready(h, dtype);
+  if (rc) return rc;
+  const PointSlot& ps = h->pts[dtype];
+  if (!prog_idx || n_pairs <= 0 || !out_value || kstride < 0 || (!consts && kstride > 0) ||
+      (!cov) != (!out_var) || ld_out < ps.n)
+    return fail(h, VSR_EINVAL, "bad predict arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  VSR_CUDA(h, cudaSetDevice(h->device));
+  // group pairs by tangent width; without a covariance, and for programs wider than VSR_MAX_DUAL,
+  // the width-0 group (values only; its variance row is 0 for k == 0 and nan otherwise)
+  std::vector<Group> groups(kNumWidths);
+  std::vector<std::vector<int32_t>> outs(kNumWidths);
+  for (int i = 0; i < kNumWidths; ++i) groups[i].K = kWidths[i];
+  for (int p = 0; p < n_pairs; ++p) {
+    const int c = prog_idx[p];
+    if (c < 0 || c >= h->n_programs) return fail(h, VSR_EINVAL, "pair %d: program %d out of range", p, c);
+    const int k = h->h_k[c];
+    if (k > kstride) return fail(h, VSR_EINVAL, "pair %d: %d constants > kstride %d", p, k, kstride);
+    if ((rc = check_vars(h, c, dtype))) return rc;
+    const int w = out_var ? pick_width(k) : 0;
+    const int gi = w < 0 ? 0 : (int)(std::find(kWidths, kWidths + kNumWidths, w) - kWidths);
+    Group& g = groups[gi];
+    g.prog.push_back(c);
+    g.slot.push_back(const_row ? const_row[p] : p);
+    g.kmax = std::max(g.kmax, k);
+    g.max_insn = std::max(g.max_insn, h->h_ninsn[c]);
+    g.max_imm = std::max(g.max_imm, h->h_nimm[c]);
+    outs[gi].push_back(p);
+  }
+  std::vector<int32_t> all;
+  std::vector<size_t> off(kNumWidths, 0);
+  for (int gi = 0; gi < kNumWidths; ++gi) {
+    off[gi] = all.size();
+    all.insert(all.end(), groups[gi].prog.begin(), groups[gi].prog.end());
+    all.insert(all.end(), groups[gi].slot.begin(), groups[gi].slot.end());
+    all.insert(all.end(), outs[gi].begin(), outs[gi].end());
+  }
+  rc = stage_lists(h, all, st);
+  if (rc) return rc;
+  const int32_t* dl = (const int32_t*)h->d_lists.p;
+  for (int gi = 0; gi < kNumWidths; ++gi) {
+    const Group& g = groups[gi];
+    const int n = (int)g.prog.size();
+    if (!n) continue;
+    const int K = g.K;
+    const int64_t tile = (int64_t)vsr::kPredictThreads * points_per_thread(K);
+    const int64_t tiles = (ps.n + tile - 1) / tile;
+    // splits of the points: enough CTAs to fill the machine several times over (no result depends
+    // on this choice)
+    const int64_t want = ((int64_t)h->num_sms * 32 + n - 1) / n;
+    vsr::PredictArgs a;
+    a.pt = table_of(h);
+    a.pts = points_of(ps);
+    a.pair_prog = dl + off[gi];
+    a.pair_row = dl + off[gi] + n;
+    a.pair_out = dl + off[gi] + 2 * n;
+    a.n_pairs = n;
+    a.kstride = kstride;
+    a.consts = consts;
+    a.cov = cov;
+    a.out_value = out_value;
+    a.out_var = out_var;
+    a.ld_out = ld_out;
+    a.nsplit = (int)std::max<int64_t>(1, std::min<int64_t>({want, tiles, 65535}));
+    const size_t smem = sizeof(double) * ((size_t)K * K + g.kmax + 1 + g.max_imm) +
+                        sizeof(vsr_insn_t) * (g.max_insn + 1);
+    cudaError_t e = dtype == VSR_F64 ? launch_predict<double>(K, a, smem, st) : launch_predict<float>(K, a, smem, st);
+    if (e != cudaSuccess) return fail(h, VSR_ECUDA, "predict kernel launch failed: %s", cudaGetErrorString(e));
+    h->launches += 1;
   }
   return VSR_OK;
 }

@@ -1,4 +1,4 @@
-// vsr_inst.cu -- one instantiation of fit_kernel / eval_kernel and their launch wrappers:
+// vsr_inst.cu -- one instantiation of fit_kernel / eval_kernel / predict_kernel and their launch wrappers:
 // compiled once per (VSR_INST_T, VSR_INST_K) pair, see the Makefile.  The double units
 // (VSR_INST_GRAM) also hold gram_kernel of their width.
 #include <algorithm>
@@ -93,6 +93,12 @@ cudaError_t launch_eval_tile_T(const EvalTileArgs& a, size_t smem, cudaStream_t 
   return cudaGetLastError();
 }
 
+template <typename T, int K>
+cudaError_t launch_predict_T(const PredictArgs& a, size_t smem, cudaStream_t st) {
+  predict_kernel<T, K, points_per_thread(K)><<<dim3(a.n_pairs, a.nsplit), kPredictThreads, smem, st>>>(a);
+  return cudaGetLastError();
+}
+
 #if defined(VSR_INST_GRAM)
 template <int K>
 cudaError_t launch_gram_K(const GramArgs& a, size_t smem, cudaStream_t st) {
@@ -115,5 +121,6 @@ template cudaError_t preload_T<VSR_INST_T, VSR_INST_K>();
 template cudaError_t launch_fit_T<VSR_INST_T, VSR_INST_K>(const FitArgs&, int, int, size_t, int, cudaStream_t);
 template cudaError_t launch_eval_T<VSR_INST_T, VSR_INST_K>(const EvalArgs&, int, size_t, cudaStream_t);
 template cudaError_t launch_eval_tile_T<VSR_INST_T, VSR_INST_K>(const EvalTileArgs&, size_t, cudaStream_t);
+template cudaError_t launch_predict_T<VSR_INST_T, VSR_INST_K>(const PredictArgs&, size_t, cudaStream_t);
 
 }  // namespace vsr

@@ -14,6 +14,8 @@
 //   eval_finalize       deterministic fixed-order sum of the split partials.
 //   gram_kernel<K,P>    fp64 sum r^2 and J^T J of (program, constants) pairs (Gauss-Newton statistics
 //                       for the covariance of fitted constants); gram_finalize sums its splits.
+//   predict_kernel<T,K,P> per-point values of (program, constants) pairs and, with a covariance, the
+//                       fp64 delta-method variance g^T C g of each point (prediction bands).
 //
 // Work mapping: lanes stride over points (coalesced column reads), P points per thread
 // share one instruction decode; per-thread partial sums are fp64 and parked in shared memory, then
@@ -1402,6 +1404,114 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const GramArgs a) {
     __syncthreads();  // the tile's values may be overwritten
   }
   if (tid < kEnt) a.partial[((int64_t)pair * a.nsplit + split) * kEnt + tid] = acc;
+}
+
+// ---- per-point values and delta-method variances of (program, constants) pairs ---------------------
+// For each pair and every point i of the slot of T:
+//   out_value[row][i] = f(x_i; c)                     stored as f64; numpy's semantics, no nan_to_num
+//   out_var[row][i]   = sum_a sum_b g_a C_ab g_b       g = d f / d c at x_i, C the pair's k x k block
+// The variance is fp64 whatever T (the tangents are widened first) and runs over a, then b, in index
+// order.  The grid is (pairs x point splits) like eval_kernel's; thread tid handles point
+// base + p * kPredictThreads + tid of each tile, so a warp's stores are coalesced.  Nothing is summed
+// across points, so a point's outputs depend only on its program, constants, covariance and the point:
+// not on the grid or on the other pairs of the call.  Width 0 serves the value-only pairs; with
+// out_var it writes 0 for k == 0 and nan for k > VSR_MAX_DUAL (no tangents).  All offsets are int64.
+struct PredictArgs {
+  ProgramTable pt;
+  Points pts;                // the slot of T
+  const int32_t* pair_prog;  // [n_pairs]
+  const int32_t* pair_row;   // [n_pairs] row of `consts` and of `cov`
+  const int32_t* pair_out;   // [n_pairs] row of the outputs
+  int32_t n_pairs;
+  int32_t kstride;
+  const double* consts;  // [rows][kstride]
+  const double* cov;     // [rows][kstride][kstride]; nullptr iff out_var is
+  double* out_value;     // [..][ld_out]
+  double* out_var;       // [..][ld_out] or nullptr
+  int64_t ld_out;
+  int32_t nsplit;
+};
+
+constexpr int kPredictThreads = 256;
+
+// dynamic shared memory of predict_kernel, in doubles: cov[K * K] | cst[k] | imm | insn
+template <typename T, int K, int P>
+__global__ void __launch_bounds__(kPredictThreads) predict_kernel(const PredictArgs a) {
+  extern __shared__ double smem[];
+  const int pair = blockIdx.x;
+  const int split = blockIdx.y;
+  const int tid = threadIdx.x;
+  constexpr int kTile = kPredictThreads * P;
+  const int prog = a.pair_prog[pair];
+  const int k = a.pt.k[prog];
+  const int64_t row = a.pair_row[pair];
+  double* s_cov = smem;  // [K][K], zero past k
+  T* cst = reinterpret_cast<T*>(s_cov + K * K);
+  double* s_imm = s_cov + K * K + k + 1;
+  const int m_imm = a.pt.imm_off[prog + 1] - a.pt.imm_off[prog];
+  vsr_insn_t* s_insn = reinterpret_cast<vsr_insn_t*>(s_imm + m_imm);
+  int n_insn, n_imm;
+  load_program(a.pt, prog, s_insn, s_imm, n_insn, n_imm);
+  const double* c = a.consts + row * a.kstride;
+  for (int i = tid; i < k; i += kPredictThreads) cst[i] = (T)c[i];
+  if (K > 0) {
+    const double* C = a.cov + row * a.kstride * a.kstride;
+    for (int e = tid; e < K * K; e += kPredictThreads) {
+      const int r = e / (K > 0 ? K : 1), q = e - r * K;
+      s_cov[e] = (r < k && q < k) ? C[(int64_t)r * a.kstride + q] : 0.0;
+    }
+  }
+  __syncthreads();
+  for (int i = tid; i < n_insn; i += kPredictThreads) s_insn[i] = predecode(s_insn[i]);
+  __syncthreads();
+
+  const int64_t N = a.pts.n;
+  const int64_t tiles = (N + kTile - 1) / kTile;
+  const int64_t per = (tiles + a.nsplit - 1) / a.nsplit;
+  const int64_t n0 = min((int64_t)split * per * kTile, N);
+  const int64_t n1 = min((int64_t)(split + 1) * per * kTile, N);
+  const int64_t out_row = (int64_t)a.pair_out[pair] * a.ld_out;
+  double* val = a.out_value + out_row;
+  double* var = a.out_var ? a.out_var + out_row : nullptr;
+  // value-only pairs with a variance row: none to carry (k == 0) or no tangents for it (k > K)
+  const double var0 = k == 0 ? 0.0 : __longlong_as_double(0x7ff8000000000000ll);
+  Stack<T, K, P> stk;
+  GlobalPoints<T, P> xs;
+  xs.X = static_cast<const T*>(a.pts.X);
+  xs.ldx = a.pts.ldx;
+  for (int64_t base = n0; base < n1; base += kTile) {
+#pragma unroll
+    for (int p = 0; p < P; ++p) {
+      const int64_t i = base + (int64_t)p * kPredictThreads + tid;
+      xs.idx[p] = i < n1 ? i : (n1 - 1);
+    }
+    Dual<T, K> v[P];
+    eval_points<T, K, P>(s_insn, s_imm, cst, xs, v, stk);
+#pragma unroll
+    for (int p = 0; p < P; ++p) {
+      const int64_t i = base + (int64_t)p * kPredictThreads + tid;
+      if (i >= n1) continue;
+      val[i] = (double)v[p].v;
+      if (K > 0) {
+        // tangents past the program's k are not constants of it: they are 0 unless an overflow made
+        // them nan (inf * 0 in a product rule), which must not reach the form through C's zero padding
+        double g[K > 0 ? K : 1];
+#pragma unroll
+        for (int t = 0; t < K; ++t) g[t] = t < k ? (double)v[p].d[t] : 0.0;
+        double q = 0.0;
+#pragma unroll
+        for (int r = 0; r < K; ++r) {
+          double cg = 0.0;
+#pragma unroll
+          for (int t = 0; t < K; ++t) cg = fma(s_cov[r * K + t], g[t], cg);
+          q = fma(g[r], cg, q);
+        }
+        var[i] = q;
+      } else if (var) {
+        var[i] = var0;
+      }
+    }
+  }
 }
 
 #if defined(VSR_API_TU)  // plain kernels: defined once, in the API translation unit

@@ -23,6 +23,10 @@ cudaError_t launch_eval_T(const EvalArgs& a, int threads, size_t smem, cudaStrea
 template <typename T, int K>
 cudaError_t launch_eval_tile_T(const EvalTileArgs& a, size_t smem, cudaStream_t st);
 
+// per-point values and variances (predict_kernel)
+template <typename T, int K>
+cudaError_t launch_predict_T(const PredictArgs& a, size_t smem, cudaStream_t st);
+
 // Gauss-Newton statistics (gram_kernel, fp64 only): compiled in the double translation units
 template <int K>
 cudaError_t launch_gram_K(const GramArgs& a, size_t smem, cudaStream_t st);

@@ -247,6 +247,51 @@ class Engine:
                                       n, _ptr(consts), kstride, _ptr(rss), _ptr(jtj), self._stream()))
         return rss, jtj
 
+    def predict(self, prog_idx, consts, cov=None, dtype=F64, const_row=None):
+        """Per-point values (``vsr_predict``) of pairs (program prog_idx[p], constants consts[row[p]])
+        over the points of ``dtype``, and with ``cov`` ([rows, k, k] f64, read for a, b < k of each
+        program) the delta-method variance ``g^T cov[row[p]] g`` of every point, g = d f / d c.
+
+        Returns device f64 tensors ``value [n, N]`` (nan / inf where numpy gives them) and ``var [n, N]``
+        (None without ``cov``; 0 for programs without constants, nan for programs with more than
+        ``isa.MAX_DUAL`` constants).
+        """
+        self.ensure_dtype(dtype)
+        prog_idx = np.ascontiguousarray(np.asarray(prog_idx, dtype=np.int32))
+        n = int(prog_idx.shape[0])
+        consts = torch.as_tensor(consts, dtype=torch.float64, device=self.device)
+        if consts.dim() == 1:
+            consts = consts.reshape(n, -1) if consts.numel() else consts.reshape(n, 0)
+        if consts.shape[1] == 0:
+            consts = torch.zeros((consts.shape[0], 1), dtype=torch.float64, device=self.device)
+        consts = consts.contiguous()
+        kstride = int(consts.shape[1])
+        n_rows = int(consts.shape[0])
+        if cov is not None:
+            cov = torch.as_tensor(cov, dtype=torch.float64, device=self.device)
+            kc = int(cov.shape[-1]) if cov.dim() == 3 else -1
+            # a pair reads row const_row[p] of consts and of cov alike
+            if kc < 0 or kc > kstride or tuple(cov.shape) != (n_rows, kc, kc):
+                raise ValueError(f"cov {tuple(cov.shape)} does not match consts {tuple(consts.shape)}")
+            if kc < kstride:
+                cov = torch.nn.functional.pad(cov, (0, kstride - kc, 0, kstride - kc))
+            cov = cov.contiguous()
+        rows = None
+        if const_row is not None:
+            rows = np.ascontiguousarray(np.asarray(const_row, dtype=np.int32))
+            if rows.shape != (n,) or (n and (rows.min() < 0 or rows.max() >= n_rows)):
+                raise ValueError(f"const_row must hold {n} rows in [0, {n_rows})")
+        elif n_rows < n:
+            raise ValueError(f"{n} pairs but {n_rows} rows of constants")
+        N = self.n_points
+        value = torch.empty((n, N), dtype=torch.float64, device=self.device)
+        var = torch.empty((n, N), dtype=torch.float64, device=self.device) if cov is not None else None
+        self._check(self.lib.vsr_predict(self._h, _np_ptr(prog_idx),
+                                         _np_ptr(rows) if rows is not None else ctypes.c_void_p(0),
+                                         n, _ptr(consts), kstride, _ptr(cov), dtype, _ptr(value), _ptr(var),
+                                         N, self._stream()))
+        return value, var
+
     def score(self, prog_idx, consts=None, dtype=F64, const_row=None):
         """Driver-side scoring (``vsr_score``): mean squared error of every pair with the
         prediction passed through numpy's ``nan_to_num`` first.  Returns a device tensor [n]."""

@@ -66,6 +66,8 @@ SIGNATURES = {
     "vsr_score": (ctypes.c_int, [vp, vp, vp, ctypes.c_int32, vp, ctypes.c_int32, ctypes.c_int32,
                                  vp, vp]),
     "vsr_gram": (ctypes.c_int, [vp, vp, vp, ctypes.c_int32, vp, ctypes.c_int32, vp, vp, vp]),
+    "vsr_predict": (ctypes.c_int, [vp, vp, vp, ctypes.c_int32, vp, ctypes.c_int32, vp, ctypes.c_int32,
+                                   vp, vp, ctypes.c_int64, vp]),
     "vsr_fit": (ctypes.c_int, [vp, vp, vp, ctypes.c_int32, vp, ctypes.c_int32,
                                ctypes.POINTER(FitOpts), vp, vp, vp, vp, vp, vp]),
     "vsr_fit_host": (ctypes.c_int, [vp, vp, vp, ctypes.c_int32, ctypes.c_int32, vp,

@@ -30,10 +30,21 @@ Conventions:
 The points are taken as given: pass the rows the fit saw (with ``idx_remove``, the kept rows).  A
 skeleton's ``x_j`` reads column j-1 of ``X``, which is the fit's convention (not the drivers'
 by-rank pairing of ``scoring.py``).
+
+``predict`` evaluates fitted expressions at new points, and with the covariances gives the
+delta-method confidence band of the mean and prediction band of a new observation at each point::
+
+    se_fit(x)^2 = g(x)^T cov g(x),   g(x) = d f(x; c) / d c at the fitted c
+    f(x) +- t se_fit(x),   f(x) +- t sqrt(se_fit(x)^2 + s^2),   t = t_{dof}((1 + level) / 2)
+
+One ``vsr_predict`` launch writes ``f`` and ``g^T cov g`` of every point for every fit of the list
+(``csrc/vsr_kernels.cuh``, ``predict_kernel``); ``bands`` assembles the rest on the device.
 """
 from dataclasses import dataclass
+from typing import Optional
 
 import numpy as np
+import scipy.stats
 import torch
 
 from .engine import fitter, hostpool
@@ -138,4 +149,116 @@ def covariances(fits, X, y, engine=None):
         cov, stderr, dof, rank = covariance_from_gram(rss[j], g, n, free)
         out[i] = ConstantCovariance(consts=c, free=free, cov=cov, stderr=stderr, rss=float(rss[j]),
                                     dof=dof, rank=rank, jtj=g)
+    return out
+
+
+@dataclass
+class Prediction:
+    """A fitted expression at N points: device float64 tensors ``[N]``.  Without a covariance only
+    ``value`` and ``level`` are set; the other fields are ``None``."""
+    value: torch.Tensor                # f(x; c)
+    se_fit: Optional[torch.Tensor]     # sqrt(max(g^T cov g, 0))
+    ci_low: Optional[torch.Tensor]     # value -+ t se_fit: confidence band of the mean
+    ci_high: Optional[torch.Tensor]
+    pi_low: Optional[torch.Tensor]     # value -+ t sqrt(se_fit^2 + s^2): prediction band of a new y
+    pi_high: Optional[torch.Tensor]
+    level: float
+    t: Optional[float]                 # Student's t quantile at (1 + level) / 2 with dof degrees of freedom
+    dof: Optional[int]
+
+
+def device_cov(cov):
+    """The covariance ``vsr_predict`` reads: the nan rows and columns of constants the prune fixed at
+    ``0.0`` become 0 (they carry no variance).  An ``inf`` (undeterminable) covariance becomes all 0:
+    ``bands`` does not read the variance of such a fit."""
+    cov = np.array(cov, dtype=np.float64)
+    cov[np.isnan(cov)] = 0.0
+    if np.isinf(cov).any():
+        cov[:] = 0.0
+    return cov
+
+
+def bands(value, var, cov, rss, dof, level=0.95):
+    """``Prediction`` from the values ``[N]`` and variances ``g^T cov g`` ``[N]`` of one fit (tensors
+    on any device), its covariance (host, as ``covariances`` gives it), ``rss`` and ``dof``.
+
+    ``s^2 = rss / dof`` and ``t = scipy.stats.t.ppf((1 + level) / 2, dof)``.  ``se_fit =
+    sqrt(max(var, 0))``: from a positive semidefinite ``cov`` in fp64 ``var`` is below 0 only by
+    rounding.  When the covariance could not be determined (an ``inf`` in ``cov``, or ``dof <= 0``)
+    ``se_fit`` is ``inf`` and every band is infinite.  A nan value (``f`` not real at the point) gives
+    nan bands.
+    """
+    if not 0.0 < level < 1.0:
+        raise ValueError(f"level {level} is not in (0, 1)")
+    value = torch.as_tensor(value, dtype=torch.float64)
+    var = torch.as_tensor(var, dtype=torch.float64, device=value.device)
+    dof = int(dof)
+    t = float(scipy.stats.t.ppf((1.0 + level) / 2.0, dof)) if dof > 0 else float("nan")
+    if dof > 0 and not np.isinf(np.asarray(cov, dtype=np.float64)).any():
+        se_fit = torch.sqrt(torch.clamp(var, min=0.0))
+        half_ci = t * se_fit
+        half_pi = t * torch.sqrt(se_fit * se_fit + float(rss) / dof)
+    else:
+        se_fit = torch.full_like(value, float("inf"))
+        half_ci = half_pi = se_fit
+    return Prediction(value=value, se_fit=se_fit, ci_low=value - half_ci, ci_high=value + half_ci,
+                      pi_low=value - half_pi, pi_high=value + half_pi, level=float(level), t=t, dof=dof)
+
+
+def predict(fits, X_new, covs=None, level=0.95, engine=None, dtype=None):
+    """Values of every fit of ``fits`` at the points ``X_new``, and with ``covs`` their confidence and
+    prediction bands.
+
+    ``fits``: ``bfgs()`` / ``bfgs_batch()`` 4-tuples ``(string, consts, loss, skeleton)``; an
+    ``Exception`` or ``None`` in the list gives ``None``.  ``X_new``: ``[N, d]`` or ``[1, N, d]`` on any
+    device; ``x_j`` reads column j-1, as in ``covariances``.  ``covs``: the list ``covariances(fits,
+    X_train, y_train)`` returned (without it only ``value`` is computed).  ``dtype``: arithmetic of the
+    sweep, ``fitter.F64`` or ``fitter.F32``; by default fp32 for fp32 points and fp64 otherwise, as the
+    fit's final score.  Returns one ``Prediction`` (or ``None``) per entry, with device float64 tensors
+    on the engine's device.
+
+    The whole list is one ``vsr_predict`` call on ``engine`` (default: the process-wide engine of X's
+    device, or of the current CUDA device); its points and programs are replaced.  Conventions (see
+    ``bands`` for the rest): constants the prune fixed at ``0.0`` carry no variance; the variance is
+    always fp64 arithmetic; a value is numpy's (nan where ``f`` is not real, +-inf on overflow); a fit
+    with more than ``isa.MAX_DUAL`` constants gets nan variances.
+    """
+    X = torch.as_tensor(X_new)
+    if X.dim() == 3:
+        X = X[0]
+    if covs is not None and len(covs) != len(fits):
+        raise ValueError(f"{len(covs)} covariances for {len(fits)} fits")
+    out = [None] * len(fits)
+    items = []
+    for i, f in enumerate(fits):
+        if f is None or isinstance(f, Exception):
+            continue
+        if covs is not None and covs[i] is None:
+            raise ValueError(f"fit {i} has no covariance")
+        items.append((i, str(f[3]), np.asarray(f[1], dtype=np.float64).reshape(-1)))
+    if not items:
+        return out
+    dt = dtype if dtype is not None else (fitter.F32 if X.dtype == torch.float32 else fitter.F64)
+    progs = _compile([(skel, c.shape[0]) for _, skel, c in items])
+    eng = engine if engine is not None else fitter.get_engine(X.device if X.is_cuda else None)
+    eng.set_points(X, torch.zeros(X.shape[0], dtype=torch.float64), dtypes=(dt,),
+                   n_vars=max(1, max(p.var_mask.bit_length() for p in progs)))
+    eng.set_programs(progs)
+    kmax = max(1, max(c.shape[0] for _, _, c in items))
+    consts = np.zeros((len(items), kmax))
+    cov = np.zeros((len(items), kmax, kmax)) if covs is not None else None
+    for j, (i, _, c) in enumerate(items):
+        k = c.shape[0]
+        consts[j, :k] = c
+        if cov is not None:
+            cov[j, :k, :k] = device_cov(covs[i].cov)
+    value, var = eng.predict(np.arange(len(items)), torch.from_numpy(consts),
+                             cov=torch.from_numpy(cov) if cov is not None else None, dtype=dt)
+    for j, (i, _, _) in enumerate(items):
+        if cov is None:
+            out[i] = Prediction(value=value[j], se_fit=None, ci_low=None, ci_high=None, pi_low=None,
+                                pi_high=None, level=float(level), t=None, dof=None)
+        else:
+            cv = covs[i]
+            out[i] = bands(value[j], var[j], cv.cov, cv.rss, cv.dof, level)
     return out
