@@ -71,6 +71,34 @@ std::vector<vsr_insn_t> predecoded(const vsr_insn_t* prog) {
   return out;
 }
 
+// value and K tangents of every point; out_tangents is row-major [N][K]
+template <typename T, int K>
+void duals(const vsr_insn_t* prog, const double* imm, const double* c, int k, const T* X, long N,
+           double* out_value, double* out_tangents) {
+  T cst[VSR_MAX_CONSTS];
+  for (int i = 0; i < k; ++i) cst[i] = (T)c[i];
+  vsr::Stack<T, K, 1> stk;
+  HostX<T> xs{X, N, 0};
+  for (long i = 0; i < N; ++i) {
+    xs.i = i;
+    vsr::Dual<T, K> acc[1];
+    vsr::eval_points<T, K, 1>(prog, imm, cst, xs, acc, stk);
+    out_value[i] = (double)acc[0].v;
+    for (int t = 0; t < K; ++t) out_tangents[i * K + t] = (double)acc[0].d[t];
+  }
+}
+
+template <typename T>
+int duals_dispatch(int K, const vsr_insn_t* prog, const double* imm, const double* c, int k,
+                   const T* X, long N, double* v, double* d) {
+  switch (K) {
+#define C(KK) case KK: duals<T, KK>(prog, imm, c, k, X, N, v, d); return 0;
+    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
+#undef C
+  }
+  return -1;
+}
+
 int pick_K(int k) {
   static const int ks[] = {0, 1, 2, 3, 4, 6, 8, 12, 16};
   for (int v : ks)
@@ -114,6 +142,19 @@ int hostsim_values(const vsr_insn_t* raw_prog, const double* imm, const double* 
   }
   return 0;
 }
+
+// value and all K tangents of every point, K one of the kernels' widths (0..8, 12, 16);
+// out_tangents is [N][K] (untouched for K = 0).  For the per-opcode edge-of-domain tests.
+int hostsim_duals(const vsr_insn_t* raw_prog, const double* imm, const double* c, int k,
+                  const void* X, long N, int dtype, int K, double* out_value, double* out_tangents) {
+  const std::vector<vsr_insn_t> pd = predecoded(raw_prog);
+  if (dtype == VSR_F64)
+    return duals_dispatch<double>(K, pd.data(), imm, c, k, (const double*)X, N, out_value, out_tangents);
+  return duals_dispatch<float>(K, pd.data(), imm, c, k, (const float*)X, N, out_value, out_tangents);
+}
+
+// the handler id the interpreter dispatches `word` to (vsr::predecode)
+int hostsim_predecode(vsr_insn_t word) { return (int)VSR_HANDLER(vsr::predecode(word)); }
 
 // mean squared residual and its gradient w.r.t. the constants (dual numbers)
 int hostsim_loss_grad(const vsr_insn_t* raw_prog, const double* imm, const double* c, int k,

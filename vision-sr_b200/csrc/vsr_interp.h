@@ -56,20 +56,30 @@ VSR_M1(VSR_MATH, m_tanh, ::tanh, ::tanhf)
 #undef VSR_M1
 VSR_MATH double m_pow(double a, double b) { return ::pow(a, b); }
 VSR_MATH float m_pow(float a, float b) { return ::powf(a, b); }
-// a**b together with ln(a) for a > 0: exp(b ln a).  libm's pow carries ln(a) in
-// double-double (~250 instructions in fp64); here the relative error of the result is
-// |b ln a| ulp of ln plus an ulp of exp, i.e. at most ~1.6e-13 (|b ln a| <= 709), inside the
-// 1e-12 budget, and the tangent rules need ln(a) anyway.  Non-positive bases keep libm's
-// exact special cases.
+// a**b together with ln(a): exp(b ln a) for a > 0.  libm's pow carries ln(a) in double-double
+// (~250 instructions in fp64); here ln a within L_log ulp and the rounding of b ln a put
+// (2 L_log + 1) |b ln a| units of roundoff into the result, plus exp's own error: at most 2.4e-13
+// relative in fp64 (|b ln a| < 708), inside the 1e-12 budget, and the tangent rules need ln(a)
+// anyway.  libm's pow keeps its exact special cases: non-positive bases, 1**b, a**0 (exp(0 * ln a)
+// is nan at a = inf), and |b ln a| from 708 (87 in fp32) on, where the result is next to overflow
+// or underflow and exp(b ln a) could land on the other side of the threshold from the value-only
+// path.
 template <typename T>
 VSR_HD T m_pow_log(T a, T b, T& lna) {
-  if (a > T(0)) {
-    lna = m_log(a);
-    if (a == T(1)) return T(1);
-    return m_exp(b * lna);
-  }
   lna = m_log(a);  // -inf at 0, nan below
+  if (a > T(0) && a != T(1) && b != T(0)) {
+    const T t = b * lna;
+    if (m_abs(t) < (sizeof(T) == 8 ? T(708) : T(87))) return m_exp(t);
+  }
   return m_pow(a, b);
+}
+// d(a**b)/da = b f / a for a != 0, f = a**b: b (f / a), or (b f) / a where f / a overflows but the
+// derivative does not (a subnormal base and |b| < 1)
+template <typename T>
+VSR_HD T m_pow_grad(T a, T b, T f) {
+  const T big = sizeof(T) == 8 ? (T)1.7976931348623157e308 : (T)3.4028234663852886e38;
+  const T g = b * (f / a);
+  return (m_abs(g) > big && m_abs(f) <= big) ? (b * f) / a : g;
 }
 VSR_MATH void m_sincos(double x, double* s, double* c) {
 #if defined(__CUDA_ARCH__)
@@ -183,14 +193,16 @@ VSR_HD void unary_apply(Dual<T, K>& x, unsigned am, int n) {
       f = m_tan(a);
       fp = T(1) + f * f;
       break;
+    // 1 - a^2 as (1 - a)(1 + a): 1 - a is exact for |a| >= 1/2, so the factor keeps its digits
+    // next to +-1 where 1 - a*a cancels
     case VSR_ASIN:
       f = m_asin(a);
-      if (live) fp = T(1) / m_sqrt(T(1) - a * a);
+      if (live) fp = T(1) / m_sqrt((T(1) - a) * (T(1) + a));
       guard = true;
       break;
     case VSR_ACOS:
       f = m_acos(a);
-      if (live) fp = T(-1) / m_sqrt(T(1) - a * a);
+      if (live) fp = T(-1) / m_sqrt((T(1) - a) * (T(1) + a));
       guard = true;
       break;
     case VSR_ATAN:
@@ -207,7 +219,13 @@ VSR_HD void unary_apply(Dual<T, K>& x, unsigned am, int n) {
       break;
     case VSR_TANH:
       f = m_tanh(a);
-      fp = T(1) - f * f;
+      // sech^2 a = 4e / (1 + e)^2 with e = exp(-2|a|): no cancellation, and it decays smoothly
+      // to 0 in saturation where 1 - tanh^2 rounds to exactly 0
+      if (live) {
+        const T e = m_exp(T(-2) * m_abs(a));
+        const T d = T(1) + e;
+        fp = (T(4) * e) / (d * d);
+      }
       break;
     case VSR_POWI: {
       const int m = n < 0 ? -n : n;
@@ -399,8 +417,9 @@ VSR_HD void binary_apply(Dual<T, K> (&acc)[P], Stack<T, K, P>& stk, int& sp, uns
         const T f = (K == 0) ? m_pow(a, bv) : m_pow_log(a, bv, lna);
         if (K > 0 && lm) {
           // d/da = b a^(b-1) = b f / a (one division instead of a second pow; pow again
-          // only at a == 0);  d/db = f ln a  (0 where a == 0 and the power vanishes)
-          const T fa = am ? (a != T(0) ? bv * (f / a) : bv * m_pow(a, bv - T(1))) : T(0);
+          // only at a == 0; 0 at b == 0, where f / a may overflow);  d/db = f ln a  (0 where
+          // a == 0 and the power vanishes)
+          const T fa = am ? (bv == T(0) ? T(0) : a != T(0) ? m_pow_grad(a, bv, f) : bv * m_pow(a, bv - T(1))) : T(0);
           T fb = T(0);
           if (bm) fb = (a == T(0) && f == T(0)) ? T(0) : f * lna;
 #pragma unroll
@@ -417,7 +436,7 @@ VSR_HD void binary_apply(Dual<T, K> (&acc)[P], Stack<T, K, P>& stk, int& sp, uns
         if (K > 0 && lm) {
           T fa = T(0);
           if (am) fa = (bv == T(0) && f == T(0)) ? T(0) : f * lnb;
-          const T fb = bm ? (bv != T(0) ? a * (f / bv) : a * m_pow(bv, a - T(1))) : T(0);
+          const T fb = bm ? (a == T(0) ? T(0) : bv != T(0) ? m_pow_grad(bv, a, f) : a * m_pow(bv, a - T(1))) : T(0);
 #pragma unroll
           for (int i = 0; i < K; ++i)
             if ((lm >> i) & 1u) x.d[i] = m_scale(x.d[i], fa) + m_scale((T)VSR_TB(i), fb);
