@@ -77,6 +77,16 @@ int vsr_set_points(vsr_handle* h, const void* X_dev, const void* y_dev, int64_t 
 int vsr_upload_points(vsr_handle* h, const void* X_host, const void* y_host, int64_t n_points,
                       int64_t ldx, int32_t n_vars, int32_t dtype, void* stream);
 
+/* Per-point weights of the points in slot `dtype` (w_i > 0, finite, n_points = the slot's N).  Caller-owned
+ * device memory, kept like vsr_set_points' pointers; NULL clears.  vsr_set_points / vsr_upload_points of that
+ * slot clear it.  Read by vsr_fit (optimiser sweeps and the per-restart final MSE), vsr_eval (loss and
+ * gradient) and vsr_gram (the F64 slot's weights: out_rss = sum w r^2, out_jtj = J^T W J).  Not read by
+ * vsr_score (the drivers' unweighted R^2) or vsr_predict (reads neither y nor w).  With weights, the loss of
+ * a fit and of vsr_eval is loss_scale * (1/N) sum_i w_i (f(x_i; c) - y_i)^2; w_i = 1 gives the unweighted
+ * results bit for bit.  The elements are of the slot's type, like y.  VSR_EINVAL: n_points is not the
+ * slot's N; VSR_ESTATE: the slot has no points. */
+int vsr_set_weights(vsr_handle* h, const void* w_dev, int64_t n_points, int32_t dtype);
+
 /* Programs.  Replaces sp.lambdify of the N-term loss, once per restart (bfgs.py:104)
  * and of the fitted expression (bfgs.py:128).  HOST arrays: instruction words of all
  * C programs back to back, insn_off[C+1], literal pools back to back, imm_off[C+1],

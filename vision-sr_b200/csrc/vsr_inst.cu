@@ -1,16 +1,19 @@
 // vsr_inst.cu -- one instantiation of fit_kernel / eval_kernel / predict_kernel and their launch wrappers:
 // compiled once per (VSR_INST_T, VSR_INST_K) pair, see the Makefile.  The double units
-// (VSR_INST_GRAM) also hold gram_kernel of their width.
+// (VSR_INST_GRAM) also hold gram_kernel of their width.  fit, eval, eval_tile and gram kernels come in an
+// unweighted (W = false) and a weighted (W = true) instantiation; a wrapper launches the weighted one
+// when it is given the slot's weights (w != nullptr).
 #include <algorithm>
 
 #include "vsr_launch.h"
 
 namespace vsr {
 
-template <typename T, int K>
-cudaError_t launch_fit_T(const FitArgs& a, int threads, int cs, size_t smem, int clusters, cudaStream_t st) {
+template <typename T, int K, bool W>
+static cudaError_t launch_fit_TW(const Weighted<FitArgs, W>& a, int threads, int cs, size_t smem, int clusters,
+                                 cudaStream_t st) {
   constexpr int P = points_per_thread(K);
-  auto kern = fit_kernel<T, K, P>;
+  auto kern = fit_kernel<T, K, P, W>;
   if (threads > fit_max_threads<T, K>()) return cudaErrorInvalidConfiguration;
   // function attributes and the occupancy answer are cached per instantiation: they are driver
   // calls, and vsr_fit launches up to eleven groups per call
@@ -68,18 +71,32 @@ cudaError_t launch_fit_T(const FitArgs& a, int threads, int cs, size_t smem, int
 }
 
 template <typename T, int K>
-cudaError_t launch_eval_T(const EvalArgs& a, int threads, size_t smem, cudaStream_t st) {
-  constexpr int P = points_per_thread(K);
-  auto kern = eval_kernel<T, K, P>;
-  dim3 grid(a.n_pairs, a.nsplit);
-  kern<<<grid, threads, smem, st>>>(a);
-  return cudaGetLastError();
+cudaError_t launch_fit_T(const FitArgs& a, int threads, int cs, size_t smem, int clusters, cudaStream_t st,
+                         const void* w) {
+  if (!w) return launch_fit_TW<T, K, false>(Weighted<FitArgs, false>{a}, threads, cs, smem, clusters, st);
+  Weighted<FitArgs, true> aw{a};
+  aw.w = w;
+  return launch_fit_TW<T, K, true>(aw, threads, cs, smem, clusters, st);
 }
 
 template <typename T, int K>
-cudaError_t launch_eval_tile_T(const EvalTileArgs& a, size_t smem, cudaStream_t st) {
+cudaError_t launch_eval_T(const EvalArgs& a, int threads, size_t smem, cudaStream_t st, const void* w) {
   constexpr int P = points_per_thread(K);
-  auto kern = eval_tile_kernel<T, K, P>;
+  dim3 grid(a.n_pairs, a.nsplit);
+  if (!w) {
+    eval_kernel<T, K, P, false><<<grid, threads, smem, st>>>(Weighted<EvalArgs, false>{a});
+  } else {
+    Weighted<EvalArgs, true> aw{a};
+    aw.w = w;
+    eval_kernel<T, K, P, true><<<grid, threads, smem, st>>>(aw);
+  }
+  return cudaGetLastError();
+}
+
+template <typename T, int K, bool W>
+static cudaError_t launch_eval_tile_TW(const Weighted<EvalTileArgs, W>& a, size_t smem, cudaStream_t st) {
+  constexpr int P = points_per_thread(K);
+  auto kern = eval_tile_kernel<T, K, P, W>;
   static size_t smem_limit[32] = {0};
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
@@ -94,6 +111,14 @@ cudaError_t launch_eval_tile_T(const EvalTileArgs& a, size_t smem, cudaStream_t 
 }
 
 template <typename T, int K>
+cudaError_t launch_eval_tile_T(const EvalTileArgs& a, size_t smem, cudaStream_t st, const void* w) {
+  if (!w) return launch_eval_tile_TW<T, K, false>(Weighted<EvalTileArgs, false>{a}, smem, st);
+  Weighted<EvalTileArgs, true> aw{a};
+  aw.w = w;
+  return launch_eval_tile_TW<T, K, true>(aw, smem, st);
+}
+
+template <typename T, int K>
 cudaError_t launch_predict_T(const PredictArgs& a, size_t smem, cudaStream_t st) {
   predict_kernel<T, K, points_per_thread(K)><<<dim3(a.n_pairs, a.nsplit), kPredictThreads, smem, st>>>(a);
   return cudaGetLastError();
@@ -101,26 +126,35 @@ cudaError_t launch_predict_T(const PredictArgs& a, size_t smem, cudaStream_t st)
 
 #if defined(VSR_INST_GRAM)
 template <int K>
-cudaError_t launch_gram_K(const GramArgs& a, size_t smem, cudaStream_t st) {
-  gram_kernel<K, points_per_thread(K)><<<dim3(a.n_pairs, a.nsplit), kGramThreads, smem, st>>>(a);
+cudaError_t launch_gram_K(const GramArgs& a, size_t smem, cudaStream_t st, const void* w) {
+  const dim3 grid(a.n_pairs, a.nsplit);
+  if (!w) {
+    gram_kernel<K, points_per_thread(K), false><<<grid, kGramThreads, smem, st>>>(Weighted<GramArgs, false>{a});
+  } else {
+    Weighted<GramArgs, true> aw{a};
+    aw.w = w;
+    gram_kernel<K, points_per_thread(K), true><<<grid, kGramThreads, smem, st>>>(aw);
+  }
   return cudaGetLastError();
 }
-template cudaError_t launch_gram_K<VSR_INST_K>(const GramArgs&, size_t, cudaStream_t);
+template cudaError_t launch_gram_K<VSR_INST_K>(const GramArgs&, size_t, cudaStream_t, const void*);
 #endif
 
 template <typename T, int K>
 cudaError_t preload_T() {
   constexpr int P = points_per_thread(K);
   cudaFuncAttributes attr;
-  cudaError_t e = cudaFuncGetAttributes(&attr, fit_kernel<T, K, P>);
+  cudaError_t e = cudaFuncGetAttributes(&attr, fit_kernel<T, K, P, false>);
   if (e != cudaSuccess) return e;
-  return cudaFuncGetAttributes(&attr, eval_kernel<T, K, P>);
+  return cudaFuncGetAttributes(&attr, eval_kernel<T, K, P, false>);
 }
 
 template cudaError_t preload_T<VSR_INST_T, VSR_INST_K>();
-template cudaError_t launch_fit_T<VSR_INST_T, VSR_INST_K>(const FitArgs&, int, int, size_t, int, cudaStream_t);
-template cudaError_t launch_eval_T<VSR_INST_T, VSR_INST_K>(const EvalArgs&, int, size_t, cudaStream_t);
-template cudaError_t launch_eval_tile_T<VSR_INST_T, VSR_INST_K>(const EvalTileArgs&, size_t, cudaStream_t);
+template cudaError_t launch_fit_T<VSR_INST_T, VSR_INST_K>(const FitArgs&, int, int, size_t, int, cudaStream_t,
+                                                          const void*);
+template cudaError_t launch_eval_T<VSR_INST_T, VSR_INST_K>(const EvalArgs&, int, size_t, cudaStream_t, const void*);
+template cudaError_t launch_eval_tile_T<VSR_INST_T, VSR_INST_K>(const EvalTileArgs&, size_t, cudaStream_t,
+                                                                const void*);
 template cudaError_t launch_predict_T<VSR_INST_T, VSR_INST_K>(const PredictArgs&, size_t, cudaStream_t);
 
 }  // namespace vsr

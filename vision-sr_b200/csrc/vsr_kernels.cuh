@@ -128,6 +128,16 @@ struct EvalArgs {
   int32_t nan_to_num;  // 1: predictions pass through numpy's nan_to_num before the residual (vsr_score)
 };
 
+// Kernel arguments of a weighted launch (W = true): the argument struct A with the per-point weights
+// w_i of the slot (the slot's element type, like y) as its LAST member, so that every member of A keeps
+// its parameter offset.  Weighted<A, false> is A itself: the unweighted kernels are unchanged.
+template <typename A, bool W>
+struct Weighted : A {
+  const void* w;
+};
+template <typename A>
+struct Weighted<A, false> : A {};
+
 // ---- point source: coalesced global loads (read-only path) --------------------------
 template <typename T, int P>
 struct GlobalPoints {
@@ -157,11 +167,14 @@ __device__ __forceinline__ void keep_in_register(int& v) { asm volatile("" : "+r
 // converged for the reduction that follows.
 // NTN: the prediction passes through numpy's nan_to_num (nan -> 0, +-inf -> +-largest finite
 // value of T) before the residual is taken: the drivers' scoring rule (Feynman_test.py:87).
-template <typename T, int K, int P, bool NTN = false>
+// W: per-point weights w (fp64 arithmetic): sum w r^2 and sum w r df/dc_t.  rw = w * r is formed once and
+// every product is the unweighted one with r replaced by rw, so w = 1.0 gives the unweighted sums bit for bit.
+template <typename T, int K, int P, bool NTN = false, bool W = false>
 __device__ __forceinline__ void sweep_points(const vsr_insn_t* prog, const double* imm,
                                              const T* cst, const T* __restrict__ X,
                                              const T* __restrict__ y, int64_t ldx, int64_t n0,
-                                             int64_t n1, double* scratch, int tid, int nt) {
+                                             int64_t n1, double* scratch, int tid, int nt,
+                                             const T* __restrict__ w = nullptr) {
   // tid / nt: index of this thread among the nt threads that take part in the sweep
   Stack<T, K, P> stk;
   GlobalPoints<T, P> xs;
@@ -190,13 +203,23 @@ __device__ __forceinline__ void sweep_points(const vsr_insn_t* prog, const doubl
           pv = pv != pv ? T(0) : (pv > big ? big : (pv < -big ? -big : pv));
         }
         const double r = (double)pv - (double)__ldg(y + xs.idx[p]);
-        ps += r * r;
+        if constexpr (W) {
+          const double rw = (double)__ldg(w + xs.idx[p]) * r;
+          ps += rw * r;
 #pragma unroll
-        for (int t = 0; t < K; ++t) {
-          const double gt = r * (double)acc[p].d[t];
-          // a tangent that blew up where the value stayed finite (exp(-exp(x)) ...) counts 0
-          // (one compare and a predicated add; nan fails the compare)
-          if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+          for (int t = 0; t < K; ++t) {
+            const double gt = rw * (double)acc[p].d[t];
+            if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+          }
+        } else {
+          ps += r * r;
+#pragma unroll
+          for (int t = 0; t < K; ++t) {
+            const double gt = r * (double)acc[p].d[t];
+            // a tangent that blew up where the value stayed finite (exp(-exp(x)) ...) counts 0
+            // (one compare and a predicated add; nan fails the compare)
+            if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+          }
         }
       }
     }
@@ -354,10 +377,11 @@ struct SlicePoints {
 };
 
 // One pass over the resident slice (cnt points); partial sums parked like sweep_points does.
-template <typename T, int K, int P, bool NTN = false>
+// W: the weights are staged like y (ws, cnt values), same residual rule as sweep_points.
+template <typename T, int K, int P, bool NTN = false, bool W = false>
 __device__ __forceinline__ void sweep_slice(const vsr_insn_t* prog, const double* imm, const T* cst,
                                             const T* xs, const T* ys, int stride, int cnt, double* scratch,
-                                            int tid, int nt) {
+                                            int tid, int nt, const T* ws = nullptr) {
   Stack<T, K, P> stk;
   SlicePoints<T, P> src;
   src.base = xs;
@@ -386,11 +410,21 @@ __device__ __forceinline__ void sweep_slice(const vsr_insn_t* prog, const double
           pv = pv != pv ? T(0) : (pv > big ? big : (pv < -big ? -big : pv));
         }
         const double r = (double)pv - (double)ys[src.idx[p]];
-        ps += r * r;
+        if constexpr (W) {
+          const double rw = (double)ws[src.idx[p]] * r;
+          ps += rw * r;
 #pragma unroll
-        for (int t = 0; t < K; ++t) {
-          const double gt = r * (double)acc[p].d[t];
-          if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+          for (int t = 0; t < K; ++t) {
+            const double gt = rw * (double)acc[p].d[t];
+            if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+          }
+        } else {
+          ps += r * r;
+#pragma unroll
+          for (int t = 0; t < K; ++t) {
+            const double gt = r * (double)acc[p].d[t];
+            if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+          }
         }
       }
     }
@@ -507,7 +541,7 @@ __device__ __forceinline__ void warp_totals(const double* scratch, int stid, int
 // dynamic shared memory (doubles):
 //   per seat [ FitState | ws | cred[cs*(K+1)] | ctrl (16 B) | cst | imm | insn ]
 //   then wpart [seats][warps][K+1], the per-thread scratch [(K+1)][threads], then the slice
-//   (n_cols + 1) * stride * sizeof(T).
+//   (n_cols + 1) * stride * sizeof(T), one column more in a weighted launch (the weights, after X's).
 // FitState / ws / cred are used in the leader CTA only; the layout is the same in every CTA so that
 // one offset addresses the same thing cluster-wide (mapa).
 constexpr int kFitStateDoubles = (int)((sizeof(FitState) + 15) / 16 * 2);
@@ -924,8 +958,11 @@ __device__ __forceinline__ bool seat_turn(const FitArgs& a, int lane, int cs, Fi
   return my_prog >= 0;
 }
 
-template <typename T, int K, int P>
-__global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>())) fit_kernel(const FitArgs a) {
+// W: weighted launch (a.w: per-point weights of the slot of T); a resident slice stages the weight
+// column after the n_cols columns of X.
+template <typename T, int K, int P, bool W>
+__global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>()))
+    fit_kernel(const Weighted<FitArgs, W> a) {
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   extern __shared__ __align__(16) double smem[];
@@ -995,16 +1032,22 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
     const bool use_tma = a.tma_ok && full > 0;
     if (tid == 0 && use_tma) {
       const uint32_t bytes = (uint32_t)full * (uint32_t)sizeof(T);
-      mbar_expect_tx(&s_bar, bytes * (uint32_t)(a.n_cols + 1));
+      mbar_expect_tx(&s_bar, bytes * (uint32_t)(a.n_cols + 1 + (W ? 1 : 0)));
       tma_bulk_load(ys, y + n0, bytes, &s_bar);
       for (int j = 0; j < VSR_MAX_VARS; ++j)
         if (a.col_of_var[j] >= 0)
           tma_bulk_load(xs + (size_t)a.col_of_var[j] * stride, X + (int64_t)j * a.pts.ldx + n0, bytes, &s_bar);
+      if constexpr (W)
+        tma_bulk_load(xs + (size_t)a.n_cols * stride, static_cast<const T*>(a.w) + n0, bytes, &s_bar);
     }
     {
       // everything TMA does not move (all of it when the caller's memory is unaligned): coalesced loads
       const int first = use_tma ? full : 0;
       for (int i = first + tid; i < cnt; i += blockDim.x) ys[i] = y[n0 + i];
+      if constexpr (W) {
+        T* wsl = xs + (size_t)a.n_cols * stride;
+        for (int i = first + tid; i < cnt; i += blockDim.x) wsl[i] = static_cast<const T*>(a.w)[n0 + i];
+      }
       for (int j = 0; j < VSR_MAX_VARS; ++j) {
         const int sj = a.col_of_var[j];
         if (sj < 0) continue;
@@ -1098,10 +1141,19 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
         if (c.prog < 0) {  // the seat is closed
           live &= ~(1u << g);
         } else {
-          if (a.resident)
-            sweep_slice<T, K, P>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt);
-          else
-            sweep_points<T, K, P>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid, snt);
+          if constexpr (W) {
+            if (a.resident)
+              sweep_slice<T, K, P, false, true>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
+                                                xs + (size_t)a.n_cols * stride);
+            else
+              sweep_points<T, K, P, false, true>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid, snt,
+                                                 static_cast<const T*>(a.w));
+          } else {
+            if (a.resident)
+              sweep_slice<T, K, P>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt);
+            else
+              sweep_points<T, K, P>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid, snt);
+          }
           double* mine = wpart + ((size_t)g * nw + warp) * (K + 1);
           warp_totals<K>(scratch, stid, snt, lane, mine);
           __syncwarp();
@@ -1133,8 +1185,9 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
 }
 
 // dynamic shared memory of eval_kernel, in doubles: red[(K+1)*threads] | cst[k] | imm | insn
-template <typename T, int K, int P>
-__global__ void __launch_bounds__(256) eval_kernel(const EvalArgs a) {
+// W: weighted sums (a.w, read from global memory like y)
+template <typename T, int K, int P, bool W>
+__global__ void __launch_bounds__(256) eval_kernel(const Weighted<EvalArgs, W> a) {
   extern __shared__ double smem[];
   const int pair = blockIdx.x;
   const int split = blockIdx.y;
@@ -1166,7 +1219,11 @@ __global__ void __launch_bounds__(256) eval_kernel(const EvalArgs a) {
   n0 = n0 < N ? n0 : N;
   n1 = n1 < N ? n1 : N;
 
-  if (K == 0 && a.nan_to_num)  // scoring rule of the drivers, value only
+  if constexpr (W)  // (vsr_score, the nan_to_num rule, is never weighted)
+    sweep_points<T, K, P, false, true>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
+                                       static_cast<const T*>(a.pts.y), a.pts.ldx, n0, n1, red, (int)threadIdx.x,
+                                       (int)blockDim.x, static_cast<const T*>(a.w));
+  else if (K == 0 && a.nan_to_num)  // scoring rule of the drivers, value only
     sweep_points<T, K, P, true>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
                                 static_cast<const T*>(a.pts.y), a.pts.ldx, n0, n1, red, (int)threadIdx.x,
                                 (int)blockDim.x);
@@ -1207,8 +1264,11 @@ __host__ __device__ inline size_t eval_tile_fixed_doubles(int K, int threads, in
   return (d + 1) & ~(size_t)1;
 }
 
-template <typename T, int K, int P>
-__global__ void __launch_bounds__((eval_tile_threads<K>()), 1) eval_tile_kernel(const EvalTileArgs a) {
+// W: weighted sums.  The weights are read from global memory (a.w, like y in eval_kernel), not staged: the
+// chunks are those of the unweighted launch, so the partial sums are formed in the same order and w = 1
+// gives the unweighted result bit for bit.
+template <typename T, int K, int P, bool W>
+__global__ void __launch_bounds__((eval_tile_threads<K>()), 1) eval_tile_kernel(const Weighted<EvalTileArgs, W> a) {
   extern __shared__ __align__(16) double smem[];
   __shared__ __align__(8) uint64_t s_bar;
   const int tid = threadIdx.x, nt = blockDim.x;
@@ -1288,7 +1348,10 @@ __global__ void __launch_bounds__((eval_tile_threads<K>()), 1) eval_tile_kernel(
     commit();
     __syncthreads();
     if (pair + 1 < a.e.n_pairs) fetch(pair + 1);
-    if (K == 0 && a.e.nan_to_num)
+    if constexpr (W)
+      sweep_slice<T, K, P, false, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
+                                        static_cast<const T*>(a.w) + n0);
+    else if (K == 0 && a.e.nan_to_num)
       sweep_slice<T, K, P, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt);
     else
       sweep_slice<T, K, P>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt);
@@ -1334,8 +1397,10 @@ __host__ __device__ inline int gram_nsplit(int64_t N, int64_t tile) {
 __host__ __device__ constexpr int gram_col_stride(int tile) { return tile + 1; }
 
 // dynamic shared memory of gram_kernel, in doubles: tile[(K+1) * gram_col_stride] | cst[k] | imm | insn
-template <int K, int P>
-__global__ void __launch_bounds__(kGramThreads) gram_kernel(const GramArgs a) {
+// W: weighted sums rss = sum w r^2, jtj[a][b] = sum w J_a J_b (J^T W J).  The tile gets one column more, the
+// weights, and every term is fma(col_a * w, col_b, acc): w = 1.0 gives the unweighted sums bit for bit.
+template <int K, int P, bool W>
+__global__ void __launch_bounds__(kGramThreads) gram_kernel(const Weighted<GramArgs, W> a) {
   extern __shared__ double smem[];
   const int pair = blockIdx.x;
   const int split = blockIdx.y;
@@ -1345,8 +1410,8 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const GramArgs a) {
   constexpr int kEnt = gram_entries(K);
   const int prog = a.pair_prog[pair];
   const int k = a.pt.k[prog];
-  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K)
-  double* cst = s_val + (K + 1) * kLd;
+  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K) (then w when W)
+  double* cst = s_val + (K + 1 + (W ? 1 : 0)) * kLd;
   double* s_imm = cst + k + 1;
   const int m_imm = a.pt.imm_off[prog + 1] - a.pt.imm_off[prog];
   vsr_insn_t* s_insn = reinterpret_cast<vsr_insn_t*>(s_imm + m_imm);
@@ -1396,11 +1461,18 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const GramArgs a) {
         s_val[j] = v[p].v - __ldg(y + xs.idx[p]);
 #pragma unroll
         for (int t = 0; t < K; ++t) s_val[(1 + t) * kLd + j] = v[p].d[t];
+        if constexpr (W) s_val[(K + 1) * kLd + j] = __ldg(static_cast<const double*>(a.w) + xs.idx[p]);
       }
     }
     __syncthreads();
-    if (tid < kEnt)
-      for (int j = 0; j < cnt; ++j) acc = fma(col_a[j], col_b[j], acc);
+    if constexpr (W) {
+      const double* col_w = s_val + (K + 1) * kLd;
+      if (tid < kEnt)
+        for (int j = 0; j < cnt; ++j) acc = fma(col_a[j] * col_w[j], col_b[j], acc);
+    } else {
+      if (tid < kEnt)
+        for (int j = 0; j < cnt; ++j) acc = fma(col_a[j], col_b[j], acc);
+    }
     __syncthreads();  // the tile's values may be overwritten
   }
   if (tid < kEnt) a.partial[((int64_t)pair * a.nsplit + split) * kEnt + tid] = acc;

@@ -497,8 +497,31 @@ def _format_all(jobs, cfg):
     return out
 
 
-def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False):
+def sigma_weights(sigma, X, cfg):
+    """Weights ``1 / sigma**2`` of a fit of points ``X`` (``[1, N, d]`` or ``[N, d]``) under ``cfg``, checked
+    in every point dtype the fit uses (``fitter.weights_from_sigma``); ``None`` without ``sigma``.  Raises
+    ``ValueError`` for a bad ``sigma`` and for ``sigma`` with ``cfg.bfgs.idx_remove``: the reference pairs
+    the kept rows with the first ``y``s (bfgs.py:78-82), so no pairing of the weights would mean anything."""
+    if sigma is None:
+        return None
+    if _opt(cfg, "idx_remove", False):
+        raise ValueError("sigma cannot be combined with cfg.bfgs.idx_remove")
+    Xt = torch.as_tensor(X)
+    n = int(Xt.shape[-2])
+    score_dtype = fitter.F32 if Xt.dtype == torch.float32 else fitter.F64
+    eval_dtype = fitter.F32 if str(_opt(cfg, "precision", "fp64")).lower() == "fp32" else fitter.F64
+    return fitter.weights_from_sigma(sigma, n, {eval_dtype, score_dtype, fitter.F64})
+
+
+def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False, sigma=None):
     """Fit every candidate of a beam in one go (see ``_bfgs_batch``).
+
+    ``sigma``: optional 1-D array of N per-point standard deviations (any device), as
+    ``scipy.optimize.curve_fit`` takes it: every fit then minimises ``loss_scale * mean(w r^2)`` with
+    ``w = 1 / sigma**2``, and the returned loss, the per-restart score that picks the restart and the
+    prune's acceptance are weighted.  ``ValueError`` for a wrong length, a sigma that is not finite and
+    > 0, a ``1/sigma**2`` that is not a finite normal number in a point dtype of the fit, or ``sigma`` with
+    ``cfg.bfgs.idx_remove``.  With a process group every rank passes its own ``sigma``, like ``X``, ``y``.
 
     With ``cfg.bfgs.collapse_duplicates`` (off by default; SURVEY 8f row 4) candidates that
     compile to the SAME bytecode -- beams that differ only in ways sympy canonicalises away,
@@ -508,8 +531,9 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     duplicate sees, not what a fit computes.
     """
     pred_strs = list(pred_strs)
+    w = sigma_weights(sigma, X, cfg)
     if not _opt(cfg, "collapse_duplicates", False) or len(pred_strs) < 2:
-        return _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=x0, engine=engine, lazy_strings=lazy_strings)
+        return _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=x0, engine=engine, lazy_strings=lazy_strings, w=w)
     variables = list(test_data.total_variables)
     first, rep_of, own_expr = {}, [], []
     for i, toks in enumerate(pred_strs):
@@ -523,7 +547,8 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     reps = sorted(set(rep_of))
     pos = {r: j for j, r in enumerate(reps)}
     sub = _bfgs_batch([pred_strs[r] for r in reps], X, y, cfg, test_data,
-                      x0=None if x0 is None else [x0[r] for r in reps], engine=engine, lazy_strings=lazy_strings)
+                      x0=None if x0 is None else [x0[r] for r in reps], engine=engine, lazy_strings=lazy_strings,
+                      w=w)
     out = []
     for i, r in enumerate(rep_of):
         res = sub[pos[r]]
@@ -533,7 +558,7 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     return out
 
 
-def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False):
+def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False, w=None):
     """Fit every candidate of a beam in one go.
 
     Returns a list with one entry per candidate: the reference's 4-tuple
@@ -541,7 +566,8 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
     ``bfgs()`` would have raised for it.  ``x0``: optional list (one per candidate) of
     ``[R, k]`` starting points; default is the reference's ``np.random.randn(k) * 10``
     per restart (bfgs.py:103).  ``lazy_strings``: ``best_expr_str`` of every candidate is a
-    ``LazyStr`` (printed through sympy when read) instead of a ``str``.
+    ``LazyStr`` (printed through sympy when read) instead of a ``str``.  ``w``: per-point weights
+    (``sigma_weights``) or ``None``.
     """
     import time as _time
     _t = [_time.perf_counter()]
@@ -599,7 +625,7 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
         devices[0] if devices else (Xt.device if Xt.is_cuda else None))
     score_dtype = fitter.F32 if Xt.dtype == torch.float32 else fitter.F64
     eval_dtype = fitter.F32 if str(_opt(cfg, "precision", "fp64")).lower() == "fp32" else fitter.F64
-    eng.set_points(Xt[0], yt_fit, dtypes=tuple({eval_dtype, score_dtype, fitter.F64}))
+    eng.set_points(Xt[0], yt_fit, dtypes=tuple({eval_dtype, score_dtype, fitter.F64}), w=w)
     opts = _engine_opts(cfg, scale, eval_dtype, score_dtype)
     main_stream = torch.cuda.current_stream(eng.device)
     points_ready = torch.cuda.Event()
@@ -867,10 +893,11 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
     return results
 
 
-def bfgs(pred_str, X, y, cfg, test_data, x0=None, engine=None):
-    """Reference signature (bfgs.py:42): one candidate, raises what the reference raises."""
+def bfgs(pred_str, X, y, cfg, test_data, x0=None, engine=None, sigma=None):
+    """Reference signature (bfgs.py:42): one candidate, raises what the reference raises.  ``sigma``: see
+    ``bfgs_batch``."""
     out = bfgs_batch([pred_str], X, y, cfg, test_data,
-                     x0=None if x0 is None else [x0], engine=engine)[0]
+                     x0=None if x0 is None else [x0], engine=engine, sigma=sigma)[0]
     if isinstance(out, Exception):
         raise out
     return out

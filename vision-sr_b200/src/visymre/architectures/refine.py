@@ -16,7 +16,7 @@ repo's own package ``architectures/model.py`` re-exports it under the reference'
 import numpy as np
 import torch
 
-from .bfgs import LazyStrings, bfgs, bfgs_batch, resolve_devices
+from .bfgs import LazyStrings, bfgs, bfgs_batch, resolve_devices, sigma_weights
 
 UNARY_NAMES = ("abs", "asin", "cos", "exp", "ln", "sin", "sqrt", "tan")   # model.py:295
 BINARY_NAMES = ("add", "div", "mul", "pow", "sub")                        # model.py:296
@@ -74,7 +74,7 @@ def _as_list(ww):
     return list(ww)
 
 
-def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None):
+def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None, sigma=None):
     """The "BFGS Parallel Part" of fitfunc2 (model.py:444-520).
 
     ``hyps``: ``generated_hyps.hyp``, a list of ``(score, tokens)``; ``X`` ``[1, N, 10]``
@@ -82,7 +82,9 @@ def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None):
     output dict.  Candidates come back in beam order (the reference's order is process
     completion order, which is not reproducible).  ``cfg_params.bfgs.devices`` spreads the fit
     over several GPUs of this process (``bfgs.resolve_devices``); an invalid value raises
-    ``ValueError`` here instead of failing every candidate.
+    ``ValueError`` here instead of failing every candidate.  ``sigma``: per-point standard deviations
+    of ``y`` (1-D, N entries, any device) for weighted fits, see ``bfgs.bfgs_batch``; a bad ``sigma``
+    raises ``ValueError`` here as well.
     """
     w2i = test_data.word2id
     arity_1 = {w2i[n] for n in UNARY_NAMES if n in w2i}
@@ -113,8 +115,10 @@ def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None):
     P_bfgs, L_bfgs, token = [], [], []
     if valid:
         resolve_devices(cfg_params)     # a wrong cfg.bfgs.devices is the caller's error, not every candidate's
+        sigma_weights(sigma, X, cfg_params)   # so is a wrong sigma
         try:
-            outs = bfgs_batch(valid, X, y, cfg_params, test_data, x0=x0, engine=engine, lazy_strings=True)
+            outs = bfgs_batch(valid, X, y, cfg_params, test_data, x0=x0, engine=engine, lazy_strings=True,
+                              sigma=sigma)
         except Exception as exc:  # noqa: BLE001 -- a batch-level failure fails every candidate
             outs = [exc] * len(valid)
         P_bfgs = LazyStrings()   # every string the reference returns; printed when read

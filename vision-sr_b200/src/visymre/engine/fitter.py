@@ -34,6 +34,29 @@ class FitResult:
     info: torch.Tensor       # [n_slots, 4] int32: status, nit, nfev, 0
 
 
+def weights_from_sigma(sigma, n, dtypes):
+    """Per-point weights ``w = 1 / sigma**2`` (fp64 tensor on sigma's device) of a 1-D ``sigma`` of length
+    ``n``, as ``scipy.optimize.curve_fit`` takes it.  Raises ``ValueError`` when ``sigma`` has the wrong
+    shape, holds a value that is not finite or not > 0, or when ``w`` is not a finite normal number in
+    every point dtype of ``dtypes`` (an fp32 slot can overflow or underflow)."""
+    s = torch.as_tensor(sigma, dtype=torch.float64)
+    if s.dim() != 1 or int(s.shape[0]) != int(n):
+        raise ValueError(f"sigma must be 1-D with {n} entries, got shape {tuple(s.shape)}")
+    if not bool((torch.isfinite(s) & (s > 0)).all()):
+        raise ValueError("every sigma must be finite and > 0")
+    w = 1.0 / (s * s)
+    _check_weights(w, dtypes)
+    return w
+
+
+def _check_weights(w, dtypes):
+    for dt in dtypes:
+        td = _TORCH_DTYPE[dt]
+        wd = w.to(td)
+        if not bool((torch.isfinite(wd) & (wd >= torch.finfo(td).tiny)).all()):
+            raise ValueError(f"a weight 1/sigma^2 is not a finite normal {td} number at every point")
+
+
 def default_opts(**over):
     lib = native.load()
     o = native.FitOpts()
@@ -60,7 +83,9 @@ class Engine:
         if rc != 0:
             raise native.VsrError(f"vsr_create failed ({rc}): {self.lib.vsr_last_error(None).decode()}")
         self._points = {}      # dtype -> (Xc [d, ld], y [N]) tensors kept alive
+        self._weights = {}     # dtype -> w [N] tensor kept alive (weighted points only)
         self._src = None       # (X2d, y1d) as given, for re-uploads with more columns
+        self._w_src = None     # fp64 weights as given (None: unweighted)
         self.n_points = 0
         self.n_vars = 0
         self.programs = []
@@ -110,11 +135,14 @@ class Engine:
         return tuple(out)
 
     # ---- points ----------------------------------------------------------------------
-    def set_points(self, X, y, dtypes=(F64,), n_vars=None):
+    def set_points(self, X, y, dtypes=(F64,), n_vars=None, w=None):
         """X: [N, d] (or [1, N, d]) tensor/array on any device; y: squeezable to [N].
 
         Columns are stored column-major on the device, one copy per requested dtype.
         Trailing all-zero columns are not stored unless a program reads them.
+        ``w``: optional per-point weights [N] (``vsr_set_weights``), stored in every dtype slot; the fit,
+        ``eval`` and ``gram`` then use ``sum w r^2``.  ``ValueError`` when a weight is not a finite normal
+        number > 0 in a requested dtype.
         """
         X = torch.as_tensor(X)
         y = torch.as_tensor(y)
@@ -127,7 +155,14 @@ class Engine:
             X = X[:, :isa.MAX_VARS]
         X = X.to(self.device, non_blocking=True)
         y = y.to(self.device, non_blocking=True)
+        if w is not None:
+            w = torch.as_tensor(w, dtype=torch.float64).reshape(-1)
+            if int(w.shape[0]) != int(X.shape[0]):
+                raise ValueError(f"{int(w.shape[0])} weights for {int(X.shape[0])} points")
+            w = w.to(self.device, non_blocking=True)
+            _check_weights(w, dtypes)
         self._src = (X, y)
+        self._w_src = w
         self.n_points = int(X.shape[0])
         if n_vars is None:
             nz = (X != 0).any(dim=0).nonzero()
@@ -147,22 +182,33 @@ class Engine:
             yc = y.to(td).contiguous()
             self._check(self.lib.vsr_set_points(self._h, _ptr(Xc), _ptr(yc), N, ld, n_vars, dt))
             self._points[dt] = (Xc, yc)
+        self._weights = {}
+        if self._w_src is not None:
+            for dt in self._want_dtypes:
+                self._weights[dt] = self._w_src.to(_TORCH_DTYPE[dt]).contiguous()
+                self._check(self.lib.vsr_set_weights(self._h, _ptr(self._weights[dt]), N, dt))
         self.n_vars = n_vars
 
     def adopt_points(self, other):
         """Use the points another engine of the same device holds (no copy: the same device tensors
         are registered with this handle): engines that fit parts of one beam concurrently."""
         self._src = other._src
+        self._w_src = other._w_src
         self.n_points = other.n_points
         self.n_vars = other.n_vars
         self._want_dtypes = tuple(other._want_dtypes)
         self._points = dict(other._points)
+        self._weights = dict(other._weights)
         for dt, (Xc, yc) in self._points.items():
             self._check(self.lib.vsr_set_points(self._h, _ptr(Xc), _ptr(yc), self.n_points, int(Xc.shape[1]),
                                                 self.n_vars, dt))
+            if dt in self._weights:
+                self._check(self.lib.vsr_set_weights(self._h, _ptr(self._weights[dt]), self.n_points, dt))
 
     def ensure_dtype(self, dt):
         if dt not in self._points:
+            if self._w_src is not None:
+                _check_weights(self._w_src, (dt,))
             self._want_dtypes = tuple(self._want_dtypes) + (dt,)
             self._upload_columns(self.n_vars)
 
@@ -419,7 +465,7 @@ def device_engines(devices, home=None):
 
 
 def share_points(engines):
-    """Give every engine the points ``engines[0]`` holds (``set_points`` was called on it).  Each other
+    """Give every engine the points (and weights) ``engines[0]`` holds (``set_points`` was called on it).  Each other
     device gets one copy, made from the home device's tensors: a peer copy on the home stream that torch
     orders before the device's own stream.  Further engines of a device adopt that device's copy."""
     home = engines[0]
@@ -430,5 +476,5 @@ def share_points(engines):
             eng.adopt_points(holder[eng.device])
             continue
         with torch.cuda.device(eng.device):
-            eng.set_points(X, y, dtypes=home._want_dtypes, n_vars=home.n_vars)
+            eng.set_points(X, y, dtypes=home._want_dtypes, n_vars=home.n_vars, w=home._w_src)
         holder[eng.device] = eng
