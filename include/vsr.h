@@ -87,6 +87,18 @@ int vsr_upload_points(vsr_handle* h, const void* X_host, const void* y_host, int
  * slot's N; VSR_ESTATE: the slot has no points. */
 int vsr_set_weights(vsr_handle* h, const void* w_dev, int64_t n_points, int32_t dtype);
 
+/* Robust loss of the points in slot `dtype`: `loss` is a VsrLoss (vsr_isa.h), scipy.optimize.least_squares'
+ * `loss`, and f_scale its `f_scale` (C).  With z_i = w_i r_i^2 / C^2 (w_i = 1 without weights) every point
+ * contributes cost_i = C^2 rho(z_i) instead of w_i r_i^2, and rho'(z_i) w_i r_i df/dc instead of
+ * w_i r_i df/dc.  vsr_set_points / vsr_upload_points of that slot reset it to VSR_LOSS_LINEAR.  Read by
+ * vsr_fit (optimiser sweeps from the eval slot, per-restart score from the score slot), vsr_eval (loss and
+ * gradient) and vsr_gram (the F64 slot's loss); not by vsr_score or vsr_predict.  A residual that is nan or
+ * +-inf contributes the linear terms; a z that overflows from a finite residual contributes scipy's rho(inf)
+ * (C^2 pi / 2 for arctan, +inf otherwise) and no gradient.  VSR_LOSS_LINEAR launches today's kernels, and
+ * huber with every z <= 1 gives the linear results bit for bit.  VSR_EINVAL: unknown loss, or f_scale^2 or
+ * 1 / f_scale^2 not a finite normal double; VSR_ESTATE: the slot has no points. */
+int vsr_set_loss(vsr_handle* h, int32_t loss, double f_scale, int32_t dtype);
+
 /* Programs.  Replaces sp.lambdify of the N-term loss, once per restart (bfgs.py:104)
  * and of the fitted expression (bfgs.py:128).  HOST arrays: instruction words of all
  * C programs back to back, insn_off[C+1], literal pools back to back, imm_off[C+1],
@@ -103,7 +115,8 @@ int vsr_upload_programs(vsr_handle* h, const uint64_t* insns, const int32_t* ins
  * (bfgs.py:120-132).  prog_idx[n_pairs] and const_row[n_pairs] are HOST int32 arrays
  * (const_row may be NULL = identity); consts[.][kstride] and out_grad[n_pairs][kstride]
  * are f64 device arrays; `dtype` picks the point slot and the arithmetic.  Pairs whose
- * program has more than VSR_MAX_DUAL constants get nan gradients. */
+ * program has more than VSR_MAX_DUAL constants get nan gradients.  With weights (vsr_set_weights) the
+ * mean is of w_i r_i^2, with a robust loss (vsr_set_loss) of C^2 rho(z_i), and the gradient follows. */
 int vsr_eval(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row,
              int32_t n_pairs, const double* consts, int32_t kstride, int32_t dtype,
              double* out_loss, double* out_grad, void* stream);
@@ -127,7 +140,10 @@ int vsr_score(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row,
  * What a covariance of fitted constants is built from (sigma^2 (J^T J)^-1, as
  * scipy.optimize.curve_fit's pcov); the reference has no counterpart.  Always reads the VSR_F64
  * point slot.  Non-finite values propagate: a point where f is not real makes both outputs nan.
- * The result of a pair does not depend on the other pairs of the call, bit for bit. */
+ * The result of a pair does not depend on the other pairs of the call, bit for bit.  With the F64
+ * slot's weights out_rss = sum w r^2 and out_jtj = J^T W J; with its robust loss (vsr_set_loss)
+ * out_rss = sum C^2 rho(z_i) and out_jtj = J^T W S J, S = diag(max(rho' + 2 z rho'', 2^-52)): the
+ * statistics of least_squares' scaled Jacobian that curve_fit's pcov uses. */
 int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, int32_t n_pairs,
              const double* consts, int32_t kstride, double* out_rss, double* out_jtj, void* stream);
 
@@ -152,7 +168,9 @@ int vsr_predict(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row
  *   x0, out_consts, out_lastx : [n_slots][kstride] f64   (out_lastx = last point the
  *                               objective saw = what the reference records, bfgs.py:116)
  *   out_loss      [n_slots] f64  objective at out_consts (scaled, penalty applied)
- *   out_final_mse [n_slots] f64  plain MSE at out_lastx in score_dtype (nan allowed)
+ *   out_final_mse [n_slots] f64  plain MSE at out_lastx in score_dtype (nan allowed); the mean of
+ *                               w r^2 with weights, of C^2 rho(z) with a robust loss on the score slot
+ * The sweeps read the eval slot's weights and robust loss (vsr_set_weights, vsr_set_loss).
  *   out_info      [n_slots][4] int32: status (VsrFitStatus), nit, nfev, reserved
  * Programs with k == 0 are not optimised: status VSR_FIT_NOT_RUN, final MSE only. */
 int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int32_t n_runs,

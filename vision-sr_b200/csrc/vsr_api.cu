@@ -1,6 +1,7 @@
 // vsr_api.cu -- C ABI of libvsr.so (declared in include/vsr.h): handle, uploads, launch
 // logic.  No torch types, no host synchronisation except in the *_host entry points.
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -80,6 +81,7 @@ struct PointSlot {
   const void* X = nullptr;
   const void* y = nullptr;
   const void* w = nullptr;  // per-point weights (vsr_set_weights), nullptr: unweighted
+  vsr::RobustLoss loss{VSR_LOSS_LINEAR, 1.0, 1.0};  // vsr_set_loss
   int64_t n = 0, ldx = 0;
   int n_vars = 0;
   DevBuf ownX, ownY;
@@ -192,6 +194,9 @@ vsr::ProgramTable table_of(const vsr_handle* h) {
   return t;
 }
 
+// the slot's robust loss for a launch (nullptr: linear, which takes today's kernels)
+const vsr::RobustLoss* robust_of(const PointSlot& s) { return s.loss.kind != VSR_LOSS_LINEAR ? &s.loss : nullptr; }
+
 vsr::Points points_of(const PointSlot& s) {
   vsr::Points p;
   p.X = s.X;
@@ -204,12 +209,16 @@ vsr::Points points_of(const PointSlot& s) {
 using vsr::points_per_thread;
 
 // the kernels are instantiated one (type, width) pair per translation unit (vsr_inst.cu) so the
-// library builds in parallel; here only the dispatch over the runtime width
+// library builds in parallel; here only the dispatch over the runtime width (and, with a robust loss
+// rl != nullptr, to the RB kernels)
 template <typename T>
 cudaError_t launch_fit(int K, const vsr::FitArgs& a, int threads, int cs, size_t smem, int clusters, cudaStream_t st,
-                       const void* w) {
+                       const void* w, const vsr::RobustLoss* rl) {
   switch (K) {
-#define C(KK) case KK: return vsr::launch_fit_T<T, KK>(a, threads, cs, smem, clusters, st, w);
+#define C(KK)                                                                                      \
+  case KK:                                                                                         \
+    return rl ? vsr::launch_fit_rb_T<T, KK>(a, threads, cs, smem, clusters, st, w, *rl)            \
+              : vsr::launch_fit_T<T, KK>(a, threads, cs, smem, clusters, st, w);
     C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
 #undef C
   }
@@ -227,9 +236,12 @@ int fit_threads_cap(int K) {
 }
 
 template <typename T>
-cudaError_t launch_eval(int K, const vsr::EvalArgs& a, int threads, size_t smem, cudaStream_t st, const void* w) {
+cudaError_t launch_eval(int K, const vsr::EvalArgs& a, int threads, size_t smem, cudaStream_t st, const void* w,
+                        const vsr::RobustLoss* rl) {
   switch (K) {
-#define C(KK) case KK: return vsr::launch_eval_T<T, KK>(a, threads, smem, st, w);
+#define C(KK)                                                                                        \
+  case KK:                                                                                           \
+    return rl ? vsr::launch_eval_rb_T<T, KK>(a, threads, smem, st, w, *rl) : vsr::launch_eval_T<T, KK>(a, threads, smem, st, w);
     C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
 #undef C
   }
@@ -237,9 +249,12 @@ cudaError_t launch_eval(int K, const vsr::EvalArgs& a, int threads, size_t smem,
 }
 
 template <typename T>
-cudaError_t launch_eval_tile(int K, const vsr::EvalTileArgs& a, size_t smem, cudaStream_t st, const void* w) {
+cudaError_t launch_eval_tile(int K, const vsr::EvalTileArgs& a, size_t smem, cudaStream_t st, const void* w,
+                             const vsr::RobustLoss* rl) {
   switch (K) {
-#define C(KK) case KK: return vsr::launch_eval_tile_T<T, KK>(a, smem, st, w);
+#define C(KK)                                                                                 \
+  case KK:                                                                                    \
+    return rl ? vsr::launch_eval_tile_rb_T<T, KK>(a, smem, st, w, *rl) : vsr::launch_eval_tile_T<T, KK>(a, smem, st, w);
     C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
 #undef C
   }
@@ -256,9 +271,10 @@ cudaError_t launch_predict(int K, const vsr::PredictArgs& a, size_t smem, cudaSt
   return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_gram(int K, const vsr::GramArgs& a, size_t smem, cudaStream_t st, const void* w) {
+cudaError_t launch_gram(int K, const vsr::GramArgs& a, size_t smem, cudaStream_t st, const void* w,
+                        const vsr::RobustLoss* rl) {
   switch (K) {
-#define C(KK) case KK: return vsr::launch_gram_K<KK>(a, smem, st, w);
+#define C(KK) case KK: return rl ? vsr::launch_gram_rb_K<KK>(a, smem, st, w, *rl) : vsr::launch_gram_K<KK>(a, smem, st, w);
     C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
 #undef C
   }
@@ -375,8 +391,10 @@ int stage_lists(vsr_handle* h, const std::vector<int32_t>& all, cudaStream_t st)
 int run_eval_group(vsr_handle* h, int K, int dtype, const int32_t* d_prog, const int32_t* d_row,
                    const int32_t* d_out, int n_pairs, int kmax, int max_insn, int max_imm,
                    const double* consts, int kstride, double* out_loss, double* out_grad,
-                   cudaStream_t st, int nan_to_num = 0, unsigned var_mask = 0, const void* w = nullptr) {
-  // w: the slot's weights for a weighted loss and gradient (nullptr: unweighted)
+                   cudaStream_t st, int nan_to_num = 0, unsigned var_mask = 0, const void* w = nullptr,
+                   const vsr::RobustLoss* rl = nullptr) {
+  // w: the slot's weights for a weighted loss and gradient (nullptr: unweighted); rl: its robust loss
+  // (nullptr: linear).  A robust launch has the geometry and staging of the linear one.
   const PointSlot& ps = h->pts[dtype];
   const int P = points_per_thread(K);
   const int64_t N = ps.n;
@@ -418,7 +436,8 @@ int run_eval_group(vsr_handle* h, int K, int dtype, const int32_t* d_prog, const
       // (a weighted launch reads the weights from global memory: the same chunks, so w = 1 gives the
       // unweighted sums bit for bit)
       const size_t smem = fixed + (size_t)(t.n_cols + 1) * chunk * elem;
-      cudaError_t e = dtype == VSR_F64 ? launch_eval_tile<double>(K, t, smem, st, w) : launch_eval_tile<float>(K, t, smem, st, w);
+      cudaError_t e = dtype == VSR_F64 ? launch_eval_tile<double>(K, t, smem, st, w, rl)
+                                         : launch_eval_tile<float>(K, t, smem, st, w, rl);
       if (e != cudaSuccess) return fail(h, VSR_ECUDA, "eval tile kernel launch failed (smem %zu): %s", smem, cudaGetErrorString(e));
       const int total = n_pairs * (K + 1);
       vsr::eval_finalize<<<(total + 127) / 128, 128, 0, st>>>(t.e.partial, d_prog, d_out, t.e.pt.k, n_pairs, (int)chunks, K,
@@ -450,8 +469,8 @@ int run_eval_group(vsr_handle* h, int K, int dtype, const int32_t* d_prog, const
   a.nsplit = nsplit;
   a.nan_to_num = nan_to_num;
   const size_t smem = sizeof(double) * (size_t)((K + 1) * threads + kmax + 2 + max_imm + max_insn + 1);  // + pad word
-  cudaError_t e = dtype == VSR_F64 ? launch_eval<double>(K, a, threads, smem, st, w)
-                                   : launch_eval<float>(K, a, threads, smem, st, w);
+  cudaError_t e = dtype == VSR_F64 ? launch_eval<double>(K, a, threads, smem, st, w, rl)
+                                   : launch_eval<float>(K, a, threads, smem, st, w, rl);
   if (e != cudaSuccess) return fail(h, VSR_ECUDA, "eval kernel launch failed: %s", cudaGetErrorString(e));
   const int total = n_pairs * (K + 1);
   vsr::eval_finalize<<<(total + 127) / 128, 128, 0, st>>>(
@@ -662,6 +681,7 @@ int vsr_set_points(vsr_handle* h, const void* X_dev, const void* y_dev, int64_t 
   s.X = X_dev;
   s.y = y_dev;
   s.w = nullptr;
+  s.loss = vsr::RobustLoss{VSR_LOSS_LINEAR, 1.0, 1.0};
   s.n = n_points;
   s.ldx = ldx;
   s.n_vars = n_vars;
@@ -689,6 +709,7 @@ int vsr_upload_points(vsr_handle* h, const void* X_host, const void* y_host, int
   s.X = s.ownX.p;
   s.y = s.ownY.p;
   s.w = nullptr;
+  s.loss = vsr::RobustLoss{VSR_LOSS_LINEAR, 1.0, 1.0};
   s.n = n_points;
   s.ldx = dld;
   s.n_vars = n_vars;
@@ -703,6 +724,19 @@ int vsr_set_weights(vsr_handle* h, const void* w_dev, int64_t n_points, int32_t 
   if (w_dev && n_points != s.n)
     return fail(h, VSR_EINVAL, "%lld weights for %lld points (dtype %d)", (long long)n_points, (long long)s.n, dtype);
   s.w = w_dev;
+  return VSR_OK;
+}
+
+int vsr_set_loss(vsr_handle* h, int32_t loss, double f_scale, int32_t dtype) {
+  if (!h) return VSR_EINVAL;
+  if (dtype != VSR_F64 && dtype != VSR_F32) return fail(h, VSR_EINVAL, "bad dtype %d", dtype);
+  if (loss < VSR_LOSS_LINEAR || loss > VSR_LOSS_ARCTAN) return fail(h, VSR_EINVAL, "unknown loss %d", loss);
+  const double c2 = f_scale * f_scale, inv_c2 = 1.0 / c2;
+  if (!std::isnormal(c2) || !std::isnormal(inv_c2))
+    return fail(h, VSR_EINVAL, "f_scale %g: its square or inverse square is not a normal double", f_scale);
+  PointSlot& s = h->pts[dtype];
+  if (!s.X || s.n <= 0) return fail(h, VSR_ESTATE, "no points uploaded for dtype %d", dtype);
+  s.loss = vsr::RobustLoss{loss, c2, inv_c2};
   return VSR_OK;
 }
 
@@ -844,7 +878,7 @@ int vsr_eval(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, i
     if (!n) continue;
     rc = run_eval_group(h, g.K, dtype, dl + off[gi], dl + off[gi] + n, dl + off[gi] + 2 * n, n,
                         g.kmax, g.max_insn, g.max_imm, consts, kstride, out_loss,
-                        g.K > 0 ? out_grad : nullptr, st, 0, g.var_mask, h->pts[dtype].w);
+                        g.K > 0 ? out_grad : nullptr, st, 0, g.var_mask, h->pts[dtype].w, robust_of(h->pts[dtype]));
     if (rc) return rc;
   }
   if (out_grad && !toowide.prog.empty()) {
@@ -926,10 +960,10 @@ int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, i
     a.consts = consts;
     a.partial = partial;
     a.nsplit = vsr::gram_nsplit(ps.n, tile);
-    const size_t cols = (size_t)(K + 1) + (ps.w ? 1 : 0);  // r, J (and w)
+    const size_t cols = (size_t)(K + 1) + (robust_of(ps) ? 2 : (ps.w ? 1 : 0));  // r, J (and w, or wq and ws)
     const size_t smem = sizeof(double) * (cols * vsr::gram_col_stride(tile) + g.kmax + 1 + g.max_imm) +
                         sizeof(vsr_insn_t) * (g.max_insn + 1);
-    cudaError_t e = launch_gram(K, a, smem, st, ps.w);
+    cudaError_t e = launch_gram(K, a, smem, st, ps.w, robust_of(ps));
     if (e != cudaSuccess) return fail(h, VSR_ECUDA, "gram kernel launch failed: %s", cudaGetErrorString(e));
     const int64_t total = (int64_t)n * (1 + (int64_t)kstride * kstride);
     vsr::gram_finalize<<<(unsigned)((total + 127) / 128), 128, 0, st>>>(partial, a.pair_prog, dl + off[gi] + 2 * n,
@@ -1274,8 +1308,10 @@ int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int
     a.queue = (int32_t*)h->d_queue.p + gi;
     const int want_clusters = (n + geo.seats - 1) / geo.seats;
     cudaError_t e = opts->eval_dtype == VSR_F64
-                        ? launch_fit<double>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.w)
-                        : launch_fit<float>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.w);
+                        ? launch_fit<double>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.w,
+                                             robust_of(ps))
+                        : launch_fit<float>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.w,
+                                            robust_of(ps));
     if (e != cudaSuccess)
       return fail(h, VSR_ECUDA, "fit kernel launch failed (K=%d threads=%d cluster=%d seats=%d smem=%zu): %s", g.K,
                   geo.threads, geo.cs, geo.seats, geo.smem, cudaGetErrorString(e));
@@ -1287,10 +1323,11 @@ int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int
   }
   if (h->profiling) VSR_CUDA(h, cudaEventRecord(ev_b, st));
   // per-restart score: plain MSE at the last evaluated point, in score_dtype (bfgs.py:120-132); with
-  // weights on the score slot the weighted mean of w r^2
+  // weights on the score slot the weighted mean of w r^2, with a robust loss the mean cost C^2 rho(z)
   rc = run_eval_group(h, 0, opts->score_dtype, dl + score_off, dl + score_off + n_runs,
                       dl + score_off + n_runs, n_runs, s_kmax, s_insn, s_imm, out_lastx, kstride,
-                      out_final_mse, nullptr, st, 0, 0, h->pts[opts->score_dtype].w);
+                      out_final_mse, nullptr, st, 0, 0, h->pts[opts->score_dtype].w,
+                      robust_of(h->pts[opts->score_dtype]));
   if (h->profiling) {
     VSR_CUDA(h, cudaEventRecord(ev_c, st));
     h->spans.push_back({ev_a, ev_b, 0, (int)groups.size()});

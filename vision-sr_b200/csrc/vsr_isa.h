@@ -105,4 +105,13 @@ enum VsrGradMode {
 // element types of the uploaded points
 enum VsrDtype { VSR_F64 = 0, VSR_F32 = 1 };
 
+// robust losses of vsr_set_loss: scipy.optimize.least_squares' `loss` (rho of z = w r^2 / f_scale^2)
+enum VsrLoss {
+  VSR_LOSS_LINEAR = 0,   // rho(z) = z: the (weighted) sum of squares
+  VSR_LOSS_SOFT_L1 = 1,  // 2 ((1 + z)^(1/2) - 1)
+  VSR_LOSS_HUBER = 2,    // z if z <= 1, else 2 z^(1/2) - 1
+  VSR_LOSS_CAUCHY = 3,   // log1p(z)
+  VSR_LOSS_ARCTAN = 4    // arctan(z)
+};
+
 #endif  // VSR_ISA_H_

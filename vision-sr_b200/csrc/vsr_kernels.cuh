@@ -28,6 +28,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "vsr_bfgs.h"
 #include "vsr_interp.h"
 #include "vsr_isa.h"
@@ -138,6 +140,91 @@ struct Weighted : A {
 template <typename A>
 struct Weighted<A, false> : A {};
 
+// Robust loss of a point slot (vsr_set_loss): kind (VsrLoss), C^2 and 1/C^2 of f_scale C.
+struct RobustLoss {
+  int32_t kind;
+  double c2, inv_c2;
+};
+
+// Kernel arguments of a robust launch (RB = true): the weighted struct with the loss appended last.  In a
+// robust kernel the weight pointer is optional at run time (nullptr: unweighted).
+template <typename A>
+struct Robust : Weighted<A, true> {
+  RobustLoss loss;
+};
+template <typename A, bool W, bool RB>
+using KernelArgs = std::conditional_t<RB, Robust<A>, Weighted<A, W>>;
+
+// Per-point factors of a robust loss at z = w r^2 / C^2 (finite, >= 0), scipy's least_squares
+// definitions: q = rho(z) / z (the cost ratio, q(0) = 1), g = rho'(z), s = rho'(z) + 2 z rho''(z).  q is
+// formed directly, never as z / z, so huber's z <= 1 branch gives q = g = s = 1 exactly.  fp64 throughout.
+__device__ __forceinline__ void robust_factors(int kind, double z, double& q, double& g, double& s) {
+  switch (kind) {
+    case VSR_LOSS_SOFT_L1: {
+      const double t = 1.0 + z, st = sqrt(t);
+      q = 2.0 / (1.0 + st);  // 2 (sqrt(1+z) - 1) / z without the cancellation
+      g = 1.0 / st;
+      s = g / t;
+      return;
+    }
+    case VSR_LOSS_HUBER:
+      if (z <= 1.0) {
+        q = g = s = 1.0;
+      } else {
+        const double sz = sqrt(z);
+        q = (2.0 * sz - 1.0) / z;
+        g = 1.0 / sz;
+        s = 0.0;
+      }
+      return;
+    case VSR_LOSS_CAUCHY:
+      q = z == 0.0 ? 1.0 : log1p(z) / z;
+      g = 1.0 / (1.0 + z);
+      s = (1.0 - z) * g * g;
+      return;
+    case VSR_LOSS_ARCTAN:
+      q = z == 0.0 ? 1.0 : atan(z) / z;
+      g = 1.0 / (1.0 + z * z);
+      s = (1.0 - 3.0 * z * z) * g * g;  // nan past z ~ 1e154 (inf * 0): the clamp to eps takes it
+      return;
+    default:
+      q = g = s = 1.0;
+  }
+}
+
+// scipy's rho at z = +inf, where z overflowed from a finite residual: C^2 pi / 2 for arctan, +inf otherwise
+__device__ __forceinline__ double robust_cost_inf(const RobustLoss& L) {
+  return L.kind == VSR_LOSS_ARCTAN ? L.c2 * 1.5707963267948966 : __longlong_as_double(0x7ff0000000000000ll);
+}
+
+// Residual step of a robust sweep (RB): adds cost = C^2 rho(z) to ps as (rw * q) * r and rho'(z) rw d_t to
+// pg[t], with rw = w r (r without weights).  A non-finite r contributes the linear terms rw r and rw d_t
+// (the penalty rule); a z that overflows from a finite r contributes scipy's rho(inf) and no gradient.  With
+// q = g = 1 the products are the linear step's, so huber with every z <= 1 gives its sums bit for bit.
+template <typename T, int K>
+__device__ __forceinline__ void robust_step(const RobustLoss& L, double r, double rw, const Dual<T, K>& d,
+                                            double& ps, double* pg) {
+  double q = 1.0, g = 1.0, s;
+  bool add = true;
+  if (fabs(r) <= 1.7976931348623157e308) {
+    const double z = rw * r * L.inv_c2;
+    if (z <= 1.7976931348623157e308) {
+      robust_factors(L.kind, z, q, g, s);
+    } else {
+      ps += robust_cost_inf(L);
+      g = 0.0;
+      add = false;
+    }
+  }
+  if (add) ps += (rw * q) * r;
+  const double rg = g * rw;
+#pragma unroll
+  for (int t = 0; t < K; ++t) {
+    const double gt = rg * (double)d.d[t];
+    if (fabs(gt) <= 1.7976931348623157e308) pg[t] += gt;
+  }
+}
+
 // ---- point source: coalesced global loads (read-only path) --------------------------
 template <typename T, int P>
 struct GlobalPoints {
@@ -169,12 +256,13 @@ __device__ __forceinline__ void keep_in_register(int& v) { asm volatile("" : "+r
 // value of T) before the residual is taken: the drivers' scoring rule (Feynman_test.py:87).
 // W: per-point weights w (fp64 arithmetic): sum w r^2 and sum w r df/dc_t.  rw = w * r is formed once and
 // every product is the unweighted one with r replaced by rw, so w = 1.0 gives the unweighted sums bit for bit.
-template <typename T, int K, int P, bool NTN = false, bool W = false>
+// RB: robust loss L (robust_step), weights optional (w = nullptr: rw = r).
+template <typename T, int K, int P, bool NTN = false, bool W = false, bool RB = false>
 __device__ __forceinline__ void sweep_points(const vsr_insn_t* prog, const double* imm,
                                              const T* cst, const T* __restrict__ X,
                                              const T* __restrict__ y, int64_t ldx, int64_t n0,
                                              int64_t n1, double* scratch, int tid, int nt,
-                                             const T* __restrict__ w = nullptr) {
+                                             const T* __restrict__ w = nullptr, RobustLoss L = {}) {
   // tid / nt: index of this thread among the nt threads that take part in the sweep
   Stack<T, K, P> stk;
   GlobalPoints<T, P> xs;
@@ -203,7 +291,9 @@ __device__ __forceinline__ void sweep_points(const vsr_insn_t* prog, const doubl
           pv = pv != pv ? T(0) : (pv > big ? big : (pv < -big ? -big : pv));
         }
         const double r = (double)pv - (double)__ldg(y + xs.idx[p]);
-        if constexpr (W) {
+        if constexpr (RB) {
+          robust_step<T, K>(L, r, w ? (double)__ldg(w + xs.idx[p]) * r : r, acc[p], ps, pg);
+        } else if constexpr (W) {
           const double rw = (double)__ldg(w + xs.idx[p]) * r;
           ps += rw * r;
 #pragma unroll
@@ -377,11 +467,11 @@ struct SlicePoints {
 };
 
 // One pass over the resident slice (cnt points); partial sums parked like sweep_points does.
-// W: the weights are staged like y (ws, cnt values), same residual rule as sweep_points.
-template <typename T, int K, int P, bool NTN = false, bool W = false>
+// W: the weights are staged like y (ws, cnt values), same residual rule as sweep_points.  RB: as there.
+template <typename T, int K, int P, bool NTN = false, bool W = false, bool RB = false>
 __device__ __forceinline__ void sweep_slice(const vsr_insn_t* prog, const double* imm, const T* cst,
                                             const T* xs, const T* ys, int stride, int cnt, double* scratch,
-                                            int tid, int nt, const T* ws = nullptr) {
+                                            int tid, int nt, const T* ws = nullptr, RobustLoss L = {}) {
   Stack<T, K, P> stk;
   SlicePoints<T, P> src;
   src.base = xs;
@@ -410,7 +500,9 @@ __device__ __forceinline__ void sweep_slice(const vsr_insn_t* prog, const double
           pv = pv != pv ? T(0) : (pv > big ? big : (pv < -big ? -big : pv));
         }
         const double r = (double)pv - (double)ys[src.idx[p]];
-        if constexpr (W) {
+        if constexpr (RB) {
+          robust_step<T, K>(L, r, ws ? (double)ws[src.idx[p]] * r : r, acc[p], ps, pg);
+        } else if constexpr (W) {
           const double rw = (double)ws[src.idx[p]] * r;
           ps += rw * r;
 #pragma unroll
@@ -959,10 +1051,11 @@ __device__ __forceinline__ bool seat_turn(const FitArgs& a, int lane, int cs, Fi
 }
 
 // W: weighted launch (a.w: per-point weights of the slot of T); a resident slice stages the weight
-// column after the n_cols columns of X.
-template <typename T, int K, int P, bool W>
+// column after the n_cols columns of X.  RB: robust launch (a.loss), weighted when a.w is set: it stages
+// exactly what the weighted or unweighted launch stages.
+template <typename T, int K, int P, bool W, bool RB = false>
 __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>()))
-    fit_kernel(const Weighted<FitArgs, W> a) {
+    fit_kernel(const KernelArgs<FitArgs, W, RB> a) {
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   extern __shared__ __align__(16) double smem[];
@@ -998,6 +1091,8 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
   const int cnt = (int)(n1 - n0);
   const T* X = static_cast<const T*>(a.pts.X);
   const T* y = static_cast<const T*>(a.pts.y);
+  const T* rb_w = nullptr;  // the weights of a robust launch (nullptr: unweighted)
+  if constexpr (RB) rb_w = static_cast<const T*>(a.w);
 
   double* wpart = smem + (size_t)G * seat_d;                      // [G][nw][K+1]
   double* scratch = wpart + (size_t)G * nw * (K + 1);             // [(K+1)][threads]
@@ -1032,13 +1127,14 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
     const bool use_tma = a.tma_ok && full > 0;
     if (tid == 0 && use_tma) {
       const uint32_t bytes = (uint32_t)full * (uint32_t)sizeof(T);
-      mbar_expect_tx(&s_bar, bytes * (uint32_t)(a.n_cols + 1 + (W ? 1 : 0)));
+      mbar_expect_tx(&s_bar, bytes * (uint32_t)(a.n_cols + 1 + (W || rb_w ? 1 : 0)));
       tma_bulk_load(ys, y + n0, bytes, &s_bar);
       for (int j = 0; j < VSR_MAX_VARS; ++j)
         if (a.col_of_var[j] >= 0)
           tma_bulk_load(xs + (size_t)a.col_of_var[j] * stride, X + (int64_t)j * a.pts.ldx + n0, bytes, &s_bar);
       if constexpr (W)
         tma_bulk_load(xs + (size_t)a.n_cols * stride, static_cast<const T*>(a.w) + n0, bytes, &s_bar);
+      if (rb_w) tma_bulk_load(xs + (size_t)a.n_cols * stride, rb_w + n0, bytes, &s_bar);
     }
     {
       // everything TMA does not move (all of it when the caller's memory is unaligned): coalesced loads
@@ -1047,6 +1143,10 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
       if constexpr (W) {
         T* wsl = xs + (size_t)a.n_cols * stride;
         for (int i = first + tid; i < cnt; i += blockDim.x) wsl[i] = static_cast<const T*>(a.w)[n0 + i];
+      }
+      if (rb_w) {
+        T* wsl = xs + (size_t)a.n_cols * stride;
+        for (int i = first + tid; i < cnt; i += blockDim.x) wsl[i] = rb_w[n0 + i];
       }
       for (int j = 0; j < VSR_MAX_VARS; ++j) {
         const int sj = a.col_of_var[j];
@@ -1141,7 +1241,14 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
         if (c.prog < 0) {  // the seat is closed
           live &= ~(1u << g);
         } else {
-          if constexpr (W) {
+          if constexpr (RB) {
+            if (a.resident)
+              sweep_slice<T, K, P, false, false, true>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
+                                                       rb_w ? xs + (size_t)a.n_cols * stride : nullptr, a.loss);
+            else
+              sweep_points<T, K, P, false, false, true>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid,
+                                                        snt, rb_w, a.loss);
+          } else if constexpr (W) {
             if (a.resident)
               sweep_slice<T, K, P, false, true>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
                                                 xs + (size_t)a.n_cols * stride);
@@ -1185,9 +1292,9 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
 }
 
 // dynamic shared memory of eval_kernel, in doubles: red[(K+1)*threads] | cst[k] | imm | insn
-// W: weighted sums (a.w, read from global memory like y)
-template <typename T, int K, int P, bool W>
-__global__ void __launch_bounds__(256) eval_kernel(const Weighted<EvalArgs, W> a) {
+// W: weighted sums (a.w, read from global memory like y).  RB: robust sums (a.loss), weighted when a.w is set.
+template <typename T, int K, int P, bool W, bool RB = false>
+__global__ void __launch_bounds__(256) eval_kernel(const KernelArgs<EvalArgs, W, RB> a) {
   extern __shared__ double smem[];
   const int pair = blockIdx.x;
   const int split = blockIdx.y;
@@ -1219,7 +1326,11 @@ __global__ void __launch_bounds__(256) eval_kernel(const Weighted<EvalArgs, W> a
   n0 = n0 < N ? n0 : N;
   n1 = n1 < N ? n1 : N;
 
-  if constexpr (W)  // (vsr_score, the nan_to_num rule, is never weighted)
+  if constexpr (RB)  // (nor robust)
+    sweep_points<T, K, P, false, false, true>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
+                                              static_cast<const T*>(a.pts.y), a.pts.ldx, n0, n1, red,
+                                              (int)threadIdx.x, (int)blockDim.x, static_cast<const T*>(a.w), a.loss);
+  else if constexpr (W)  // (vsr_score, the nan_to_num rule, is never weighted)
     sweep_points<T, K, P, false, true>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
                                        static_cast<const T*>(a.pts.y), a.pts.ldx, n0, n1, red, (int)threadIdx.x,
                                        (int)blockDim.x, static_cast<const T*>(a.w));
@@ -1266,9 +1377,10 @@ __host__ __device__ inline size_t eval_tile_fixed_doubles(int K, int threads, in
 
 // W: weighted sums.  The weights are read from global memory (a.w, like y in eval_kernel), not staged: the
 // chunks are those of the unweighted launch, so the partial sums are formed in the same order and w = 1
-// gives the unweighted result bit for bit.
-template <typename T, int K, int P, bool W>
-__global__ void __launch_bounds__((eval_tile_threads<K>()), 1) eval_tile_kernel(const Weighted<EvalTileArgs, W> a) {
+// gives the unweighted result bit for bit.  RB: robust sums (a.loss), weights as in W when a.w is set.
+template <typename T, int K, int P, bool W, bool RB = false>
+__global__ void __launch_bounds__((eval_tile_threads<K>()), 1)
+    eval_tile_kernel(const KernelArgs<EvalTileArgs, W, RB> a) {
   extern __shared__ __align__(16) double smem[];
   __shared__ __align__(8) uint64_t s_bar;
   const int tid = threadIdx.x, nt = blockDim.x;
@@ -1348,7 +1460,10 @@ __global__ void __launch_bounds__((eval_tile_threads<K>()), 1) eval_tile_kernel(
     commit();
     __syncthreads();
     if (pair + 1 < a.e.n_pairs) fetch(pair + 1);
-    if constexpr (W)
+    if constexpr (RB)
+      sweep_slice<T, K, P, false, false, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
+                                               a.w ? static_cast<const T*>(a.w) + n0 : nullptr, a.loss);
+    else if constexpr (W)
       sweep_slice<T, K, P, false, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
                                         static_cast<const T*>(a.w) + n0);
     else if (K == 0 && a.e.nan_to_num)
@@ -1399,8 +1514,14 @@ __host__ __device__ constexpr int gram_col_stride(int tile) { return tile + 1; }
 // dynamic shared memory of gram_kernel, in doubles: tile[(K+1) * gram_col_stride] | cst[k] | imm | insn
 // W: weighted sums rss = sum w r^2, jtj[a][b] = sum w J_a J_b (J^T W J).  The tile gets one column more, the
 // weights, and every term is fma(col_a * w, col_b, acc): w = 1.0 gives the unweighted sums bit for bit.
-template <int K, int P, bool W>
-__global__ void __launch_bounds__(kGramThreads) gram_kernel(const Weighted<GramArgs, W> a) {
+// RB: curve_fit's statistics under a robust loss (a.loss, weighted when a.w is set): rss = sum C^2 rho(z),
+// jtj[a][b] = sum w s J_a J_b with s = max(rho' + 2 z rho'', 2^-52) (least_squares' scaled Jacobian).  The
+// tile gets two factor columns where W parks w: w q (q = rho(z)/z) for rss and w s for the J entries, so the
+// terms are fma(r * wq, r, acc) and fma(J_a * ws, J_b, acc), the unweighted / weighted sums when q = s = 1.
+// A non-finite r gets q = s = 1 (the outputs become non-finite, as in the linear kernel); a z that overflows
+// from a finite r parks r = 1 and wq = rho(inf) C^2, and s = 2^-52.
+template <int K, int P, bool W, bool RB = false>
+__global__ void __launch_bounds__(kGramThreads) gram_kernel(const KernelArgs<GramArgs, W, RB> a) {
   extern __shared__ double smem[];
   const int pair = blockIdx.x;
   const int split = blockIdx.y;
@@ -1410,8 +1531,8 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const Weighted<GramA
   constexpr int kEnt = gram_entries(K);
   const int prog = a.pair_prog[pair];
   const int k = a.pt.k[prog];
-  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K) (then w when W)
-  double* cst = s_val + (K + 1 + (W ? 1 : 0)) * kLd;
+  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K) (then w when W, then wq and ws when RB)
+  double* cst = s_val + (K + 1 + (W ? 1 : 0) + (RB ? 2 : 0)) * kLd;
   double* s_imm = cst + k + 1;
   const int m_imm = a.pt.imm_off[prog + 1] - a.pt.imm_off[prog];
   vsr_insn_t* s_insn = reinterpret_cast<vsr_insn_t*>(s_imm + m_imm);
@@ -1462,10 +1583,33 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const Weighted<GramA
 #pragma unroll
         for (int t = 0; t < K; ++t) s_val[(1 + t) * kLd + j] = v[p].d[t];
         if constexpr (W) s_val[(K + 1) * kLd + j] = __ldg(static_cast<const double*>(a.w) + xs.idx[p]);
+        if constexpr (RB) {
+          const double r = s_val[j];
+          const double w = a.w ? __ldg(static_cast<const double*>(a.w) + xs.idx[p]) : 1.0;
+          double q = 1.0, g, s = 1.0, wq;
+          bool over = false;
+          if (fabs(r) <= 1.7976931348623157e308) {
+            const double z = w * r * r * a.loss.inv_c2;
+            if (z <= 1.7976931348623157e308) {
+              robust_factors(a.loss.kind, z, q, g, s);
+            } else {
+              over = true;
+              s_val[j] = 1.0;
+              s = 0.0;
+            }
+          }
+          wq = over ? robust_cost_inf(a.loss) : w * q;
+          s_val[(K + 1) * kLd + j] = wq;
+          s_val[(K + 2) * kLd + j] = w * (s > 0x1p-52 ? s : 0x1p-52);  // (nan fails the compare)
+        }
       }
     }
     __syncthreads();
-    if constexpr (W) {
+    if constexpr (RB) {
+      const double* col_f = s_val + (K + (tid == 0 ? 1 : 2)) * kLd;
+      if (tid < kEnt)
+        for (int j = 0; j < cnt; ++j) acc = fma(col_a[j] * col_f[j], col_b[j], acc);
+    } else if constexpr (W) {
       const double* col_w = s_val + (K + 1) * kLd;
       if (tid < kEnt)
         for (int j = 0; j < cnt; ++j) acc = fma(col_a[j] * col_w[j], col_b[j], acc);

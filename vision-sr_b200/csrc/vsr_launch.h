@@ -33,6 +33,20 @@ cudaError_t launch_predict_T(const PredictArgs& a, size_t smem, cudaStream_t st)
 template <int K>
 cudaError_t launch_gram_K(const GramArgs& a, size_t smem, cudaStream_t st, const void* w);
 
+// robust launches (RB kernels, compiled in the VSR_INST_RB units): the same arguments, the slot's weights
+// (nullptr: unweighted) and its loss (L.kind != VSR_LOSS_LINEAR; linear launches take the wrappers above)
+template <typename T, int K>
+cudaError_t launch_fit_rb_T(const FitArgs& a, int threads, int cs, size_t smem, int clusters, cudaStream_t st,
+                            const void* w, const RobustLoss& L);
+template <typename T, int K>
+cudaError_t launch_eval_rb_T(const EvalArgs& a, int threads, size_t smem, cudaStream_t st, const void* w,
+                             const RobustLoss& L);
+template <typename T, int K>
+cudaError_t launch_eval_tile_rb_T(const EvalTileArgs& a, size_t smem, cudaStream_t st, const void* w,
+                                  const RobustLoss& L);
+template <int K>
+cudaError_t launch_gram_rb_K(const GramArgs& a, size_t smem, cudaStream_t st, const void* w, const RobustLoss& L);
+
 // forces the (lazily loaded) kernels of one instantiation onto the device
 template <typename T, int K>
 cudaError_t preload_T();

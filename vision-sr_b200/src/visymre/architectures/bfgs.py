@@ -513,7 +513,8 @@ def sigma_weights(sigma, X, cfg):
     return fitter.weights_from_sigma(sigma, n, {eval_dtype, score_dtype, fitter.F64})
 
 
-def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False, sigma=None):
+def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False, sigma=None,
+               loss="linear", f_scale=1.0):
     """Fit every candidate of a beam in one go (see ``_bfgs_batch``).
 
     ``sigma``: optional 1-D array of N per-point standard deviations (any device), as
@@ -522,6 +523,14 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     prune's acceptance are weighted.  ``ValueError`` for a wrong length, a sigma that is not finite and
     > 0, a ``1/sigma**2`` that is not a finite normal number in a point dtype of the fit, or ``sigma`` with
     ``cfg.bfgs.idx_remove``.  With a process group every rank passes its own ``sigma``, like ``X``, ``y``.
+
+    ``loss``, ``f_scale``: a robust loss, as ``scipy.optimize.curve_fit`` passes them to ``least_squares``
+    (``"linear"``, ``"soft_l1"``, ``"huber"``, ``"cauchy"``, ``"arctan"``; ``fitter.robust_loss``).  Every
+    fit then minimises ``loss_scale * mean(C**2 rho(w r**2 / C**2))`` with ``C = f_scale``, and the
+    returned loss, the per-restart score that picks the restart and the prune's acceptance are that robust
+    mean.  ``ValueError`` for another name or an ``f_scale`` that is not finite and > 0 (or whose square
+    or inverse square is not a normal double), before the engine is touched.  ``"linear"`` (the default)
+    is the sum of squares.  With a process group every rank passes the same values.
 
     With ``cfg.bfgs.collapse_duplicates`` (off by default; SURVEY 8f row 4) candidates that
     compile to the SAME bytecode -- beams that differ only in ways sympy canonicalises away,
@@ -532,8 +541,10 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     """
     pred_strs = list(pred_strs)
     w = sigma_weights(sigma, X, cfg)
+    rl = fitter.robust_loss(loss, f_scale)
     if not _opt(cfg, "collapse_duplicates", False) or len(pred_strs) < 2:
-        return _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=x0, engine=engine, lazy_strings=lazy_strings, w=w)
+        return _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=x0, engine=engine, lazy_strings=lazy_strings, w=w,
+                           rl=rl)
     variables = list(test_data.total_variables)
     first, rep_of, own_expr = {}, [], []
     for i, toks in enumerate(pred_strs):
@@ -548,7 +559,7 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     pos = {r: j for j, r in enumerate(reps)}
     sub = _bfgs_batch([pred_strs[r] for r in reps], X, y, cfg, test_data,
                       x0=None if x0 is None else [x0[r] for r in reps], engine=engine, lazy_strings=lazy_strings,
-                      w=w)
+                      w=w, rl=rl)
     out = []
     for i, r in enumerate(rep_of):
         res = sub[pos[r]]
@@ -558,7 +569,7 @@ def bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strin
     return out
 
 
-def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False, w=None):
+def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_strings=False, w=None, rl=None):
     """Fit every candidate of a beam in one go.
 
     Returns a list with one entry per candidate: the reference's 4-tuple
@@ -567,7 +578,7 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
     ``[R, k]`` starting points; default is the reference's ``np.random.randn(k) * 10``
     per restart (bfgs.py:103).  ``lazy_strings``: ``best_expr_str`` of every candidate is a
     ``LazyStr`` (printed through sympy when read) instead of a ``str``.  ``w``: per-point weights
-    (``sigma_weights``) or ``None``.
+    (``sigma_weights``) or ``None``.  ``rl``: the robust loss (``fitter.robust_loss``) or ``None``.
     """
     import time as _time
     _t = [_time.perf_counter()]
@@ -625,7 +636,7 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
         devices[0] if devices else (Xt.device if Xt.is_cuda else None))
     score_dtype = fitter.F32 if Xt.dtype == torch.float32 else fitter.F64
     eval_dtype = fitter.F32 if str(_opt(cfg, "precision", "fp64")).lower() == "fp32" else fitter.F64
-    eng.set_points(Xt[0], yt_fit, dtypes=tuple({eval_dtype, score_dtype, fitter.F64}), w=w)
+    eng.set_points(Xt[0], yt_fit, dtypes=tuple({eval_dtype, score_dtype, fitter.F64}), w=w, loss=rl)
     opts = _engine_opts(cfg, scale, eval_dtype, score_dtype)
     main_stream = torch.cuda.current_stream(eng.device)
     points_ready = torch.cuda.Event()
@@ -893,11 +904,11 @@ def _bfgs_batch(pred_strs, X, y, cfg, test_data, x0=None, engine=None, lazy_stri
     return results
 
 
-def bfgs(pred_str, X, y, cfg, test_data, x0=None, engine=None, sigma=None):
-    """Reference signature (bfgs.py:42): one candidate, raises what the reference raises.  ``sigma``: see
-    ``bfgs_batch``."""
+def bfgs(pred_str, X, y, cfg, test_data, x0=None, engine=None, sigma=None, loss="linear", f_scale=1.0):
+    """Reference signature (bfgs.py:42): one candidate, raises what the reference raises.  ``sigma``,
+    ``loss``, ``f_scale``: see ``bfgs_batch``."""
     out = bfgs_batch([pred_str], X, y, cfg, test_data,
-                     x0=None if x0 is None else [x0], engine=engine, sigma=sigma)[0]
+                     x0=None if x0 is None else [x0], engine=engine, sigma=sigma, loss=loss, f_scale=f_scale)[0]
     if isinstance(out, Exception):
         raise out
     return out

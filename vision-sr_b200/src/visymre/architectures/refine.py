@@ -16,6 +16,7 @@ repo's own package ``architectures/model.py`` re-exports it under the reference'
 import numpy as np
 import torch
 
+from ..engine import fitter
 from .bfgs import LazyStrings, bfgs, bfgs_batch, resolve_devices, sigma_weights
 
 UNARY_NAMES = ("abs", "asin", "cos", "exp", "ln", "sin", "sqrt", "tan")   # model.py:295
@@ -74,7 +75,8 @@ def _as_list(ww):
     return list(ww)
 
 
-def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None, sigma=None):
+def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None, sigma=None, loss="linear",
+                      f_scale=1.0):
     """The "BFGS Parallel Part" of fitfunc2 (model.py:444-520).
 
     ``hyps``: ``generated_hyps.hyp``, a list of ``(score, tokens)``; ``X`` ``[1, N, 10]``
@@ -84,7 +86,8 @@ def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None, s
     over several GPUs of this process (``bfgs.resolve_devices``); an invalid value raises
     ``ValueError`` here instead of failing every candidate.  ``sigma``: per-point standard deviations
     of ``y`` (1-D, N entries, any device) for weighted fits, see ``bfgs.bfgs_batch``; a bad ``sigma``
-    raises ``ValueError`` here as well.
+    raises ``ValueError`` here as well.  ``loss``, ``f_scale``: a robust loss (see ``bfgs.bfgs_batch``); the
+    candidates are then fitted and ranked by the robust objective, and a bad value raises ``ValueError``.
     """
     w2i = test_data.word2id
     arity_1 = {w2i[n] for n in UNARY_NAMES if n in w2i}
@@ -116,9 +119,10 @@ def refine_hypotheses(hyps, X, y, cfg_params, test_data, x0=None, engine=None, s
     if valid:
         resolve_devices(cfg_params)     # a wrong cfg.bfgs.devices is the caller's error, not every candidate's
         sigma_weights(sigma, X, cfg_params)   # so is a wrong sigma
+        fitter.robust_loss(loss, f_scale)     # and a wrong loss
         try:
             outs = bfgs_batch(valid, X, y, cfg_params, test_data, x0=x0, engine=engine, lazy_strings=True,
-                              sigma=sigma)
+                              sigma=sigma, loss=loss, f_scale=f_scale)
         except Exception as exc:  # noqa: BLE001 -- a batch-level failure fails every candidate
             outs = [exc] * len(valid)
         P_bfgs = LazyStrings()   # every string the reference returns; printed when read

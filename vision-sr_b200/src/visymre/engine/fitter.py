@@ -4,6 +4,8 @@
 used for device memory and streams only; every number is produced by libvsr.so.
 """
 import ctypes
+import math
+import sys
 from dataclasses import dataclass
 
 import numpy as np
@@ -57,6 +59,29 @@ def _check_weights(w, dtypes):
             raise ValueError(f"a weight 1/sigma^2 is not a finite normal {td} number at every point")
 
 
+# scipy.optimize.least_squares' `loss` names of the robust losses (vsr_set_loss), linear first
+LOSSES = ("linear", "soft_l1", "huber", "cauchy", "arctan")
+
+
+def robust_loss(loss="linear", f_scale=1.0):
+    """The validated ``(loss, f_scale)`` of a fit, ``None`` for ``loss="linear"`` (today's sum of squares).
+    ``loss`` is one of ``LOSSES``; ``f_scale`` (C) is a finite number > 0 whose ``C**2`` and ``1 / C**2``
+    are finite normal doubles.  Raises ``ValueError`` otherwise."""
+    if not isinstance(loss, str) or loss not in LOSSES:
+        raise ValueError(f"loss must be one of {LOSSES}, got {loss!r}")
+    try:
+        c = float(f_scale)
+    except (TypeError, ValueError):
+        raise ValueError(f"f_scale must be a number, got {f_scale!r}") from None
+    if not (math.isfinite(c) and c > 0):
+        raise ValueError(f"f_scale must be finite and > 0, got {f_scale!r}")
+    c2 = c * c
+    if not (math.isfinite(c2) and c2 >= sys.float_info.min and math.isfinite(1.0 / c2)
+            and 1.0 / c2 >= sys.float_info.min):
+        raise ValueError(f"f_scale {c!r}: f_scale**2 and 1/f_scale**2 must be finite normal doubles")
+    return None if loss == "linear" else (loss, c)
+
+
 def default_opts(**over):
     lib = native.load()
     o = native.FitOpts()
@@ -86,6 +111,7 @@ class Engine:
         self._weights = {}     # dtype -> w [N] tensor kept alive (weighted points only)
         self._src = None       # (X2d, y1d) as given, for re-uploads with more columns
         self._w_src = None     # fp64 weights as given (None: unweighted)
+        self._loss = None      # robust loss (name, f_scale) of every slot (None: linear)
         self.n_points = 0
         self.n_vars = 0
         self.programs = []
@@ -135,7 +161,7 @@ class Engine:
         return tuple(out)
 
     # ---- points ----------------------------------------------------------------------
-    def set_points(self, X, y, dtypes=(F64,), n_vars=None, w=None):
+    def set_points(self, X, y, dtypes=(F64,), n_vars=None, w=None, loss=None):
         """X: [N, d] (or [1, N, d]) tensor/array on any device; y: squeezable to [N].
 
         Columns are stored column-major on the device, one copy per requested dtype.
@@ -143,7 +169,11 @@ class Engine:
         ``w``: optional per-point weights [N] (``vsr_set_weights``), stored in every dtype slot; the fit,
         ``eval`` and ``gram`` then use ``sum w r^2``.  ``ValueError`` when a weight is not a finite normal
         number > 0 in a requested dtype.
+        ``loss``: optional robust loss ``(name, f_scale)`` (``vsr_set_loss``, names of ``LOSSES``), stored in
+        every dtype slot; the fit, ``eval`` and ``gram`` then use ``sum C^2 rho(w r^2 / C^2)``.  ``None`` or
+        ``("linear", ...)``: the sum of squares.  ``ValueError`` for an unknown name or a bad ``f_scale``.
         """
+        loss = robust_loss(*loss) if loss is not None else None
         X = torch.as_tensor(X)
         y = torch.as_tensor(y)
         if X.dim() == 3:
@@ -163,6 +193,7 @@ class Engine:
             _check_weights(w, dtypes)
         self._src = (X, y)
         self._w_src = w
+        self._loss = loss
         self.n_points = int(X.shape[0])
         if n_vars is None:
             nz = (X != 0).any(dim=0).nonzero()
@@ -187,13 +218,21 @@ class Engine:
             for dt in self._want_dtypes:
                 self._weights[dt] = self._w_src.to(_TORCH_DTYPE[dt]).contiguous()
                 self._check(self.lib.vsr_set_weights(self._h, _ptr(self._weights[dt]), N, dt))
+        for dt in self._want_dtypes:
+            self._set_loss(dt)
         self.n_vars = n_vars
+
+    def _set_loss(self, dt):
+        if self._loss is not None:
+            name, c = self._loss
+            self._check(self.lib.vsr_set_loss(self._h, isa.LOSS["VSR_LOSS_" + name.upper()], c, dt))
 
     def adopt_points(self, other):
         """Use the points another engine of the same device holds (no copy: the same device tensors
         are registered with this handle): engines that fit parts of one beam concurrently."""
         self._src = other._src
         self._w_src = other._w_src
+        self._loss = other._loss
         self.n_points = other.n_points
         self.n_vars = other.n_vars
         self._want_dtypes = tuple(other._want_dtypes)
@@ -204,6 +243,7 @@ class Engine:
                                                 self.n_vars, dt))
             if dt in self._weights:
                 self._check(self.lib.vsr_set_weights(self._h, _ptr(self._weights[dt]), self.n_points, dt))
+            self._set_loss(dt)
 
     def ensure_dtype(self, dt):
         if dt not in self._points:
@@ -465,7 +505,7 @@ def device_engines(devices, home=None):
 
 
 def share_points(engines):
-    """Give every engine the points (and weights) ``engines[0]`` holds (``set_points`` was called on it).  Each other
+    """Give every engine the points (weights and loss) ``engines[0]`` holds (``set_points`` was called on it).  Each other
     device gets one copy, made from the home device's tensors: a peer copy on the home stream that torch
     orders before the device's own stream.  Further engines of a device adopt that device's copy."""
     home = engines[0]
@@ -476,5 +516,5 @@ def share_points(engines):
             eng.adopt_points(holder[eng.device])
             continue
         with torch.cuda.device(eng.device):
-            eng.set_points(X, y, dtypes=home._want_dtypes, n_vars=home.n_vars, w=home._w_src)
+            eng.set_points(X, y, dtypes=home._want_dtypes, n_vars=home.n_vars, w=home._w_src, loss=home._loss)
         holder[eng.device] = eng

@@ -52,6 +52,7 @@ SRC = _ENUMS["VsrSrc"]
 FIT_STATUS = _ENUMS["VsrFitStatus"]
 GRAD_MODE = _ENUMS["VsrGradMode"]
 DTYPE = _ENUMS["VsrDtype"]
+LOSS = _ENUMS["VsrLoss"]
 OP_NAME = {v: k for k, v in OP.items()}
 SRC_NAME = {v: k for k, v in SRC.items()}
 

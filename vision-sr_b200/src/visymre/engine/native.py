@@ -61,6 +61,7 @@ SIGNATURES = {
     "vsr_upload_points": (ctypes.c_int, [vp, vp, vp, ctypes.c_int64, ctypes.c_int64,
                                          ctypes.c_int32, ctypes.c_int32, vp]),
     "vsr_set_weights": (ctypes.c_int, [vp, vp, ctypes.c_int64, ctypes.c_int32]),
+    "vsr_set_loss": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_double, ctypes.c_int32]),
     "vsr_upload_programs": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int32, vp]),
     "vsr_eval": (ctypes.c_int, [vp, vp, vp, ctypes.c_int32, vp, ctypes.c_int32, ctypes.c_int32,
                                 vp, vp, vp]),

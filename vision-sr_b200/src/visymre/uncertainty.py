@@ -50,6 +50,17 @@ The rank test and the ``inf`` rules above apply unchanged.  For the prediction b
 whose sigma is ``sigma_new``, the noise term is ``s^2 sigma_new^2`` for a relative covariance (the default
 ``sigma_new = 1`` gives ``s^2``) and ``sigma_new^2`` for an absolute one, whose bands use the normal
 quantile instead of Student's t because the scale is known.
+
+Robust losses (curve_fit's ``loss`` and ``f_scale``, which it passes to ``least_squares``).  With
+``z_i = w_i r_i^2 / C^2`` (``C = f_scale``), one robust ``vsr_gram`` launch gives least_squares'
+statistics at the fitted point::
+
+    rss = sum C^2 rho(z_i)                                  (curve_fit's cost = 2 res.cost)
+    jtj = J^T W S J,  S = diag(max(rho'(z_i) + 2 z_i rho''(z_i), 2^-52))   (its scaled Jacobian)
+
+and ``covariance_from_gram`` applies unchanged: ``cov = s^2 jtj^-1`` with ``s^2 = rss / dof``, or
+``jtj^-1`` with ``absolute_sigma``.  So ``rss`` holds the robust cost, and the ``s^2`` that ``predict``
+and ``bands`` take from it for the prediction band is curve_fit's ``s_sq`` under that loss.
 """
 from dataclasses import dataclass
 from typing import Optional
@@ -74,11 +85,13 @@ class ConstantCovariance:
     free: np.ndarray     # [k] bool: False for a constant the prune fixed at 0.0
     cov: np.ndarray      # [k, k] covariance; nan in rows / columns of fixed constants
     stderr: np.ndarray   # [k] sqrt(diag(cov))
-    rss: float           # sum of squared residuals at consts
+    rss: float           # sum of squared residuals at consts (sum C^2 rho(z) under a robust loss)
     dof: int             # N - number of free constants
     rank: int            # numerical rank of J^T J over the free constants
-    jtj: np.ndarray      # [k, k] J^T J over all constants
+    jtj: np.ndarray      # [k, k] J^T J over all constants (J^T W S J under weights and a robust loss)
     absolute_sigma: bool = False   # cov = (J^T W J)^-1 without the s^2 factor (see the module docstring)
+    loss: str = "linear"           # the robust loss of the statistics (module docstring)
+    f_scale: float = 1.0
 
 
 def covariance_from_gram(rss, jtj, n, free, absolute_sigma=False):
@@ -126,7 +139,7 @@ def _compile(items):
     return out
 
 
-def covariances(fits, X, y, engine=None, sigma=None, absolute_sigma=False):
+def covariances(fits, X, y, engine=None, sigma=None, absolute_sigma=False, loss="linear", f_scale=1.0):
     """Covariance of the constants of every fit of ``fits``.
 
     ``fits``: ``bfgs()`` / ``bfgs_batch()`` 4-tuples ``(string, consts, loss, skeleton)``; an
@@ -137,12 +150,15 @@ def covariances(fits, X, y, engine=None, sigma=None, absolute_sigma=False):
     replaced.  ``sigma``: optional 1-D per-point standard deviations of ``y`` (N entries, any device), as
     curve_fit's ``sigma``; ``absolute_sigma``: curve_fit's flag (module docstring).  ``ValueError`` for a
     bad ``sigma`` (wrong length, not finite and > 0, ``1/sigma^2`` not a finite normal fp64 number).
+    ``loss``, ``f_scale``: curve_fit's robust loss (``fitter.robust_loss``; module docstring), ``ValueError``
+    for a bad one.
     """
     X = torch.as_tensor(X)
     if X.dim() == 3:
         X = X[0]
     y = torch.as_tensor(y).reshape(-1)
     w = fitter.weights_from_sigma(sigma, X.shape[0], (fitter.F64,)) if sigma is not None else None
+    rl = fitter.robust_loss(loss, f_scale)
     out = [None] * len(fits)
     items = []
     for i, f in enumerate(fits):
@@ -153,7 +169,8 @@ def covariances(fits, X, y, engine=None, sigma=None, absolute_sigma=False):
         return out
     progs = _compile([(skel, c.shape[0]) for _, skel, c in items])
     eng = engine if engine is not None else fitter.get_engine(X.device if X.is_cuda else None)
-    eng.set_points(X, y, dtypes=(fitter.F64,), n_vars=max(1, max(p.var_mask.bit_length() for p in progs)), w=w)
+    eng.set_points(X, y, dtypes=(fitter.F64,), n_vars=max(1, max(p.var_mask.bit_length() for p in progs)), w=w,
+                   loss=rl)
     eng.set_programs(progs)
     consts = np.zeros((len(items), max(1, max(c.shape[0] for _, _, c in items))))
     for j, (_, _, c) in enumerate(items):
@@ -167,7 +184,8 @@ def covariances(fits, X, y, engine=None, sigma=None, absolute_sigma=False):
         g = jtj[j, :k, :k].copy()
         cov, stderr, dof, rank = covariance_from_gram(rss[j], g, n, free, absolute_sigma)
         out[i] = ConstantCovariance(consts=c, free=free, cov=cov, stderr=stderr, rss=float(rss[j]),
-                                    dof=dof, rank=rank, jtj=g, absolute_sigma=bool(absolute_sigma))
+                                    dof=dof, rank=rank, jtj=g, absolute_sigma=bool(absolute_sigma), loss=loss,
+                                    f_scale=float(f_scale))
     return out
 
 
