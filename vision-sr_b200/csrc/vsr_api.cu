@@ -8,6 +8,8 @@
 #include <cstring>
 #include <string>
 #include <mutex>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/vsr.h"
@@ -18,6 +20,19 @@ namespace {
 
 constexpr int kWidths[] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 12, 16};
 constexpr int kNumWidths = sizeof(kWidths) / sizeof(kWidths[0]);
+
+// Calls f(std::integral_constant<int, KK>{}) for the compiled tangent width KK == K and returns its result
+// (`otherwise` for a width without kernels): the one dispatch from a run-time width to the instantiations.
+template <typename R, typename F, size_t... I>
+R with_width(int K, R otherwise, F&& f, std::index_sequence<I...>) {
+  R r = otherwise;
+  (void)((K == kWidths[I] && (r = f(std::integral_constant<int, kWidths[I]>{}), true)) || ...);
+  return r;
+}
+template <typename R, typename F>
+R with_width(int K, R otherwise, F&& f) {
+  return with_width(K, otherwise, f, std::make_index_sequence<kNumWidths>{});
+}
 
 int pick_width(int k) {
   for (int w : kWidths)
@@ -77,11 +92,13 @@ struct PinnedBuf {
   }
 };
 
+// no weights, linear loss: the loss of a slot after vsr_set_points / vsr_upload_points
+constexpr vsr::PointLoss kLinearLoss{nullptr, {VSR_LOSS_LINEAR, 1.0, 1.0}};
+
 struct PointSlot {
   const void* X = nullptr;
   const void* y = nullptr;
-  const void* w = nullptr;  // per-point weights (vsr_set_weights), nullptr: unweighted
-  vsr::RobustLoss loss{VSR_LOSS_LINEAR, 1.0, 1.0};  // vsr_set_loss
+  vsr::PointLoss pl = kLinearLoss;  // weights (vsr_set_weights) and loss (vsr_set_loss)
   int64_t n = 0, ldx = 0;
   int n_vars = 0;
   DevBuf ownX, ownY;
@@ -194,8 +211,24 @@ vsr::ProgramTable table_of(const vsr_handle* h) {
   return t;
 }
 
-// the slot's robust loss for a launch (nullptr: linear, which takes today's kernels)
-const vsr::RobustLoss* robust_of(const PointSlot& s) { return s.loss.kind != VSR_LOSS_LINEAR ? &s.loss : nullptr; }
+// the kernels of a slot's loss: robust with a robust loss (weighted or not), else weighted with weights
+vsr::LossMode mode_of(const vsr::PointLoss& pl) {
+  if (pl.loss.kind != VSR_LOSS_LINEAR) return vsr::LossMode::kRobust;
+  return pl.w ? vsr::LossMode::kWeighted : vsr::LossMode::kLinear;
+}
+
+// calls f(KK, M) for the compiled tangent width KK == K and the mode M of pl (see with_width)
+template <typename F>
+cudaError_t with_kernel(int K, const vsr::PointLoss& pl, F&& f) {
+  using vsr::LossMode;
+  return with_width(K, cudaErrorInvalidValue, [&](auto KK) {
+    switch (mode_of(pl)) {
+      case LossMode::kRobust: return f(KK, std::integral_constant<LossMode, LossMode::kRobust>{});
+      case LossMode::kWeighted: return f(KK, std::integral_constant<LossMode, LossMode::kWeighted>{});
+      default: return f(KK, std::integral_constant<LossMode, LossMode::kLinear>{});
+    }
+  });
+}
 
 vsr::Points points_of(const PointSlot& s) {
   vsr::Points p;
@@ -208,86 +241,44 @@ vsr::Points points_of(const PointSlot& s) {
 
 using vsr::points_per_thread;
 
-// the kernels are instantiated one (type, width) pair per translation unit (vsr_inst.cu) so the
-// library builds in parallel; here only the dispatch over the runtime width (and, with a robust loss
-// rl != nullptr, to the RB kernels)
+// the kernels are instantiated one (type, width, mode) per translation unit (vsr_inst.cu) so the
+// library builds in parallel; here only the dispatch over the runtime width and the slot's loss
 template <typename T>
 cudaError_t launch_fit(int K, const vsr::FitArgs& a, int threads, int cs, size_t smem, int clusters, cudaStream_t st,
-                       const void* w, const vsr::RobustLoss* rl) {
-  switch (K) {
-#define C(KK)                                                                                      \
-  case KK:                                                                                         \
-    return rl ? vsr::launch_fit_rb_T<T, KK>(a, threads, cs, smem, clusters, st, w, *rl)            \
-              : vsr::launch_fit_T<T, KK>(a, threads, cs, smem, clusters, st, w);
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return cudaErrorInvalidValue;
+                       const vsr::PointLoss& pl) {
+  return with_kernel(K, pl, [&](auto KK, auto M) {
+    return vsr::launch_fit_T<T, KK, M>(a, threads, cs, smem, clusters, st, pl);
+  });
 }
 
 template <typename T>
 int fit_threads_cap(int K) {
-  switch (K) {
-#define C(KK) case KK: return vsr::fit_max_threads<T, KK>();
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return 256;
+  return with_width(K, 256, [](auto KK) { return vsr::fit_max_threads<T, KK>(); });
 }
 
 template <typename T>
-cudaError_t launch_eval(int K, const vsr::EvalArgs& a, int threads, size_t smem, cudaStream_t st, const void* w,
-                        const vsr::RobustLoss* rl) {
-  switch (K) {
-#define C(KK)                                                                                        \
-  case KK:                                                                                           \
-    return rl ? vsr::launch_eval_rb_T<T, KK>(a, threads, smem, st, w, *rl) : vsr::launch_eval_T<T, KK>(a, threads, smem, st, w);
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return cudaErrorInvalidValue;
+cudaError_t launch_eval(int K, const vsr::EvalArgs& a, int threads, size_t smem, cudaStream_t st,
+                        const vsr::PointLoss& pl) {
+  return with_kernel(K, pl, [&](auto KK, auto M) { return vsr::launch_eval_T<T, KK, M>(a, threads, smem, st, pl); });
 }
 
 template <typename T>
-cudaError_t launch_eval_tile(int K, const vsr::EvalTileArgs& a, size_t smem, cudaStream_t st, const void* w,
-                             const vsr::RobustLoss* rl) {
-  switch (K) {
-#define C(KK)                                                                                 \
-  case KK:                                                                                    \
-    return rl ? vsr::launch_eval_tile_rb_T<T, KK>(a, smem, st, w, *rl) : vsr::launch_eval_tile_T<T, KK>(a, smem, st, w);
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return cudaErrorInvalidValue;
+cudaError_t launch_eval_tile(int K, const vsr::EvalTileArgs& a, size_t smem, cudaStream_t st,
+                             const vsr::PointLoss& pl) {
+  return with_kernel(K, pl, [&](auto KK, auto M) { return vsr::launch_eval_tile_T<T, KK, M>(a, smem, st, pl); });
 }
 
 template <typename T>
 cudaError_t launch_predict(int K, const vsr::PredictArgs& a, size_t smem, cudaStream_t st) {
-  switch (K) {
-#define C(KK) case KK: return vsr::launch_predict_T<T, KK>(a, smem, st);
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return cudaErrorInvalidValue;
+  return with_width(K, cudaErrorInvalidValue, [&](auto KK) { return vsr::launch_predict_T<T, KK>(a, smem, st); });
 }
 
-cudaError_t launch_gram(int K, const vsr::GramArgs& a, size_t smem, cudaStream_t st, const void* w,
-                        const vsr::RobustLoss* rl) {
-  switch (K) {
-#define C(KK) case KK: return rl ? vsr::launch_gram_rb_K<KK>(a, smem, st, w, *rl) : vsr::launch_gram_K<KK>(a, smem, st, w);
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return cudaErrorInvalidValue;
+cudaError_t launch_gram(int K, const vsr::GramArgs& a, size_t smem, cudaStream_t st, const vsr::PointLoss& pl) {
+  return with_kernel(K, pl, [&](auto KK, auto M) { return vsr::launch_gram_K<KK, M>(a, smem, st, pl); });
 }
 
 int eval_tile_threads_of(int K) {
-  switch (K) {
-#define C(KK) case KK: return vsr::eval_tile_threads<KK>();
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
-  }
-  return 512;
+  return with_width(K, 512, [](auto KK) { return vsr::eval_tile_threads<KK>(); });
 }
 
 int next_pow2(int64_t v) {
@@ -391,10 +382,10 @@ int stage_lists(vsr_handle* h, const std::vector<int32_t>& all, cudaStream_t st)
 int run_eval_group(vsr_handle* h, int K, int dtype, const int32_t* d_prog, const int32_t* d_row,
                    const int32_t* d_out, int n_pairs, int kmax, int max_insn, int max_imm,
                    const double* consts, int kstride, double* out_loss, double* out_grad,
-                   cudaStream_t st, int nan_to_num = 0, unsigned var_mask = 0, const void* w = nullptr,
-                   const vsr::RobustLoss* rl = nullptr) {
-  // w: the slot's weights for a weighted loss and gradient (nullptr: unweighted); rl: its robust loss
-  // (nullptr: linear).  A robust launch has the geometry and staging of the linear one.
+                   cudaStream_t st, int nan_to_num = 0, unsigned var_mask = 0,
+                   const vsr::PointLoss& pl = kLinearLoss) {
+  // pl: the slot's weights and loss (vsr_score: linear).  Weighted and robust launches have the geometry
+  // and staging of the linear one.
   const PointSlot& ps = h->pts[dtype];
   const int P = points_per_thread(K);
   const int64_t N = ps.n;
@@ -436,8 +427,8 @@ int run_eval_group(vsr_handle* h, int K, int dtype, const int32_t* d_prog, const
       // (a weighted launch reads the weights from global memory: the same chunks, so w = 1 gives the
       // unweighted sums bit for bit)
       const size_t smem = fixed + (size_t)(t.n_cols + 1) * chunk * elem;
-      cudaError_t e = dtype == VSR_F64 ? launch_eval_tile<double>(K, t, smem, st, w, rl)
-                                         : launch_eval_tile<float>(K, t, smem, st, w, rl);
+      cudaError_t e = dtype == VSR_F64 ? launch_eval_tile<double>(K, t, smem, st, pl)
+                                         : launch_eval_tile<float>(K, t, smem, st, pl);
       if (e != cudaSuccess) return fail(h, VSR_ECUDA, "eval tile kernel launch failed (smem %zu): %s", smem, cudaGetErrorString(e));
       const int total = n_pairs * (K + 1);
       vsr::eval_finalize<<<(total + 127) / 128, 128, 0, st>>>(t.e.partial, d_prog, d_out, t.e.pt.k, n_pairs, (int)chunks, K,
@@ -469,8 +460,8 @@ int run_eval_group(vsr_handle* h, int K, int dtype, const int32_t* d_prog, const
   a.nsplit = nsplit;
   a.nan_to_num = nan_to_num;
   const size_t smem = sizeof(double) * (size_t)((K + 1) * threads + kmax + 2 + max_imm + max_insn + 1);  // + pad word
-  cudaError_t e = dtype == VSR_F64 ? launch_eval<double>(K, a, threads, smem, st, w, rl)
-                                   : launch_eval<float>(K, a, threads, smem, st, w, rl);
+  cudaError_t e = dtype == VSR_F64 ? launch_eval<double>(K, a, threads, smem, st, pl)
+                                   : launch_eval<float>(K, a, threads, smem, st, pl);
   if (e != cudaSuccess) return fail(h, VSR_ECUDA, "eval kernel launch failed: %s", cudaGetErrorString(e));
   const int total = n_pairs * (K + 1);
   vsr::eval_finalize<<<(total + 127) / 128, 128, 0, st>>>(
@@ -543,11 +534,12 @@ int vsr_create(int device, vsr_handle** out) {
   // the 44 kernels would otherwise stall a fit by milliseconds), once per process and device.
   static bool preloaded[64] = {false};
   if (device < 64 && !preloaded[device]) {
-#define C(KK)                                                        \
-  if (e == cudaSuccess) e = vsr::preload_T<double, KK>();            \
-  if (e == cudaSuccess) e = vsr::preload_T<float, KK>();
-    C(0) C(1) C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(12) C(16)
-#undef C
+    for (int K : kWidths)
+      if (e == cudaSuccess)
+        e = with_width(K, cudaErrorInvalidValue, [](auto KK) {
+          cudaError_t r = vsr::preload_T<double, KK>();
+          return r == cudaSuccess ? vsr::preload_T<float, KK>() : r;
+        });
     if (e != cudaSuccess) return fail(nullptr, VSR_ECUDA, "loading the kernels: %s", cudaGetErrorString(e));
     preloaded[device] = true;
   }
@@ -680,8 +672,7 @@ int vsr_set_points(vsr_handle* h, const void* X_dev, const void* y_dev, int64_t 
   PointSlot& s = h->pts[dtype];
   s.X = X_dev;
   s.y = y_dev;
-  s.w = nullptr;
-  s.loss = vsr::RobustLoss{VSR_LOSS_LINEAR, 1.0, 1.0};
+  s.pl = kLinearLoss;
   s.n = n_points;
   s.ldx = ldx;
   s.n_vars = n_vars;
@@ -708,8 +699,7 @@ int vsr_upload_points(vsr_handle* h, const void* X_host, const void* y_host, int
   VSR_CUDA(h, cudaMemcpyAsync(s.ownY.p, y_host, n_points * es, cudaMemcpyHostToDevice, st));
   s.X = s.ownX.p;
   s.y = s.ownY.p;
-  s.w = nullptr;
-  s.loss = vsr::RobustLoss{VSR_LOSS_LINEAR, 1.0, 1.0};
+  s.pl = kLinearLoss;
   s.n = n_points;
   s.ldx = dld;
   s.n_vars = n_vars;
@@ -723,7 +713,7 @@ int vsr_set_weights(vsr_handle* h, const void* w_dev, int64_t n_points, int32_t 
   if (!s.X || s.n <= 0) return fail(h, VSR_ESTATE, "no points uploaded for dtype %d", dtype);
   if (w_dev && n_points != s.n)
     return fail(h, VSR_EINVAL, "%lld weights for %lld points (dtype %d)", (long long)n_points, (long long)s.n, dtype);
-  s.w = w_dev;
+  s.pl.w = w_dev;
   return VSR_OK;
 }
 
@@ -736,7 +726,7 @@ int vsr_set_loss(vsr_handle* h, int32_t loss, double f_scale, int32_t dtype) {
     return fail(h, VSR_EINVAL, "f_scale %g: its square or inverse square is not a normal double", f_scale);
   PointSlot& s = h->pts[dtype];
   if (!s.X || s.n <= 0) return fail(h, VSR_ESTATE, "no points uploaded for dtype %d", dtype);
-  s.loss = vsr::RobustLoss{loss, c2, inv_c2};
+  s.pl.loss = vsr::RobustLoss{loss, c2, inv_c2};
   return VSR_OK;
 }
 
@@ -878,7 +868,7 @@ int vsr_eval(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, i
     if (!n) continue;
     rc = run_eval_group(h, g.K, dtype, dl + off[gi], dl + off[gi] + n, dl + off[gi] + 2 * n, n,
                         g.kmax, g.max_insn, g.max_imm, consts, kstride, out_loss,
-                        g.K > 0 ? out_grad : nullptr, st, 0, g.var_mask, h->pts[dtype].w, robust_of(h->pts[dtype]));
+                        g.K > 0 ? out_grad : nullptr, st, 0, g.var_mask, h->pts[dtype].pl);
     if (rc) return rc;
   }
   if (out_grad && !toowide.prog.empty()) {
@@ -960,10 +950,12 @@ int vsr_gram(vsr_handle* h, const int32_t* prog_idx, const int32_t* const_row, i
     a.consts = consts;
     a.partial = partial;
     a.nsplit = vsr::gram_nsplit(ps.n, tile);
-    const size_t cols = (size_t)(K + 1) + (robust_of(ps) ? 2 : (ps.w ? 1 : 0));  // r, J (and w, or wq and ws)
+    // r, J, then the factor columns: w (weighted), or wq and ws (robust)
+    const vsr::LossMode mode = mode_of(ps.pl);
+    const size_t cols = (size_t)(K + 1) + (mode == vsr::LossMode::kRobust ? 2 : mode == vsr::LossMode::kWeighted ? 1 : 0);
     const size_t smem = sizeof(double) * (cols * vsr::gram_col_stride(tile) + g.kmax + 1 + g.max_imm) +
                         sizeof(vsr_insn_t) * (g.max_insn + 1);
-    cudaError_t e = launch_gram(K, a, smem, st, ps.w, robust_of(ps));
+    cudaError_t e = launch_gram(K, a, smem, st, ps.pl);
     if (e != cudaSuccess) return fail(h, VSR_ECUDA, "gram kernel launch failed: %s", cudaGetErrorString(e));
     const int64_t total = (int64_t)n * (1 + (int64_t)kstride * kstride);
     vsr::gram_finalize<<<(unsigned)((total + 127) / 128), 128, 0, st>>>(partial, a.pair_prog, dl + off[gi] + 2 * n,
@@ -1199,7 +1191,7 @@ int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int
   const PointSlot& ps = h->pts[opts->eval_dtype];
   const int elem = opts->eval_dtype == VSR_F64 ? 8 : 4;
   const bool tma_ok = ((uintptr_t)ps.X % 16 == 0) && ((uintptr_t)ps.y % 16 == 0) && ((ps.ldx * elem) % 16 == 0) &&
-                      ((uintptr_t)ps.w % 16 == 0);
+                      ((uintptr_t)ps.pl.w % 16 == 0);
   cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_c = nullptr;
   if (h->profiling) {
     ev_a = take_event(h);
@@ -1279,7 +1271,7 @@ int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int
     g.max_insn = all_insn;
     // a weighted launch stages one column more (the weights) into a resident slice
     Geometry geo = choose_geometry(g.kmax == 0 ? 1 : ps.n, P, cap, opts->warps_per_run, g.kmax, g.K, g.max_insn,
-                                   n_cols + (ps.w ? 1 : 0), elem, max_cluster,
+                                   n_cols + (ps.pl.w ? 1 : 0), elem, max_cluster,
                                    hook_seats > 0 ? hook_seats : kDefaultSeats, hook_reserved);
     if (g.kmax == 0) {  // runs without constants are only marked "not run": no points needed
       geo.resident = 0;
@@ -1308,10 +1300,8 @@ int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int
     a.queue = (int32_t*)h->d_queue.p + gi;
     const int want_clusters = (n + geo.seats - 1) / geo.seats;
     cudaError_t e = opts->eval_dtype == VSR_F64
-                        ? launch_fit<double>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.w,
-                                             robust_of(ps))
-                        : launch_fit<float>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.w,
-                                            robust_of(ps));
+                        ? launch_fit<double>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.pl)
+                        : launch_fit<float>(g.K, a, geo.threads, geo.cs, geo.smem, want_clusters, gs, ps.pl);
     if (e != cudaSuccess)
       return fail(h, VSR_ECUDA, "fit kernel launch failed (K=%d threads=%d cluster=%d seats=%d smem=%zu): %s", g.K,
                   geo.threads, geo.cs, geo.seats, geo.smem, cudaGetErrorString(e));
@@ -1326,8 +1316,7 @@ int vsr_fit(vsr_handle* h, const int32_t* run_prog, const int32_t* run_slot, int
   // weights on the score slot the weighted mean of w r^2, with a robust loss the mean cost C^2 rho(z)
   rc = run_eval_group(h, 0, opts->score_dtype, dl + score_off, dl + score_off + n_runs,
                       dl + score_off + n_runs, n_runs, s_kmax, s_insn, s_imm, out_lastx, kstride,
-                      out_final_mse, nullptr, st, 0, 0, h->pts[opts->score_dtype].w,
-                      robust_of(h->pts[opts->score_dtype]));
+                      out_final_mse, nullptr, st, 0, 0, h->pts[opts->score_dtype].pl);
   if (h->profiling) {
     VSR_CUDA(h, cudaEventRecord(ev_c, st));
     h->spans.push_back({ev_a, ev_b, 0, (int)groups.size()});

@@ -130,30 +130,30 @@ struct EvalArgs {
   int32_t nan_to_num;  // 1: predictions pass through numpy's nan_to_num before the residual (vsr_score)
 };
 
-// Kernel arguments of a weighted launch (W = true): the argument struct A with the per-point weights
-// w_i of the slot (the slot's element type, like y) as its LAST member, so that every member of A keeps
-// its parameter offset.  Weighted<A, false> is A itself: the unweighted kernels are unchanged.
-template <typename A, bool W>
-struct Weighted : A {
-  const void* w;
-};
-template <typename A>
-struct Weighted<A, false> : A {};
-
 // Robust loss of a point slot (vsr_set_loss): kind (VsrLoss), C^2 and 1/C^2 of f_scale C.
 struct RobustLoss {
   int32_t kind;
   double c2, inv_c2;
 };
 
-// Kernel arguments of a robust launch (RB = true): the weighted struct with the loss appended last.  In a
-// robust kernel the weight pointer is optional at run time (nullptr: unweighted).
-template <typename A>
-struct Robust : Weighted<A, true> {
+// The point objective a fit, eval, eval-tile or Gram kernel is compiled for: sum r^2 (kLinear), sum w r^2
+// with per-point weights w_i (kWeighted), or a robust loss sum C^2 rho(w r^2 / C^2) (kRobust, weights
+// optional at run time).
+enum class LossMode { kLinear, kWeighted, kRobust };
+
+// Kernel arguments of a launch of mode M: the argument struct A, then the slot's weights (the slot's
+// element type, like y) and then its loss, so that every member of A keeps its parameter offset.
+template <typename A, LossMode M>
+struct LaunchArgs : A {  // kRobust
+  const void* w;         // nullptr: unweighted
   RobustLoss loss;
 };
-template <typename A, bool W, bool RB>
-using KernelArgs = std::conditional_t<RB, Robust<A>, Weighted<A, W>>;
+template <typename A>
+struct LaunchArgs<A, LossMode::kWeighted> : A {
+  const void* w;
+};
+template <typename A>
+struct LaunchArgs<A, LossMode::kLinear> : A {};
 
 // Per-point factors of a robust loss at z = w r^2 / C^2 (finite, >= 0), scipy's least_squares
 // definitions: q = rho(z) / z (the cost ratio, q(0) = 1), g = rho'(z), s = rho'(z) + 2 z rho''(z).  q is
@@ -197,7 +197,7 @@ __device__ __forceinline__ double robust_cost_inf(const RobustLoss& L) {
   return L.kind == VSR_LOSS_ARCTAN ? L.c2 * 1.5707963267948966 : __longlong_as_double(0x7ff0000000000000ll);
 }
 
-// Residual step of a robust sweep (RB): adds cost = C^2 rho(z) to ps as (rw * q) * r and rho'(z) rw d_t to
+// Residual step of a robust sweep (kRobust): adds cost = C^2 rho(z) to ps as (rw * q) * r and rho'(z) rw d_t to
 // pg[t], with rw = w r (r without weights).  A non-finite r contributes the linear terms rw r and rw d_t
 // (the penalty rule); a z that overflows from a finite r contributes scipy's rho(inf) and no gradient.  With
 // q = g = 1 the products are the linear step's, so huber with every z <= 1 gives its sums bit for bit.
@@ -254,10 +254,10 @@ __device__ __forceinline__ void keep_in_register(int& v) { asm volatile("" : "+r
 // converged for the reduction that follows.
 // NTN: the prediction passes through numpy's nan_to_num (nan -> 0, +-inf -> +-largest finite
 // value of T) before the residual is taken: the drivers' scoring rule (Feynman_test.py:87).
-// W: per-point weights w (fp64 arithmetic): sum w r^2 and sum w r df/dc_t.  rw = w * r is formed once and
-// every product is the unweighted one with r replaced by rw, so w = 1.0 gives the unweighted sums bit for bit.
-// RB: robust loss L (robust_step), weights optional (w = nullptr: rw = r).
-template <typename T, int K, int P, bool NTN = false, bool W = false, bool RB = false>
+// M (LossMode): kWeighted: per-point weights w (fp64 arithmetic): sum w r^2 and sum w r df/dc_t.  rw = w * r
+// is formed once and every product is the linear one with r replaced by rw, so w = 1.0 gives the linear sums
+// bit for bit.  kRobust: robust loss L (robust_step), weights optional (w = nullptr: rw = r).
+template <typename T, int K, int P, bool NTN = false, LossMode M = LossMode::kLinear>
 __device__ __forceinline__ void sweep_points(const vsr_insn_t* prog, const double* imm,
                                              const T* cst, const T* __restrict__ X,
                                              const T* __restrict__ y, int64_t ldx, int64_t n0,
@@ -291,9 +291,9 @@ __device__ __forceinline__ void sweep_points(const vsr_insn_t* prog, const doubl
           pv = pv != pv ? T(0) : (pv > big ? big : (pv < -big ? -big : pv));
         }
         const double r = (double)pv - (double)__ldg(y + xs.idx[p]);
-        if constexpr (RB) {
+        if constexpr (M == LossMode::kRobust) {
           robust_step<T, K>(L, r, w ? (double)__ldg(w + xs.idx[p]) * r : r, acc[p], ps, pg);
-        } else if constexpr (W) {
+        } else if constexpr (M == LossMode::kWeighted) {
           const double rw = (double)__ldg(w + xs.idx[p]) * r;
           ps += rw * r;
 #pragma unroll
@@ -467,8 +467,8 @@ struct SlicePoints {
 };
 
 // One pass over the resident slice (cnt points); partial sums parked like sweep_points does.
-// W: the weights are staged like y (ws, cnt values), same residual rule as sweep_points.  RB: as there.
-template <typename T, int K, int P, bool NTN = false, bool W = false, bool RB = false>
+// The weights (kWeighted, kRobust) are staged like y (ws, cnt values); same residual rule as sweep_points.
+template <typename T, int K, int P, bool NTN = false, LossMode M = LossMode::kLinear>
 __device__ __forceinline__ void sweep_slice(const vsr_insn_t* prog, const double* imm, const T* cst,
                                             const T* xs, const T* ys, int stride, int cnt, double* scratch,
                                             int tid, int nt, const T* ws = nullptr, RobustLoss L = {}) {
@@ -500,9 +500,9 @@ __device__ __forceinline__ void sweep_slice(const vsr_insn_t* prog, const double
           pv = pv != pv ? T(0) : (pv > big ? big : (pv < -big ? -big : pv));
         }
         const double r = (double)pv - (double)ys[src.idx[p]];
-        if constexpr (RB) {
+        if constexpr (M == LossMode::kRobust) {
           robust_step<T, K>(L, r, ws ? (double)ws[src.idx[p]] * r : r, acc[p], ps, pg);
-        } else if constexpr (W) {
+        } else if constexpr (M == LossMode::kWeighted) {
           const double rw = (double)ws[src.idx[p]] * r;
           ps += rw * r;
 #pragma unroll
@@ -1050,12 +1050,12 @@ __device__ __forceinline__ bool seat_turn(const FitArgs& a, int lane, int cs, Fi
   return my_prog >= 0;
 }
 
-// W: weighted launch (a.w: per-point weights of the slot of T); a resident slice stages the weight
-// column after the n_cols columns of X.  RB: robust launch (a.loss), weighted when a.w is set: it stages
-// exactly what the weighted or unweighted launch stages.
-template <typename T, int K, int P, bool W, bool RB = false>
+// kWeighted (a.w: per-point weights of the slot of T): a resident slice stages the weight column after the
+// n_cols columns of X.  kRobust (a.loss), weighted when a.w is set: it stages exactly what the weighted or
+// linear launch stages.
+template <typename T, int K, int P, LossMode M>
 __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>()))
-    fit_kernel(const KernelArgs<FitArgs, W, RB> a) {
+    fit_kernel(const LaunchArgs<FitArgs, M> a) {
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   extern __shared__ __align__(16) double smem[];
@@ -1092,7 +1092,7 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
   const T* X = static_cast<const T*>(a.pts.X);
   const T* y = static_cast<const T*>(a.pts.y);
   const T* rb_w = nullptr;  // the weights of a robust launch (nullptr: unweighted)
-  if constexpr (RB) rb_w = static_cast<const T*>(a.w);
+  if constexpr (M == LossMode::kRobust) rb_w = static_cast<const T*>(a.w);
 
   double* wpart = smem + (size_t)G * seat_d;                      // [G][nw][K+1]
   double* scratch = wpart + (size_t)G * nw * (K + 1);             // [(K+1)][threads]
@@ -1127,12 +1127,12 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
     const bool use_tma = a.tma_ok && full > 0;
     if (tid == 0 && use_tma) {
       const uint32_t bytes = (uint32_t)full * (uint32_t)sizeof(T);
-      mbar_expect_tx(&s_bar, bytes * (uint32_t)(a.n_cols + 1 + (W || rb_w ? 1 : 0)));
+      mbar_expect_tx(&s_bar, bytes * (uint32_t)(a.n_cols + 1 + (M == LossMode::kWeighted || rb_w ? 1 : 0)));
       tma_bulk_load(ys, y + n0, bytes, &s_bar);
       for (int j = 0; j < VSR_MAX_VARS; ++j)
         if (a.col_of_var[j] >= 0)
           tma_bulk_load(xs + (size_t)a.col_of_var[j] * stride, X + (int64_t)j * a.pts.ldx + n0, bytes, &s_bar);
-      if constexpr (W)
+      if constexpr (M == LossMode::kWeighted)
         tma_bulk_load(xs + (size_t)a.n_cols * stride, static_cast<const T*>(a.w) + n0, bytes, &s_bar);
       if (rb_w) tma_bulk_load(xs + (size_t)a.n_cols * stride, rb_w + n0, bytes, &s_bar);
     }
@@ -1140,7 +1140,7 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
       // everything TMA does not move (all of it when the caller's memory is unaligned): coalesced loads
       const int first = use_tma ? full : 0;
       for (int i = first + tid; i < cnt; i += blockDim.x) ys[i] = y[n0 + i];
-      if constexpr (W) {
+      if constexpr (M == LossMode::kWeighted) {
         T* wsl = xs + (size_t)a.n_cols * stride;
         for (int i = first + tid; i < cnt; i += blockDim.x) wsl[i] = static_cast<const T*>(a.w)[n0 + i];
       }
@@ -1241,19 +1241,19 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
         if (c.prog < 0) {  // the seat is closed
           live &= ~(1u << g);
         } else {
-          if constexpr (RB) {
+          if constexpr (M == LossMode::kRobust) {
             if (a.resident)
-              sweep_slice<T, K, P, false, false, true>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
+              sweep_slice<T, K, P, false, M>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
                                                        rb_w ? xs + (size_t)a.n_cols * stride : nullptr, a.loss);
             else
-              sweep_points<T, K, P, false, false, true>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid,
+              sweep_points<T, K, P, false, M>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid,
                                                         snt, rb_w, a.loss);
-          } else if constexpr (W) {
+          } else if constexpr (M == LossMode::kWeighted) {
             if (a.resident)
-              sweep_slice<T, K, P, false, true>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
+              sweep_slice<T, K, P, false, M>(c_insn, c_imm, c_cst, xs, ys, stride, cnt, scratch, stid, snt,
                                                 xs + (size_t)a.n_cols * stride);
             else
-              sweep_points<T, K, P, false, true>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid, snt,
+              sweep_points<T, K, P, false, M>(c_insn, c_imm, c_cst, X, y, a.pts.ldx, n0, n1, scratch, stid, snt,
                                                  static_cast<const T*>(a.w));
           } else {
             if (a.resident)
@@ -1292,9 +1292,10 @@ __global__ void __launch_bounds__((fit_max_threads<T, K>()), (fit_min_ctas<T, K>
 }
 
 // dynamic shared memory of eval_kernel, in doubles: red[(K+1)*threads] | cst[k] | imm | insn
-// W: weighted sums (a.w, read from global memory like y).  RB: robust sums (a.loss), weighted when a.w is set.
-template <typename T, int K, int P, bool W, bool RB = false>
-__global__ void __launch_bounds__(256) eval_kernel(const KernelArgs<EvalArgs, W, RB> a) {
+// kWeighted: weighted sums (a.w, read from global memory like y).  kRobust: robust sums (a.loss), weighted
+// when a.w is set.
+template <typename T, int K, int P, LossMode M>
+__global__ void __launch_bounds__(256) eval_kernel(const LaunchArgs<EvalArgs, M> a) {
   extern __shared__ double smem[];
   const int pair = blockIdx.x;
   const int split = blockIdx.y;
@@ -1326,12 +1327,12 @@ __global__ void __launch_bounds__(256) eval_kernel(const KernelArgs<EvalArgs, W,
   n0 = n0 < N ? n0 : N;
   n1 = n1 < N ? n1 : N;
 
-  if constexpr (RB)  // (nor robust)
-    sweep_points<T, K, P, false, false, true>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
+  if constexpr (M == LossMode::kRobust)  // (nor robust)
+    sweep_points<T, K, P, false, M>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
                                               static_cast<const T*>(a.pts.y), a.pts.ldx, n0, n1, red,
                                               (int)threadIdx.x, (int)blockDim.x, static_cast<const T*>(a.w), a.loss);
-  else if constexpr (W)  // (vsr_score, the nan_to_num rule, is never weighted)
-    sweep_points<T, K, P, false, true>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
+  else if constexpr (M == LossMode::kWeighted)  // (vsr_score, the nan_to_num rule, is never weighted)
+    sweep_points<T, K, P, false, M>(s_insn, s_imm, cst, static_cast<const T*>(a.pts.X),
                                        static_cast<const T*>(a.pts.y), a.pts.ldx, n0, n1, red, (int)threadIdx.x,
                                        (int)blockDim.x, static_cast<const T*>(a.w));
   else if (K == 0 && a.nan_to_num)  // scoring rule of the drivers, value only
@@ -1375,12 +1376,13 @@ __host__ __device__ inline size_t eval_tile_fixed_doubles(int K, int threads, in
   return (d + 1) & ~(size_t)1;
 }
 
-// W: weighted sums.  The weights are read from global memory (a.w, like y in eval_kernel), not staged: the
-// chunks are those of the unweighted launch, so the partial sums are formed in the same order and w = 1
-// gives the unweighted result bit for bit.  RB: robust sums (a.loss), weights as in W when a.w is set.
-template <typename T, int K, int P, bool W, bool RB = false>
+// kWeighted: weighted sums.  The weights are read from global memory (a.w, like y in eval_kernel), not
+// staged: the chunks are those of the linear launch, so the partial sums are formed in the same order and
+// w = 1 gives the linear result bit for bit.  kRobust: robust sums (a.loss), weights as in kWeighted when
+// a.w is set.
+template <typename T, int K, int P, LossMode M>
 __global__ void __launch_bounds__((eval_tile_threads<K>()), 1)
-    eval_tile_kernel(const KernelArgs<EvalTileArgs, W, RB> a) {
+    eval_tile_kernel(const LaunchArgs<EvalTileArgs, M> a) {
   extern __shared__ __align__(16) double smem[];
   __shared__ __align__(8) uint64_t s_bar;
   const int tid = threadIdx.x, nt = blockDim.x;
@@ -1460,11 +1462,11 @@ __global__ void __launch_bounds__((eval_tile_threads<K>()), 1)
     commit();
     __syncthreads();
     if (pair + 1 < a.e.n_pairs) fetch(pair + 1);
-    if constexpr (RB)
-      sweep_slice<T, K, P, false, false, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
+    if constexpr (M == LossMode::kRobust)
+      sweep_slice<T, K, P, false, M>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
                                                a.w ? static_cast<const T*>(a.w) + n0 : nullptr, a.loss);
-    else if constexpr (W)
-      sweep_slice<T, K, P, false, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
+    else if constexpr (M == LossMode::kWeighted)
+      sweep_slice<T, K, P, false, M>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt,
                                         static_cast<const T*>(a.w) + n0);
     else if (K == 0 && a.e.nan_to_num)
       sweep_slice<T, K, P, true>(s_insn, s_imm, cst, xs, ys, a.stride, cnt, red, tid, nt);
@@ -1512,16 +1514,16 @@ __host__ __device__ inline int gram_nsplit(int64_t N, int64_t tile) {
 __host__ __device__ constexpr int gram_col_stride(int tile) { return tile + 1; }
 
 // dynamic shared memory of gram_kernel, in doubles: tile[(K+1) * gram_col_stride] | cst[k] | imm | insn
-// W: weighted sums rss = sum w r^2, jtj[a][b] = sum w J_a J_b (J^T W J).  The tile gets one column more, the
+// kWeighted: weighted sums rss = sum w r^2, jtj[a][b] = sum w J_a J_b (J^T W J).  The tile gets one column more, the
 // weights, and every term is fma(col_a * w, col_b, acc): w = 1.0 gives the unweighted sums bit for bit.
-// RB: curve_fit's statistics under a robust loss (a.loss, weighted when a.w is set): rss = sum C^2 rho(z),
+// kRobust: curve_fit's statistics under a robust loss (a.loss, weighted when a.w is set): rss = sum C^2 rho(z),
 // jtj[a][b] = sum w s J_a J_b with s = max(rho' + 2 z rho'', 2^-52) (least_squares' scaled Jacobian).  The
-// tile gets two factor columns where W parks w: w q (q = rho(z)/z) for rss and w s for the J entries, so the
+// tile gets two factor columns where kWeighted parks w: w q (q = rho(z)/z) for rss and w s for the J entries, so the
 // terms are fma(r * wq, r, acc) and fma(J_a * ws, J_b, acc), the unweighted / weighted sums when q = s = 1.
 // A non-finite r gets q = s = 1 (the outputs become non-finite, as in the linear kernel); a z that overflows
 // from a finite r parks r = 1 and wq = rho(inf) C^2, and s = 2^-52.
-template <int K, int P, bool W, bool RB = false>
-__global__ void __launch_bounds__(kGramThreads) gram_kernel(const KernelArgs<GramArgs, W, RB> a) {
+template <int K, int P, LossMode M>
+__global__ void __launch_bounds__(kGramThreads) gram_kernel(const LaunchArgs<GramArgs, M> a) {
   extern __shared__ double smem[];
   const int pair = blockIdx.x;
   const int split = blockIdx.y;
@@ -1531,8 +1533,8 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const KernelArgs<Gra
   constexpr int kEnt = gram_entries(K);
   const int prog = a.pair_prog[pair];
   const int k = a.pt.k[prog];
-  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K) (then w when W, then wq and ws when RB)
-  double* cst = s_val + (K + 1 + (W ? 1 : 0) + (RB ? 2 : 0)) * kLd;
+  double* s_val = smem;  // [K+1][kLd]: r, then J[0..K) (then w when kWeighted, wq and ws when kRobust)
+  double* cst = s_val + (K + 1 + (M == LossMode::kWeighted ? 1 : 0) + (M == LossMode::kRobust ? 2 : 0)) * kLd;
   double* s_imm = cst + k + 1;
   const int m_imm = a.pt.imm_off[prog + 1] - a.pt.imm_off[prog];
   vsr_insn_t* s_insn = reinterpret_cast<vsr_insn_t*>(s_imm + m_imm);
@@ -1582,8 +1584,8 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const KernelArgs<Gra
         s_val[j] = v[p].v - __ldg(y + xs.idx[p]);
 #pragma unroll
         for (int t = 0; t < K; ++t) s_val[(1 + t) * kLd + j] = v[p].d[t];
-        if constexpr (W) s_val[(K + 1) * kLd + j] = __ldg(static_cast<const double*>(a.w) + xs.idx[p]);
-        if constexpr (RB) {
+        if constexpr (M == LossMode::kWeighted) s_val[(K + 1) * kLd + j] = __ldg(static_cast<const double*>(a.w) + xs.idx[p]);
+        if constexpr (M == LossMode::kRobust) {
           const double r = s_val[j];
           const double w = a.w ? __ldg(static_cast<const double*>(a.w) + xs.idx[p]) : 1.0;
           double q = 1.0, g, s = 1.0, wq;
@@ -1605,11 +1607,11 @@ __global__ void __launch_bounds__(kGramThreads) gram_kernel(const KernelArgs<Gra
       }
     }
     __syncthreads();
-    if constexpr (RB) {
+    if constexpr (M == LossMode::kRobust) {
       const double* col_f = s_val + (K + (tid == 0 ? 1 : 2)) * kLd;
       if (tid < kEnt)
         for (int j = 0; j < cnt; ++j) acc = fma(col_a[j] * col_f[j], col_b[j], acc);
-    } else if constexpr (W) {
+    } else if constexpr (M == LossMode::kWeighted) {
       const double* col_w = s_val + (K + 1) * kLd;
       if (tid < kEnt)
         for (int j = 0; j < cnt; ++j) acc = fma(col_a[j] * col_w[j], col_b[j], acc);
